@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- MPC inner-loop benchmark (BASELINE.json metric: candidate rollouts/s and MPC solves/s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload cfg2|cfg4]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload cfg2|cfg4] [--dump-outputs DIR]
 
 Headline workload at every N (weak scaling: fixed work per GPU, robots are independent -- no collective):
   cfg2 = BASELINE.json configs[1]: 1,024 independent robots per GPU, horizon 3, FULL tree
@@ -38,6 +38,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the bench leaves the tree as it found it (it may be read-only)
 
 import numpy as np  # noqa: E402
 
@@ -572,6 +573,20 @@ def leg_leafwalk(solver, nat, C, torch, dev, ext, wl, scen, pk):
                 executed=dict(mufu_per_rollout=ex["mufu"], instructions_per_rollout=ex["instr"]))
 
 
+def dump_outputs(directory, tensors, dist, world, rank):
+    """Writes the arrays a caller of the timed step receives as DIR/<name>.npy in float64 (the int64 leaf index is
+    exact there), every robot of every rank in the global robot order: ~106 KB a GPU for cfg2, so nothing is sampled."""
+    arrays = {k: t.cpu().numpy().astype(np.float64) for k, t in tensors.items()}
+    if world > 1:
+        parts = [None] * world
+        dist.all_gather_object(parts, arrays)
+        arrays = {k: np.concatenate([p[k] for p in parts]) for k in arrays}
+    if rank == 0:
+        os.makedirs(directory, exist_ok=True)
+        for k, a in arrays.items():
+            np.save(os.path.join(directory, k + ".npy"), a)
+
+
 def run_gpu(args):
     import torch
     import torch.distributed as dist
@@ -657,6 +672,9 @@ def run_gpu(args):
     value = rollouts_per_step * args.steps / (total_ms * 1e-3)
     dev_index = oi.cpu().numpy().copy()
     dev_cost = oc.cpu().numpy().copy()
+    if args.dump_outputs:
+        # the last timed step's outputs, before the later legs reuse the buffers
+        dump_outputs(args.dump_outputs, dict(cost=oc, index=oi, traj=ot, first_control=ou), dist, world, rank)
 
     # ---------------- end-to-end through the host-buffer C-ABI call (pinned inputs, H2D + D2H inside)
     out_np = None
@@ -803,7 +821,13 @@ def main():
                     help="exhaustive prefix pass 1: 0 = MUFU.SQRT per leaf, 1 = screened (library default)")
     ap.add_argument("--algo", default="auto", choices=["auto", "prefix", "leafwalk"],
                     help="expansion kernel: prefix (default for this workload) or the one-thread-per-leaf design")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs (cost, index, traj, first_control) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the GPU step's outputs; the reference arm only counts leaves")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         run_reference(args)
