@@ -61,8 +61,11 @@ static void dfs(const ctx_t *c, int depth, double x, double y, double phi, int64
 }
 
 
+/* n work items: one per first control or -- split -- one per (first, second) control pair,
+ * item k = (i0 - i0_begin) * S + i1, so that a range of a few first controls still spreads over every core.
+ * Items in ascending order cover ascending, contiguous leaf-index ranges either way. */
 typedef struct {
-    const ctx_t *c; const double *state; int64_t i0_begin, n; int64_t next; double *bc; int64_t *bi;
+    const ctx_t *c; const double *state; int64_t i0_begin, n; int split; int64_t next; double *bc; int64_t *bi;
 } job_t;
 
 static int mpco_threads = 0;          /* 0 = all online cores */
@@ -76,7 +79,7 @@ static void *worker(void *arg)
     for (;;) {
         int64_t k = __atomic_fetch_add(&jb->next, 1, __ATOMIC_RELAXED);
         if (k >= jb->n) break;
-        int64_t i0 = jb->i0_begin + k;
+        int64_t i0 = jb->i0_begin + (jb->split ? k / c->S : k);
         double best = INFINITY;
         int64_t idx = -1;
         double p = jb->state[2] + c->dphi[i0];
@@ -85,6 +88,18 @@ static void *worker(void *arg)
         if (c->H == 1) {
             double J = leaf_cost(c, nx, ny, p);
             if (J < best) { best = J; idx = i0; }
+        } else if (jb->split) {           /* the second step as dfs() takes it */
+            int i1 = (int)(k % c->S);
+            double p1 = p + c->dphi[i1];
+            double x1 = nx + c->vv[i1] * cos(p1) * c->dt;
+            double y1 = ny + c->vv[i1] * sin(p1) * c->dt;
+            int64_t j = i0 * c->S + i1;
+            if (c->H == 2) {
+                double J = leaf_cost(c, x1, y1, p1);
+                if (J < best) { best = J; idx = j; }
+            } else {
+                dfs(c, 2, x1, y1, p1, j, &best, &idx);
+            }
         } else {
             dfs(c, 1, nx, ny, p, i0, &best, &idx);
         }
@@ -103,10 +118,12 @@ int mpco_solve_full(const double *vv, const double *dphi, int S, int H, int cost
     c.line_norm = sqrt((c.yt - c.y0) * (c.yt - c.y0) + (c.xt - c.x0) * (c.xt - c.x0));
     int64_t n = i0_end - i0_begin;
     if (n <= 0) { *out_cost = INFINITY; *out_index = -1; return 0; }
+    int nt = mpco_threads > 0 ? mpco_threads : (int)sysconf(_SC_NPROCESSORS_ONLN);
+    const int split = H >= 2 && n < 4 * (int64_t)nt;   /* few first controls: hand out (i0, i1) pairs */
+    if (split) n *= S;
     double *bc = (double *)malloc(sizeof(double) * n);
     int64_t *bi = (int64_t *)malloc(sizeof(int64_t) * n);
-    job_t job = {&c, state, i0_begin, n, 0, bc, bi};
-    int nt = mpco_threads > 0 ? mpco_threads : (int)sysconf(_SC_NPROCESSORS_ONLN);
+    job_t job = {&c, state, i0_begin, n, split, 0, bc, bi};
     if (nt > n) nt = (int)n;
     if (nt < 1) nt = 1;
     pthread_t *th = (pthread_t *)malloc(sizeof(pthread_t) * nt);
@@ -116,7 +133,7 @@ int mpco_solve_full(const double *vv, const double *dphi, int S, int H, int cost
     free(th);
     double best = INFINITY; int64_t idx = -1;
     for (int64_t k = 0; k < n; ++k)
-        if (bc[k] < best) { best = bc[k]; idx = bi[k]; }   /* ascending i0, strict: lowest index wins ties */
+        if (bc[k] < best) { best = bc[k]; idx = bi[k]; }   /* ascending items, strict: lowest index wins ties */
     free(bc); free(bi);
     *out_cost = best; *out_index = idx;
     return 0;
