@@ -102,6 +102,7 @@ def load():
     lib.mpcb_held_closed_loop_host.argtypes = loop
     lib.mpcb_held_closed_loop_device.argtypes = loop
     lib.mpcb_held_closed_loop_events_host.argtypes = loop[:8] + [vp, C.c_int32, C.c_double] + loop[8:] + [vp]
+    lib.mpcb_held_closed_loop_actual_host.argtypes = loop[:8] + [vp, C.c_int32, C.c_double, vp] + loop[8:] + [vp]
     lib.mpcb_held_tick_host.argtypes = [vp, vp, C.c_int, vp, C.c_int, C.c_double, C.c_double, C.c_double, C.c_int, C.c_int,
                                         vp, vp, vp, C.c_double, C.c_int, vp, vp, vp, vp]
     win = [vp, C.POINTER(LoopParams), C.c_int64, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
@@ -293,12 +294,15 @@ class Solver:
         return dict(cost=cost_o, index=idx_o, traj=traj_o, first_control=ctl_o, shape=shape_o)
 
     def held_closed_loop(self, params: "LoopParams", init, target, origin, first_threshold=None, slow_steps=None,
-                         events=None, radius_u_turn=0.0):
+                         events=None, radius_u_turn=0.0, rng_state=None):
         """Whole closed loops of the online controller for a batch of robots on the device
         (mpcb_held_closed_loop_host / _events_host). ``events``: an operator script [(tick, kind, a, b), ...] with kind
         EVENT_NEW_TARGET (a, b = the new target) or EVENT_TURN_LEFT / _RIGHT (a = distance), applied to every robot
         after the tick it names; ``radius_u_turn`` = L / sin(beta_max) for the turns.
-        Returns dict(log[N,max_ticks,5], ticks[N], status[N], final[N,6] = x_t, y_t, x_0, y_0, steps_for_slowing, m)."""
+        ``rng_state`` [N][625] uint32 (per robot numpy RandomState key[624] + pos): the "actual" run with actuator noise
+        (mpcb_held_closed_loop_actual_host); the input is not modified.
+        Returns dict(log[N,max_ticks,5], ticks[N], status[N], final[N,6] = x_t, y_t, x_0, y_0, steps_for_slowing, m),
+        with ``rng_state`` also the generators' states after the run."""
         ini = _arr(init, np.float64, (-1, 5))
         N = ini.shape[0]
         tg = _arr(np.broadcast_to(np.asarray(target, np.float64).reshape(-1, 2), (N, 2)), np.float64)
@@ -312,11 +316,20 @@ class Solver:
         for i, (tick, kind, a, b) in enumerate(events or ()):
             ev[i] = LoopEvent(int(tick), int(kind), float(a), float(b))
         final = np.empty((N, 6))
-        self._ck(self.lib.mpcb_held_closed_loop_events_host(self.h, C.byref(params), N, _ptr(ini), _ptr(tg), _ptr(og),
+        if rng_state is None:
+            self._ck(self.lib.mpcb_held_closed_loop_events_host(self.h, C.byref(params), N, _ptr(ini), _ptr(tg), _ptr(og),
+                                                                _ptr(thr), _ptr(sl), ev if events else None,
+                                                                len(events or ()), float(radius_u_turn), _ptr(log),
+                                                                _ptr(ticks), _ptr(status), _ptr(final)))
+            return dict(log=log, ticks=ticks, status=status, final=final)
+        rs = np.array(rng_state, dtype=np.uint32, order="C")         # a copy: the library updates it in place
+        if rs.shape != (N, 625):
+            raise ValueError(f"rng_state must be [N][625] = [{N}][625] (key[624] + pos per robot), got {rs.shape}")
+        self._ck(self.lib.mpcb_held_closed_loop_actual_host(self.h, C.byref(params), N, _ptr(ini), _ptr(tg), _ptr(og),
                                                             _ptr(thr), _ptr(sl), ev if events else None,
-                                                            len(events or ()), float(radius_u_turn), _ptr(log),
+                                                            len(events or ()), float(radius_u_turn), _ptr(rs), _ptr(log),
                                                             _ptr(ticks), _ptr(status), _ptr(final)))
-        return dict(log=log, ticks=ticks, status=status, final=final)
+        return dict(log=log, ticks=ticks, status=status, final=final, rng_state=rs)
 
     def full_closed_loop(self, cost, H, init_state, target, origin, first_threshold=None, eps=0.001, max_ticks=256):
         """Closed loop of the FULL-tree scripts for a batch of robots (mpcb_full_closed_loop_host): one batched

@@ -7,6 +7,7 @@
 #include "mpcb_types.cuh"
 #include "mpcb_bounds.cuh"
 #include "mpcb_handle.cuh"
+#include "mpcb_noise.cuh"
 
 #include <algorithm>
 #include <cmath>
@@ -281,7 +282,7 @@ int mpcb_destroy(mpcb_handle *h) {
                       &h->ctl32_slow, &h->sp, &h->segmin, &h->worklist, &h->misc, &h->tau, &h->bestJ, &h->bestIdx,
                       &h->lock, &h->ub, &h->tile_list, &h->reduce_scratch, &h->in_state, &h->in_target, &h->in_origin, &h->in_thr, &h->in_flags, &h->out_cost,
                       &h->out_index, &h->out_traj, &h->out_ctl, &h->dump_rec, &h->dump_j, &h->loop_log, &h->loop_ticks,
-                      &h->loop_status, &h->loop_events, &h->loop_final, &h->small_in, &h->small_out, &h->fl_last, &h->fl_k, &h->fl_have, &h->fl_flags,
+                      &h->loop_status, &h->loop_events, &h->loop_final, &h->loop_rng, &h->small_in, &h->small_out, &h->fl_last, &h->fl_k, &h->fl_have, &h->fl_flags,
                       &h->fl_count, &h->nccl_scratch, &h->cand, &h->cand_J, &h->cand_sel, &h->node_list})
         b->release();
     if (h->pin_in) cudaFreeHost(h->pin_in);
@@ -800,11 +801,12 @@ int mpcb_dump_leaves_host(mpcb_handle *h, int mode, int cost_kind, int H, int al
     return MPCB_OK;
 }
 
-// device pointers throughout; events / out_final may be null
+// device pointers throughout; events / out_final / rng_state may be null
 static int held_loop_core(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, const double *init,
                           const double *target, const double *origin, const double *first_threshold,
                           const int32_t *slow_steps, const mpcb_loop_event *events, int n_events, double radius_u_turn,
-                          double *out_log, int32_t *out_ticks, int32_t *out_status, double *out_final) {
+                          uint32_t *rng_state, double *out_log, int32_t *out_ticks, int32_t *out_status,
+                          double *out_final) {
     if (!h || !p) return MPCB_ERR_INVALID;
     if (N < 0 || N >= (1LL << 31)) return fail(h, MPCB_ERR_INVALID, "N out of range");
     if (N == 0) return MPCB_OK;
@@ -819,6 +821,7 @@ static int held_loop_core(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, 
     a.init = init; a.target = target; a.origin = origin; a.first_threshold = first_threshold;
     a.slow_steps = slow_steps; a.out_log = out_log; a.out_ticks = out_ticks; a.out_status = out_status;
     a.events = events; a.n_events = events ? n_events : 0; a.radius_u_turn = radius_u_turn; a.out_final = out_final;
+    a.rng_state = rng_state;
     CK(launch_held_loop(h->stream, a, h->sms));
     h->stats = mpcb_stats{};
     h->stats.kernel_launches = 1;
@@ -829,8 +832,8 @@ static int held_loop_core(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, 
 int mpcb_held_closed_loop_device(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, const double *init,
                                  const double *target, const double *origin, const double *first_threshold,
                                  const int32_t *slow_steps, double *out_log, int32_t *out_ticks, int32_t *out_status) {
-    return held_loop_core(h, p, N, init, target, origin, first_threshold, slow_steps, nullptr, 0, 0.0, out_log, out_ticks,
-                          out_status, nullptr);
+    return held_loop_core(h, p, N, init, target, origin, first_threshold, slow_steps, nullptr, 0, 0.0, nullptr, out_log,
+                          out_ticks, out_status, nullptr);
 }
 
 int mpcb_held_closed_loop_host(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, const double *init,
@@ -840,12 +843,11 @@ int mpcb_held_closed_loop_host(mpcb_handle *h, const mpcb_loop_params *p, int64_
                                              out_log, out_ticks, out_status, nullptr);
 }
 
-int mpcb_held_closed_loop_events_host(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, const double *init,
-                                      const double *target, const double *origin, const double *first_threshold,
-                                      const int32_t *slow_steps, const mpcb_loop_event *events, int32_t n_events,
-                                      double radius_u_turn, double *out_log, int32_t *out_ticks, int32_t *out_status,
-                                      double *out_final) {
-    if (!h || !p) return MPCB_ERR_INVALID;
+// host pointers; rng_state null = the noise-free loop
+static int held_loop_host(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, const double *init, const double *target,
+                          const double *origin, const double *first_threshold, const int32_t *slow_steps,
+                          const mpcb_loop_event *events, int32_t n_events, double radius_u_turn, uint32_t *rng_state,
+                          double *out_log, int32_t *out_ticks, int32_t *out_status, double *out_final) {
     if (n_events < 0 || n_events > 4096 || (n_events > 0 && !events))
         return fail(h, MPCB_ERR_INVALID, "closed loop: bad event script (n_events=%d)", n_events);
     for (int e = 0; e < n_events; ++e)
@@ -885,18 +887,52 @@ int mpcb_held_closed_loop_events_host(mpcb_handle *h, const mpcb_loop_params *p,
         CK(cudaMemcpyAsync(h->loop_events.p, events, sizeof(mpcb_loop_event) * n_events, cudaMemcpyHostToDevice, st));
         d_events = h->loop_events.as<mpcb_loop_event>();
     }
+    const size_t nrng = (size_t)N * mpcb::kMtWords;
+    if (rng_state) {
+        CK(h->loop_rng.ensure(sizeof(uint32_t) * nrng));
+        CK(cudaMemcpyAsync(h->loop_rng.p, rng_state, sizeof(uint32_t) * nrng, cudaMemcpyHostToDevice, st));
+    }
     if (out_final) CK(h->loop_final.ensure(sizeof(double) * 6 * N));
     CK(cudaMemsetAsync(h->loop_log.p, 0xFF, sizeof(double) * nlog, st));     // NaN pattern for the rows no tick wrote
     int rc = held_loop_core(h, p, N, h->in_state.as<double>(), h->in_target.as<double>(), h->in_origin.as<double>(), d_thr,
-                            d_slow, d_events, n_events, radius_u_turn, h->loop_log.as<double>(), h->loop_ticks.as<int>(),
-                            h->loop_status.as<int>(), out_final ? h->loop_final.as<double>() : nullptr);
+                            d_slow, d_events, n_events, radius_u_turn, rng_state ? h->loop_rng.as<uint32_t>() : nullptr,
+                            h->loop_log.as<double>(), h->loop_ticks.as<int>(), h->loop_status.as<int>(),
+                            out_final ? h->loop_final.as<double>() : nullptr);
     if (rc) return rc;
+    if (rng_state) CK(cudaMemcpyAsync(rng_state, h->loop_rng.p, sizeof(uint32_t) * nrng, cudaMemcpyDeviceToHost, st));
     if (out_final) CK(cudaMemcpyAsync(out_final, h->loop_final.p, sizeof(double) * 6 * N, cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(out_log, h->loop_log.p, sizeof(double) * nlog, cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(out_ticks, h->loop_ticks.p, sizeof(int) * N, cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(out_status, h->loop_status.p, sizeof(int) * N, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     return MPCB_OK;
+}
+
+int mpcb_held_closed_loop_events_host(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, const double *init,
+                                      const double *target, const double *origin, const double *first_threshold,
+                                      const int32_t *slow_steps, const mpcb_loop_event *events, int32_t n_events,
+                                      double radius_u_turn, double *out_log, int32_t *out_ticks, int32_t *out_status,
+                                      double *out_final) {
+    if (!h || !p) return MPCB_ERR_INVALID;
+    return held_loop_host(h, p, N, init, target, origin, first_threshold, slow_steps, events, n_events, radius_u_turn,
+                          nullptr, out_log, out_ticks, out_status, out_final);
+}
+
+int mpcb_held_closed_loop_actual_host(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, const double *init,
+                                      const double *target, const double *origin, const double *first_threshold,
+                                      const int32_t *slow_steps, const mpcb_loop_event *events, int32_t n_events,
+                                      double radius_u_turn, uint32_t *rng_state, double *out_log, int32_t *out_ticks,
+                                      int32_t *out_status, double *out_final) {
+    if (!h || !p) return MPCB_ERR_INVALID;
+    if (!rng_state) return fail(h, MPCB_ERR_INVALID, "actual closed loop: null rng_state");
+    for (int64_t n = 0; n < N; ++n) {
+        const uint32_t pos = rng_state[n * mpcb::kMtWords + mpcb::kMtN];
+        if (pos > (uint32_t)mpcb::kMtN)
+            return fail(h, MPCB_ERR_INVALID, "actual closed loop: robot %lld has generator position %u (outside [0, 624])",
+                        (long long)n, pos);
+    }
+    return held_loop_host(h, p, N, init, target, origin, first_threshold, slow_steps, events, n_events, radius_u_turn,
+                          rng_state, out_log, out_ticks, out_status, out_final);
 }
 
 static int check_window_params(mpcb_handle *h, const mpcb_loop_params *p) {

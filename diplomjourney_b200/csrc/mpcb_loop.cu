@@ -7,14 +7,19 @@
 //             apply     finishing heuristic m, result pose, threshold reset math_model_tree.py:388-429
 //             stop      is_on_target, repeated-position ("Recursive error") math_model_tree.py:48-52,559-563
 //             events    new_target / turn_left / turn_right + slow_down     math_model_tree.py:118-226,564-569
+//             noise     (actual run only) get_actual_velocity / _beta_angle math_model_tree.py:259-275,590-597
 // Operator events come as a script {tick, kind, a, b} (the reference's demo: turn_right at tick 60, turn_left at 90,
 // new_target at 110); thread 0 applies an event after the tick it names, to the robot's own pose, and the CTA
 // reloads target, line and cost constants from shared memory.
+// The "actual" run (math_mpc(..., True)) gives every robot its own numpy RandomState (key[624] + pos, mpcb_noise.cuh):
+// the CTA keeps it in shared memory while it runs the robot, and thread 0 perturbs the applied (v, beta) after every
+// tick, draw for draw as the reference does.  A template flag keeps the noise-free loop free of all of it.
 //
 // A HELD tick is tiny (S <= 451 candidates x H steps), so the loop is latency-bound, not
 // throughput-bound: everything is evaluated directly in float64 with the reference's formula and
 // operation order -- no fp32 stage, no refinement -- and the batch dimension (robots) fills the GPU.
 #include "mpcb_events.cuh"
+#include "mpcb_noise.cuh"
 
 #include <cmath>
 
@@ -142,6 +147,7 @@ __device__ __forceinline__ void load_cost(LoopCost &cost, const double *target, 
     cost.kind = kind;
 }
 
+template <bool kNoise>
 __global__ void __launch_bounds__(kLoopThreads) held_loop_kernel(const LoopArgs a) {
     __shared__ double s_V[kMaxWin], s_B[kMaxWin], s_tanB[kMaxWin];
     __shared__ double s_J[kLoopThreads / 32];
@@ -155,6 +161,7 @@ __global__ void __launch_bounds__(kLoopThreads) held_loop_kernel(const LoopArgs 
     // a flag: every thread compares it with its own copy after the tick's last barrier, so it never has to be cleared)
     __shared__ double s_line[4];
     __shared__ int s_events;
+    extern __shared__ unsigned s_mt[];  // kNoise: the running robot's generator, key[624] + pos (dynamic, kMtWords words)
     const mpcb_loop_params &p = a.p;
     const int tid = threadIdx.x;
     if (tid == 0) s_events = 0;
@@ -175,6 +182,8 @@ __global__ void __launch_bounds__(kLoopThreads) held_loop_kernel(const LoopArgs 
             for (int k = 0; k < 5; ++k) s_state[k] = a.init[5 * n + k];
             xprev = s_state[0]; yprev = s_state[1];
         }
+        if constexpr (kNoise)
+            for (int i = tid; i < kMtWords; i += kLoopThreads) s_mt[i] = a.rng_state[(size_t)n * kMtWords + i];
         __syncthreads();
 
         for (;;) {
@@ -225,9 +234,16 @@ __global__ void __launch_bounds__(kLoopThreads) held_loop_kernel(const LoopArgs 
                     if (pick > p.H - 1) pick = p.H - 1;
                     const double rx = opt[3 * pick], ry = opt[3 * pick + 1], rphi = opt[3 * pick + 2];
                     thr = 9223372036854775807.0;            // sys.maxsize (math_model_tree.py:428)
+                    // the applied (v, beta): the commanded ones, or in the actual run what the actuators make of them
+                    // (math_model_tree.py:590-597) -- velocity drawn first, then beta, and before the stall stop
+                    double av = res_v, ab = res_beta;
+                    if constexpr (kNoise) {
+                        av = actual_velocity(res_v, s_mt);
+                        ab = actual_beta(res_beta, s_mt);
+                    }
                     double *log = a.out_log + ((size_t)n * p.max_ticks + ticks) * 5;
-                    log[0] = rx; log[1] = ry; log[2] = rphi; log[3] = res_v; log[4] = res_beta;
-                    s_state[0] = rx; s_state[1] = ry; s_state[2] = rphi; s_state[3] = res_v; s_state[4] = res_beta;
+                    log[0] = rx; log[1] = ry; log[2] = rphi; log[3] = av; log[4] = ab;
+                    s_state[0] = rx; s_state[1] = ry; s_state[2] = rphi; s_state[3] = av; s_state[4] = ab;
                     ticks += 1;
                     if (recursive) { stop = 1; status = 1; }        // "Recursive error." (math_model_tree.py:559-561)
                     else {
@@ -261,6 +277,8 @@ __global__ void __launch_bounds__(kLoopThreads) held_loop_kernel(const LoopArgs 
                 f[0] = cost.xt; f[1] = cost.yt; f[2] = cost.ox; f[3] = cost.oy; f[4] = (double)slow_steps; f[5] = (double)m;
             }
         }
+        if constexpr (kNoise)       // thread 0's last draw came before the barrier that ended the loop
+            for (int i = tid; i < kMtWords; i += kLoopThreads) a.rng_state[(size_t)n * kMtWords + i] = s_mt[i];
     }
 }
 
@@ -444,14 +462,21 @@ cudaError_t launch_full_apply(cudaStream_t st, const FullLoopArgs &a) {
     return cudaGetLastError();
 }
 
-cudaError_t launch_held_loop(cudaStream_t st, const LoopArgs &a, int sms) {
+template <bool kNoise>
+static cudaError_t launch_held_loop_t(cudaStream_t st, const LoopArgs &a, int sms) {
+    const size_t smem = kNoise ? sizeof(unsigned) * kMtWords : 0;
     int per_sm = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, held_loop_kernel, kLoopThreads, 0) != cudaSuccess || per_sm < 1)
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, held_loop_kernel<kNoise>, kLoopThreads, smem) != cudaSuccess ||
+        per_sm < 1)
         per_sm = 1;
     long long grid = (long long)sms * per_sm;
     if (grid > a.N) grid = a.N;
-    held_loop_kernel<<<(unsigned)grid, kLoopThreads, 0, st>>>(a);
+    held_loop_kernel<kNoise><<<(unsigned)grid, kLoopThreads, smem, st>>>(a);
     return cudaGetLastError();
+}
+
+cudaError_t launch_held_loop(cudaStream_t st, const LoopArgs &a, int sms) {
+    return a.rng_state ? launch_held_loop_t<true>(st, a, sms) : launch_held_loop_t<false>(st, a, sms);
 }
 
 }  // namespace mpcb

@@ -321,6 +321,8 @@ scripted_events = True      # the demo run's operator events at ticks 1/60/90/11
 # the programmed run's script (math_model_tree.py:564-569) in the form mpcb_held_closed_loop_events takes
 DEMO_EVENTS = ((60, _native.EVENT_TURN_RIGHT, 2.0, 0.0), (90, _native.EVENT_TURN_LEFT, 2.0, 0.0),
                (110, _native.EVENT_NEW_TARGET, 2.0, 3.0))
+# the actual run's script (:617-624): new_target(2, 3) after the first tick, then the programmed run's
+ACTUAL_EVENTS = ((1, _native.EVENT_NEW_TARGET, 2.0, 3.0),) + DEMO_EVENTS
 
 
 def _scripted_events(tick, px, py, pphi, pv, isActual):
@@ -466,8 +468,30 @@ def _math_mpc_batch_ticks(ini, tgt, org, first, max_ticks, cost_kind, isActual, 
                 status=np.array([c["status"] for c in robots], np.int32), robots=robots)
 
 
+def _pack_generators(gens):
+    """[N][625] uint32: key[624] + pos of each generator's legacy MT19937 state (RandomState.get_state())."""
+    out = np.empty((len(gens), 625), np.uint32)
+    for i, g in enumerate(gens):
+        st = g.get_state()
+        out[i, :624], out[i, 624] = st[1], st[2]
+    return out
+
+
+def _math_mpc_batch_device_noise(params, ini, tgt, org, first, rngs, events):
+    """The actual run on the device (mpcb_held_closed_loop_actual): each robot draws from its own generator, whose state
+    goes to the device as get_state() and comes back through set_state (has_gauss / cached_gaussian kept)."""
+    gens = [random] if rngs is None else rngs
+    script = ACTUAL_EVENTS if events is True else list(events or ())
+    r = _solver().held_closed_loop(params, ini, tgt, org, first_threshold=first, events=script or None,
+                                   radius_u_turn=radius_u_turn, rng_state=_pack_generators(gens))
+    for g, st in zip(gens, r.pop("rng_state")):
+        old = g.get_state()
+        g.set_state((old[0], st[:624].copy(), int(st[624]), old[3], old[4]))
+    return r
+
+
 def math_mpc_batch(initial_coordinates, target_coordinates, max_ticks=512, origin=None, cost_kind=None,
-                   isActual=False, rngs=None, events=False, host_loop=False):
+                   isActual=False, rngs=None, events=False, host_loop=False, device_noise=False):
     """EXTENSION (not in the reference): the closed loop of ``math_mpc`` for a whole batch of robots.
     ``initial_coordinates`` [N][5] = x, y, phi, v, beta; ``target_coordinates`` [N][2].  The tracked line starts at
     the module's x_0, y_0 unless ``origin`` [N][2] is given.
@@ -483,6 +507,13 @@ def math_mpc_batch(initial_coordinates, target_coordinates, max_ticks=512, origi
       (``mpcb_solve_held_windows``).  The returned dict then also carries ``robots``: per robot the state and log
       lists of the reference module (``actual_result_trajectory_x`` ...).  ``host_loop=True`` takes this per-tick
       path for a noise-free run as well (events then = the demo script, applied by the module's own functions).
+    * ``isActual=True, device_noise=True``: the whole noisy run in ONE launch (``mpcb_held_closed_loop_actual``): every
+      robot draws from its own generator on the device, draw for draw as the per-tick path draws from it, and
+      ``rngs[i]`` is left in exactly the state the per-tick path leaves it in.  ``rngs=None`` uses (and advances) the
+      module generator ``np.random``, for N == 1 only: one generator shared by several robots interleaves their draws,
+      which one CTA per robot cannot reproduce.  ``events=True`` is the actual run's script (new_target(2, 3) after tick
+      1, then the demo script), or any ``[(tick, kind, a, b), ...]``.  Returns log, ticks, status and final as the
+      noise-free device loop does (no ``robots``).
 
     Returns dict(log[N][max_ticks][5], ticks[N], status[N])."""
     from . import config as _cfg
@@ -490,6 +521,22 @@ def math_mpc_batch(initial_coordinates, target_coordinates, max_ticks=512, origi
     org = np.array([[x_0, y_0]], dtype=np.float64) if origin is None else np.asarray(origin, np.float64).reshape(-1, 2)
     tgt = np.asarray(target_coordinates, dtype=np.float64).reshape(-1, 2)
     n = ini.shape[0]
+    if device_noise:
+        if not isActual:
+            raise ValueError("device_noise=True is the actual run's actuator noise: it needs isActual=True")
+        if host_loop:
+            raise ValueError("device_noise=True runs the whole loop on the device; host_loop=True is the per-tick path")
+        if rngs is None:
+            if n != 1:
+                raise ValueError("rngs=None shares the module generator among the robots, which interleaves their draws; "
+                                 "pass one numpy RandomState per robot (or run one robot)")
+        else:
+            rngs = list(rngs)
+            if len(rngs) != n:
+                raise ValueError(f"rngs holds {len(rngs)} generators for {n} robots")
+            for g in rngs:
+                if not isinstance(g, np.random.RandomState):
+                    raise TypeError(f"rngs entries must be numpy RandomState (the legacy MT19937 stream), not {type(g)!r}")
     org = np.broadcast_to(org, (n, 2))
     tgt = np.broadcast_to(tgt, (n, 2))
     # optimal_criterion before the first tick = control_criterion of the line origin (math_model_tree.py:676)
@@ -502,13 +549,15 @@ def math_mpc_batch(initial_coordinates, target_coordinates, max_ticks=512, origi
             first[i] = control_criterion([org[i, 0], org[i, 1], phi_0])
     finally:
         g.update(x_t=saved[0], y_t=saved[1], x_0=saved[2], y_0=saved[3])
+    params = _native.LoopParams.from_config(_cfg, _native.COST_TREE if cost_kind is None else cost_kind,
+                                            prediction_horizon, max_ticks)
+    if device_noise:
+        return _math_mpc_batch_device_noise(params, ini, tgt, org, first, rngs, events)
     if isActual or host_loop:
         if not isinstance(events, bool) and events is not None:
             raise ValueError("a custom event script runs on the device loop only (isActual=False, host_loop=False); "
                              "the per-tick path applies the demo script (events=True) with the module's own functions")
         return _math_mpc_batch_ticks(ini, tgt, org, first, max_ticks, cost_kind, isActual, rngs, bool(events))
-    params = _native.LoopParams.from_config(_cfg, _native.COST_TREE if cost_kind is None else cost_kind,
-                                            prediction_horizon, max_ticks)
     script = DEMO_EVENTS if events is True else list(events or ())
     return _solver().held_closed_loop(params, ini, tgt, org, first_threshold=first, events=script or None,
                                       radius_u_turn=radius_u_turn)

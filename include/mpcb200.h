@@ -249,6 +249,22 @@ MPCB_API int mpcb_held_closed_loop_events_host(mpcb_handle *h, const mpcb_loop_p
                                       const mpcb_loop_event *events, int32_t n_events, double radius_u_turn,
                                       double *out_log, int32_t *out_ticks, int32_t *out_status, double *out_final);
 
+/* The same loop as the reference's "actual" run math_mpc(..., True) (math_model_tree.py:580-629): after every tick the
+ * applied (v, beta) are perturbed by get_actual_velocity / get_actual_beta_angle (:259-275), drawn from the robot's OWN
+ * numpy RandomState -- the legacy MT19937 stream, its random() and masked-rejection randint(), bit for bit.  The noisy
+ * values are logged (columns 3-4) and build the next tick's acceleration windows.  Velocity is drawn first, then beta,
+ * also on the tick that ends in the repeated-position stop; the on-target, max-ticks and no-leaf stops draw nothing.
+ * Events as for mpcb_held_closed_loop_events_host (the reference's actual run adds new_target(2, 3) after tick 1).
+ *   rng_state[N][625]  in/out: per robot RandomState.get_state()'s key[624] followed by pos (0..624); on return
+ *                      the state the generator has after the robot's draws.  NULL, or a pos outside [0, 624], is
+ *                      MPCB_ERR_INVALID (checked before anything is copied). */
+MPCB_API int mpcb_held_closed_loop_actual_host(mpcb_handle *h, const mpcb_loop_params *p, int64_t N,
+                                      const double *init, const double *target, const double *origin,
+                                      const double *first_threshold, const int32_t *slow_steps,
+                                      const mpcb_loop_event *events, int32_t n_events, double radius_u_turn,
+                                      uint32_t *rng_state,
+                                      double *out_log, int32_t *out_ticks, int32_t *out_status, double *out_final);
+
 /* ONE online tick for a batch of robots that each have their OWN acceleration window (SURVEY 8f row f2).  The
  * reference rebuilds the control window per robot and per tick around the robot's current (v, beta)
  * (vector_of_velocities / vector_of_beta_angles, math_model_tree.py:239-256, called at :543-545 and -- with the noisy
