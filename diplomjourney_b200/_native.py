@@ -34,7 +34,7 @@ class MpcbError(RuntimeError):
 class Stats(C.Structure):
     _fields_ = [("units", C.c_int64), ("leaves_per_solve", C.c_int64), ("segments", C.c_int64),
                 ("refine_segments", C.c_int64), ("refine_candidates", C.c_int64), ("pruned_units", C.c_int64),
-                ("algo", C.c_int32), ("kernel_launches", C.c_int32)]
+                ("algo", C.c_int32), ("kernel_launches", C.c_int32), ("stage2_units", C.c_int64)]
 
 
 class LoopParams(C.Structure):

@@ -241,6 +241,12 @@ static int ensure_tables(mpcb_handle *h) {
     g.nv = nv; g.ppr = rows_fit ? ppr : 0;
     g.ctl32 = h->ctl32.as<float2>(); g.ctl32_slow = h->ctl32_slow.as<float2>();
     g.S = S; g.nb = nb; g.dt = delta_t; g.smax = smax; g.dphimax = dphimax; g.smin = smin;
+    g.sbox = ScreenBox{l32[0].x, l32[0].x, l32[0].y, l32[0].y, l32[0].w, l32[0].w};
+    for (int c = 1; c < S; ++c) {
+        g.sbox.amin = std::min(g.sbox.amin, l32[c].x); g.sbox.amax = std::max(g.sbox.amax, l32[c].x);
+        g.sbox.bmin = std::min(g.sbox.bmin, l32[c].y); g.sbox.bmax = std::max(g.sbox.bmax, l32[c].y);
+        g.sbox.gmin = std::min(g.sbox.gmin, l32[c].w); g.sbox.gmax = std::max(g.sbox.gmax, l32[c].w);
+    }
     h->tables_ready = true;
     return MPCB_OK;
 }
@@ -320,7 +326,10 @@ int mpcb_set_option(mpcb_handle *h, const char *name, double value) {
     }
     else if (!strcmp(name, "prune")) h->prune = value != 0.0;
     else if (!strcmp(name, "dump_direct")) h->dump_direct = value != 0.0;
-    else if (!strcmp(name, "screen")) h->screen = value != 0.0;
+    else if (!strcmp(name, "screen")) {
+        if (value != 0.0 && value != 1.0 && value != 2.0) return fail(h, MPCB_ERR_INVALID, "screen must be 0, 1 or 2");
+        h->screen = (int)value;
+    }
     else if (!strcmp(name, "prefilter")) h->prefilter = value != 0.0;
     else if (!strcmp(name, "subtree_cut")) {
         if (value != 0.0 && value != 1.0 && value != 2.0 && value != 3.0) return fail(h, MPCB_ERR_INVALID, "subtree_cut must be 0, 1, 2 or 3");
@@ -416,7 +425,8 @@ static int solve_core(mpcb_handle *h, int mode, int cost_kind, int H, int64_t N,
     CK(h->ub.ensure(sizeof(unsigned long long) * N));
     // misc: [0..3] work_count (u32) | [8..11] tile_count (u32, subtree cut) | [16..47] counters (4 x u64) |
     //       [48..55] frontier counts (2 x u32) | [56..59] frontier overflow flag (u32) | [60..63] candidate count (u32) |
-    //       [4..7] listed refinement nodes (u32) | [64..71] next work item of the refinement filter (u64)
+    //       [4..7] listed refinement nodes (u32) | [64..71] next work item of the refinement filter (u64) |
+    //       [72..79] nodes that passed stage 1 of the two-stage screen (u64, counters[7])
     unsigned *work_count = h->misc.as<unsigned>();
     unsigned long long *counters = reinterpret_cast<unsigned long long *>(h->misc.as<char>() + 16);
     CK(cudaMemsetAsync(h->misc.p, 0, 128, h->stream));
@@ -578,12 +588,13 @@ int mpcb_get_stats(mpcb_handle *h, mpcb_stats *out) {
     if (!h || !out) return MPCB_ERR_INVALID;
     CK(cudaSetDevice(h->device));
     if (h->stats.refine_segments < 0 && h->misc.p) {
-        unsigned long long c[3] = {0, 0, 0};
+        unsigned long long c[8] = {};
         CK(cudaStreamSynchronize(h->stream));
         CK(cudaMemcpy(c, h->misc.as<char>() + 16, sizeof c, cudaMemcpyDeviceToHost));
         h->stats.refine_segments = (int64_t)c[0];
         h->stats.refine_candidates = (int64_t)c[1];
         h->stats.pruned_units = (int64_t)c[2];
+        h->stats.stage2_units = (int64_t)c[7];
     }
     *out = h->stats;
     return MPCB_OK;

@@ -51,7 +51,8 @@ struct mpcb_handle_s {
     int npt = 2;          // exhaustive prefix pass 1: nodes per thread (2: +6 %, tools/ubench)
     unsigned long long frontier_cap = mpcb::kFrontierCap;   // entries per frontier list (option, diagnostics: a tiny value forces the fallback)
     int subtree_cut = 2;       // pruned pass 1, H >= 3: 0 off, 1 depth-(H-2) bound per 256-node tile, 2 auto (frontier descent from the root for trees of more than one tile batch), 3 frontier always
-    int screen = 1;       // exhaustive prefix pass 1 (prune = 0): 1 = screen loop without MUFU + rare full re-run, 0 = sqrt per leaf
+    int screen = 2;       // exhaustive prefix pass 1 (prune = 0): 2 = screen in two stages (distance first), 1 = screen loop without
+                          // MUFU + rare full re-run, 0 = sqrt per leaf
     int prefilter = 1;    // pruned pass 1: fp32 pre-filter before the float64 node set-up (identical results)
     int prune = 1;        // exact branch-and-bound in the prefix kernel (identical results, fewer leaves evaluated)   // host-API HELD solves with few candidates take the one-launch float64 path
     // scratch

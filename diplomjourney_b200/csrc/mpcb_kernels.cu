@@ -47,6 +47,9 @@
 #define MPCB_UNROLL_ROWS 4  // pairs per unrolled iteration of the row loop (a row of the cfg2 grid has 21 pairs: 3 / 4 / 7 / 8 / 21
                             // = 3.15 / 3.20 / 3.20 / 3.07 / 3.17e12)
 #endif
+#ifndef MPCB_UNROLL_DIST
+#define MPCB_UNROLL_DIST 7  // pairs per unrolled iteration of the stage-1 row loop of the two-stage screen (a cfg2 row = 3 x 7 pairs)
+#endif
 #ifndef MPCB_UNROLL
 #define MPCB_UNROLL 8   // pairs per unrolled iteration of the pass-1 loop (4..16 are within 1 %, profiles/r1b_variants.txt)
 #endif
@@ -531,6 +534,43 @@ __device__ __forceinline__ void prefix_screen_loop_rows(const float4 *__restrict
     for (int k = 0; k < NPT; ++k) mx[k] = m[k];
 }
 
+// Stage 1 of the two-stage screen (option screen = 2, mpcb_screen.cuh): the same walk over the row table, forming only
+// -dd -- the same operands and operations as prefix_screen_loop_rows, so the very same values -- and keeping its maximum
+// per node: 2 FFMA2 + 1 FMNMX3 per node and leaf pair and one LDS.128 (the pair's a, b) instead of 7 + 1 + 1 and
+// LDS.128 + LDS.64.  The line and heading terms enter through a per-node bound (screen_stage1_tmax).
+template <int NPT>
+__device__ __forceinline__ void prefix_dist_loop_rows(const float4 *__restrict__ tab, int nv, int ppr,
+                                                      const ParentRegs (&p)[NPT], float (&mx)[NPT]) {
+    float2 U[NPT], W[NPT];
+    float nD[NPT], m[NPT];
+#pragma unroll
+    for (int k = 0; k < NPT; ++k) {
+        U[k] = make_float2(-p[k].u2s, -p[k].u2s); W[k] = make_float2(-p[k].w2s, -p[k].w2s);
+        nD[k] = -p[k].D2s;
+        m[k] = -INFINITY;
+    }
+    constexpr int kUnroll = NPT == 2 ? MPCB_UNROLL_DIST : MPCB_UNROLL4;
+    for (int iv = 0; iv < nv; ++iv) {
+        const float4 *__restrict__ row = tab + 2 * iv * ppr;
+        const float rv = row[1].x;
+        float2 DV[NPT];
+#pragma unroll
+        for (int k = 0; k < NPT; ++k) { const float d = __fmaf_rn(-kWd2f, rv, nD[k]); DV[k] = make_float2(d, d); }
+#pragma unroll kUnroll
+        for (int i = 0; i < ppr; ++i) {
+            const float4 t0 = row[2 * i];
+            const float2 A = make_float2(t0.x, t0.y), B = make_float2(t0.z, t0.w);
+#pragma unroll
+            for (int k = 0; k < NPT; ++k) {
+                const float2 ndd = __ffma2_rn(U[k], A, __ffma2_rn(W[k], B, DV[k]));                    // -dd
+                m[k] = fmaxf(m[k], fmaxf(ndd.x, ndd.y));
+            }
+        }
+    }
+#pragma unroll
+    for (int k = 0; k < NPT; ++k) mx[k] = m[k];
+}
+
 // scalar flavour on the same pair table: NEAR regime, or a node sitting exactly on the line origin
 template <bool HEAD>
 __device__ __forceinline__ float prefix_min_loop_scalar(const float4 *__restrict__ tab, int npairs, const ParentRegs &pr,
@@ -961,10 +1001,12 @@ __global__ void __launch_bounds__(kThreads, 4) refine_scan_kernel(const LaunchAr
 // Pass 1, exhaustive only (option "nodes_per_thread" = 2 or 4): a CTA of 1024/NPT threads covers the same four 256-node
 // tiles as prefix_kernel<1>, thread t holding nodes t, t + 1024/NPT, ... of the work item (NPT = 4: two such CTAs per
 // SM).  Same arithmetic per node, so the segment minima (and everything downstream) are bit-identical to the
-// one-node kernel.
+// one-node kernel.  SCREEN (option screen): 0 = MUFU.SQRT per leaf, 1 = the screen loop, 2 = the screen in two stages
+// (prefix_dist_loop_rows first, the screen loop only if a node of the thread passes stage 1; tables that do not fit one
+// chunk as a row table run the flat screen loop as with 1).
 __host__ __device__ constexpr int prefixn_cta(int npt) { return npt == 2 ? MPCB_PN_CTA2 : kPrefixCta / npt; }
 
-template <bool HEAD, int NPT, bool SCREEN = false>
+template <bool HEAD, int NPT, int SCREEN = 0>
 __global__ void __launch_bounds__(prefixn_cta(NPT), NPT / 2) prefixn_kernel(const LaunchArgs a) {
     extern __shared__ float4 s_leaf[];
     constexpr int kCta = prefixn_cta(NPT);
@@ -984,6 +1026,8 @@ __global__ void __launch_bounds__(prefixn_cta(NPT), NPT / 2) prefixn_kernel(cons
     static_assert(kCta * NPT % kThreads == 0, "a work item is a whole number of tiles");
     const unsigned long long qps = (a.tiles_per_solve + groups - 1) / groups;
     const unsigned long long nwork = (unsigned long long)a.N * qps;
+    // SCREEN == 2: nodes that passed stage 1 (statistics), added to the global counter once per warp after the loop
+    unsigned long long stage2_acc = 0;
     for (unsigned long long w = blockIdx.x; w < nwork; w += gridDim.x) {
         const long long n = (long long)(w / qps);
         const unsigned long long tile0 = (w - (unsigned long long)n * qps) * groups;
@@ -1029,12 +1073,29 @@ __global__ void __launch_bounds__(prefixn_cta(NPT), NPT / 2) prefixn_kernel(cons
             }
             const int npairs = rows ? a.g.nv * a.g.ppr : (cn_ + 1) >> 1;
             if (all && SCREEN) {
-                float mx[NPT];
-                if (rows) prefix_screen_loop_rows<HEAD, NPT>(s_leaf, a.g.nv, a.g.ppr, pr, cn, mx);
-                else prefix_screen_loop_far2xN<HEAD, NPT>(s_leaf, npairs, pr, cn, mx);
+                // two stages: the screen loop only runs if stage 1 passes a node of the thread (almost never on the cfg2
+                // bench); it then runs for all of them, and a node stage 1 rejected has no leaf with t^2 - dd > 0 there
+                bool stage2 = true;
+                if (SCREEN == 2 && rows) {
+                    float mdd[NPT];
+                    prefix_dist_loop_rows<NPT>(s_leaf, a.g.nv, a.g.ppr, pr, mdd);
+                    stage2 = false;
 #pragma unroll
-                for (int k = 0; k < NPT; ++k)       // some leaf of the node has t^2 - dd > 0: it may matter
-                    if (mx[k] > 0.f) { best[k] = prefix_min_loop_far2<HEAD>(s_leaf, npairs, pr[k], best[k]); hit[k] = true; }
+                    for (int k = 0; k < NPT; ++k) {
+                        const float tmax = screen_stage1_tmax(a.g.sbox, HEAD, cn[k], pr[k].nu, pr[k].nw, pr[k].eh, pr[k].nhh);
+                        const bool pass = screen_stage1_pass(tmax, mdd[k]);
+                        stage2 = stage2 || pass;
+                        stage2_acc += pass ? 1u : 0u;
+                    }
+                }
+                if (stage2) {
+                    float mx[NPT];
+                    if (rows) prefix_screen_loop_rows<HEAD, NPT>(s_leaf, a.g.nv, a.g.ppr, pr, cn, mx);
+                    else prefix_screen_loop_far2xN<HEAD, NPT>(s_leaf, npairs, pr, cn, mx);
+#pragma unroll
+                    for (int k = 0; k < NPT; ++k)       // some leaf of the node has t^2 - dd > 0: it may matter
+                        if (mx[k] > 0.f) { best[k] = prefix_min_loop_far2<HEAD>(s_leaf, npairs, pr[k], best[k]); hit[k] = true; }
+                }
             } else if (all) {
                 prefix_min_loop_far2xN<HEAD, NPT>(s_leaf, npairs, pr, best);
             } else {
@@ -1067,6 +1128,11 @@ __global__ void __launch_bounds__(prefixn_cta(NPT), NPT / 2) prefixn_kernel(cons
             const double v = active[k] ? base[k] + (double)best[k] : INFINITY;
             publish_segmin(a, seg[k], (!SCREEN || v <= ubw) ? v : INFINITY);
         }
+    }
+    if (SCREEN == 2) {
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) stage2_acc += __shfl_xor_sync(0xffffffffu, stage2_acc, o);
+        if ((tid & 31) == 0 && stage2_acc) atomicAdd(a.counters + 7, stage2_acc);
     }
 }
 
@@ -2004,8 +2070,8 @@ cudaError_t launch_pass(cudaStream_t st, const LaunchArgs &a, int pass, bool pre
 #define MPCB_PN(NPT_, SCR_)                                                                                      \
     (head ? launch_persistent(prefixn_kernel<true, NPT_, SCR_>, a, pass, sm, sms, st, prefixn_cta(NPT_))         \
           : launch_persistent(prefixn_kernel<false, NPT_, SCR_>, a, pass, sm, sms, st, prefixn_cta(NPT_)))
-        if (pass == 1 && a.npt == 4) return a.screen ? MPCB_PN(4, true) : MPCB_PN(4, false);
-        if (pass == 1 && a.npt == 2) return a.screen ? MPCB_PN(2, true) : MPCB_PN(2, false);
+        if (pass == 1 && a.npt == 4) return a.screen == 2 ? MPCB_PN(4, 2) : a.screen ? MPCB_PN(4, 1) : MPCB_PN(4, 0);
+        if (pass == 1 && a.npt == 2) return a.screen == 2 ? MPCB_PN(2, 2) : a.screen ? MPCB_PN(2, 1) : MPCB_PN(2, 0);
 #undef MPCB_PN
         if (pass == 1)
             return head ? launch_persistent(prefix_kernel<1, true>, a, pass, sm, sms, st, kPrefixCta)

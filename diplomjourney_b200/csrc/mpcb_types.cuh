@@ -10,6 +10,7 @@
 #include <cuda_runtime.h>
 
 #include "../../include/mpcb200.h"
+#include "mpcb_screen.cuh"
 
 namespace mpcb {
 
@@ -137,6 +138,7 @@ struct GridTables {
     double dt;
     double smax, dphimax;       // max |s_c|, max |dphi_c| (both variants) -- error model, pruning bounds
     double smin;                // min s_c (both variants) -- pruning bounds
+    ScreenBox sbox;             // range of leaf32's a, b, g: the intervals of stage 1 of the two-stage screen (mpcb_screen.cuh)
 };
 
 // Per solve (float64). Built by prep_kernel from the raw inputs.
@@ -203,11 +205,13 @@ struct LaunchArgs {
     double *bestJ;                         // [N] exact cost of the best candidate so far
     long long *bestIdx;                    // [N]
     int *lock;                             // [N]
-    unsigned long long *counters;          // [0] refine segments, [1] candidates, [2] pruned depth-(H-1) nodes, [3] same, frontier descent (added to [2] when the descent completes)
+    unsigned long long *counters;          // [0] refine segments, [1] candidates, [2] pruned depth-(H-1) nodes, [3] same, frontier descent (added to [2] when the descent completes),
+                                           // [7] nodes that passed stage 1 of the two-stage screen ([4..6] are other fields of the same buffer)
     unsigned long long *ub;                // [N] ordered key of an upper bound on each solve's minimal J_rel (pruning), or null
     int prune;
     int prefilter;                         // pruned pass 1: fp32 pre-filter of the node bound (mpcb_bounds.cuh)
-    int screen;                            // exhaustive prefix pass 1: 0 = MUFU.SQRT per leaf, 1 = screened (sqrt only on nodes that can matter)
+    int screen;                            // exhaustive prefix pass 1: 0 = MUFU.SQRT per leaf, 1 = screened (sqrt only on nodes that can matter),
+                                           // 2 = screened in two stages (distance first, mpcb_screen.cuh)
     float bc32[7];                         // smax, smin, dphimax, cosk[0], sink[0], cosk[1], sink[1] rounded to float (fp32 pre-filter)
     double cosk[kMaxH], sink[kMaxH];       // cos / sin of (i+1) dphi_max: the heading range reachable in i+1 steps (cos = -2: the whole circle)
     // subtree cut (pruned pass 1, H >= 3): tiles that survived the depth-(H-2) bound, as global tile numbers

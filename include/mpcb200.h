@@ -103,12 +103,15 @@ MPCB_API int mpcb_set_grid(mpcb_handle *h, const double *v, int nv, const double
  * each node, and only the children of the depth-(H-2) survivors are ever set up; the call then synchronises the stream
  * once to read whether a frontier outgrew "frontier_cap" entries (default 2^22), in which case mode 1 redoes pass 1.
  * 2, default: mode 3 for trees of more than 2^23 tiles per call, mode 1 otherwise.  0: node-level cut only),
- * "screen" (exhaustive prefix pass 1, i.e. prune = 0; identical results.  1, default: every leaf's cost terms -- scaled
+ * "screen" (exhaustive prefix pass 1, i.e. prune = 0; identical results.  1: every leaf's cost terms -- scaled
  * squared distance dd, line offset q, heading offset gg -- are formed, but the MUFU.SQRT that turns them into the value
  * sqrt(dd) + q^2 + gg^2 is only spent in nodes holding a leaf that can still matter: with cn the largest value a leaf
  * of the node may have and still beat the solve's upper bound (an exact probe of the S held sequences, tightened by
  * every node that found something), a leaf matters iff t = cn - q^2 - gg^2 > 0 and fma(t, t, -dd) > 0; such nodes are
- * re-run with the square roots.  0: one MUFU.SQRT per leaf, no upper bound involved),
+ * re-run with the square roots.  2, default: the same screen in two stages -- every leaf's dd first, with a per-node
+ * bound on q^2 + gg^2 in place of the leaf's own terms; only the nodes that pass go through the screen of 1, and the
+ * nodes the screen flags are exactly those of 1 (grids whose row table does not fit one shared-memory chunk run 1).
+ * 0: one MUFU.SQRT per leaf, no upper bound involved),
  * "prefilter" (1, default; identical results: in the pruned pass 1 a node's bound is first evaluated in fp32 from an fp32
  * walk and the node dropped if that exceeds the upper bound by a margin of 8 error bounds -- which the float64 test would
  * do as well -- so that the float64 set-up is only paid by nodes near the bound; 0 = float64 test for every node),
@@ -181,6 +184,8 @@ typedef struct {
     int64_t pruned_units;     /* depth-(H-1) nodes (x N solves) skipped by the exact branch-and-bound */
     int32_t algo;             /* MPCB_ALGO_* actually used */
     int32_t kernel_launches;  /* kernels enqueued by the last solve */
+    int64_t stage2_units;     /* depth-(H-1) nodes (x N solves) that passed stage 1 of the two-stage screen ("screen" 2, row
+                                 table), i.e. whose line and heading terms were formed leaf by leaf; 0 otherwise */
 } mpcb_stats;
 MPCB_API int mpcb_get_stats(mpcb_handle *h, mpcb_stats *out);
 
