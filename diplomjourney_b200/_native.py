@@ -8,6 +8,7 @@ from __future__ import annotations
 
 import ctypes as C
 import math
+import operator
 import os
 
 import numpy as np
@@ -103,6 +104,9 @@ def load():
     lib.mpcb_held_closed_loop_device.argtypes = loop
     lib.mpcb_held_closed_loop_events_host.argtypes = loop[:8] + [vp, C.c_int32, C.c_double] + loop[8:] + [vp]
     lib.mpcb_held_closed_loop_actual_host.argtypes = loop[:8] + [vp, C.c_int32, C.c_double, vp] + loop[8:] + [vp]
+    lib.mpcb_held_closed_loop_actual_device.argtypes = lib.mpcb_held_closed_loop_actual_host.argtypes
+    lib.mpcb_held_closed_loop_seeded_host.argtypes = loop[:8] + [vp, C.c_int32, C.c_double, vp, C.c_int32, vp] + loop[8:] + [vp]
+    lib.mpcb_rng_seed_device.argtypes = [vp, C.c_int64, vp, C.c_int32, vp]
     lib.mpcb_held_tick_host.argtypes = [vp, vp, C.c_int, vp, C.c_int, C.c_double, C.c_double, C.c_double, C.c_int, C.c_int,
                                         vp, vp, vp, C.c_double, C.c_int, vp, vp, vp, vp]
     win = [vp, C.POINTER(LoopParams), C.c_int64, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
@@ -129,6 +133,53 @@ def _arr(a, dtype, shape=None):
 
 def _ptr(a):
     return None if a is None else a.ctypes.data_as(C.c_void_p)
+
+
+MAX_KEY_LEN = 4096
+_SEED_RANGE = "Seed must be between 0 and 2**32 - 1"
+
+
+def seed_keys(seeds, n):
+    """numpy's legacy seeds of ``n`` generators in the form mpcb_rng_seed_device takes them.  ``seeds`` [n] holds one
+    integer seed per generator, as RandomState(seeds[i]); [n][K] holds one key of K words per generator, as
+    RandomState(list(seeds[i])) -- also for K == 1 (numpy squeezes a one-element *array* to an integer seed, but
+    RandomState(5) and RandomState([5]) are different streams, and here the shape decides).  Returns
+    (uint32 array, key_len), key_len = 0 for integer seeds.  Raises numpy's errors for what RandomState would refuse."""
+    try:
+        a = np.asarray(seeds)
+    except ValueError:
+        raise ValueError("seeds must be [N] integer seeds or [N][K] keys of one length K") from None
+    if a.ndim not in (1, 2):
+        raise ValueError(f"seeds must be [N] integer seeds or [N][K] keys (each key 1-d), got shape {a.shape}")
+    if a.shape[0] != n:
+        raise ValueError(f"seeds holds {a.shape[0]} rows for {n} robots")
+    if a.ndim == 2 and a.shape[1] == 0 and n:
+        raise ValueError("Seed must be non-empty")
+    if a.ndim == 2 and a.shape[1] > MAX_KEY_LEN:
+        raise ValueError(f"keys of {a.shape[1]} words: at most {MAX_KEY_LEN} per generator")
+    if a.size and a.dtype == object:
+        try:
+            vals = [operator.index(x) for x in a.ravel()]
+        except TypeError:
+            raise TypeError("seeds must be integers") from None
+        if any(v < 0 or v > 0xFFFFFFFF for v in vals):
+            raise ValueError(_SEED_RANGE)
+        a = np.array(vals, np.int64).reshape(a.shape)
+    elif a.size and a.dtype.kind not in "iu":
+        raise TypeError(f"seeds must be integers, not {a.dtype}")
+    if a.size and (a.min() < 0 or a.max() > 0xFFFFFFFF):
+        raise ValueError(_SEED_RANGE)
+    return np.ascontiguousarray(a, dtype=np.uint32), (a.shape[1] if a.ndim == 2 else 0)
+
+
+def _event_script(events):
+    """(mpcb_loop_event array or None, count) of a script [(tick, kind, a, b), ...]."""
+    if not events:
+        return None, 0
+    ev = (LoopEvent * len(events))()
+    for i, (tick, kind, a, b) in enumerate(events):
+        ev[i] = LoopEvent(int(tick), int(kind), float(a), float(b))
+    return ev, len(events)
 
 
 class Solver:
@@ -294,15 +345,18 @@ class Solver:
         return dict(cost=cost_o, index=idx_o, traj=traj_o, first_control=ctl_o, shape=shape_o)
 
     def held_closed_loop(self, params: "LoopParams", init, target, origin, first_threshold=None, slow_steps=None,
-                         events=None, radius_u_turn=0.0, rng_state=None):
+                         events=None, radius_u_turn=0.0, rng_state=None, seeds=None, return_rng_state=True):
         """Whole closed loops of the online controller for a batch of robots on the device
         (mpcb_held_closed_loop_host / _events_host). ``events``: an operator script [(tick, kind, a, b), ...] with kind
         EVENT_NEW_TARGET (a, b = the new target) or EVENT_TURN_LEFT / _RIGHT (a = distance), applied to every robot
         after the tick it names; ``radius_u_turn`` = L / sin(beta_max) for the turns.
         ``rng_state`` [N][625] uint32 (per robot numpy RandomState key[624] + pos): the "actual" run with actuator noise
         (mpcb_held_closed_loop_actual_host); the input is not modified.
+        ``seeds`` [N] integer seeds or [N][K] keys (see ``seed_keys``): the actual run with the generators of
+        RandomState(seeds[i]), seeded on the device (mpcb_held_closed_loop_seeded_host); not together with
+        ``rng_state``.  ``return_rng_state=False`` leaves the seeded generators' final states on the device.
         Returns dict(log[N,max_ticks,5], ticks[N], status[N], final[N,6] = x_t, y_t, x_0, y_0, steps_for_slowing, m),
-        with ``rng_state`` also the generators' states after the run."""
+        with ``rng_state`` or ``seeds`` also the generators' states after the run."""
         ini = _arr(init, np.float64, (-1, 5))
         N = ini.shape[0]
         tg = _arr(np.broadcast_to(np.asarray(target, np.float64).reshape(-1, 2), (N, 2)), np.float64)
@@ -312,24 +366,56 @@ class Solver:
         log = np.full((N, params.max_ticks, 5), np.nan)
         ticks = np.empty(N, np.int32)
         status = np.empty(N, np.int32)
-        ev = (LoopEvent * max(1, len(events or ())))()
-        for i, (tick, kind, a, b) in enumerate(events or ()):
-            ev[i] = LoopEvent(int(tick), int(kind), float(a), float(b))
+        ev, n_ev = _event_script(events)
         final = np.empty((N, 6))
+        if seeds is not None:
+            if rng_state is not None:
+                raise ValueError("seeds and rng_state both give the generators: pass one of them")
+            keys, key_len = seed_keys(seeds, N)
+            rs = np.empty((N, 625), np.uint32) if return_rng_state else None
+            self._ck(self.lib.mpcb_held_closed_loop_seeded_host(self.h, C.byref(params), N, _ptr(ini), _ptr(tg), _ptr(og),
+                                                                _ptr(thr), _ptr(sl), ev, n_ev, float(radius_u_turn),
+                                                                _ptr(keys), key_len, _ptr(rs), _ptr(log), _ptr(ticks),
+                                                                _ptr(status), _ptr(final)))
+            out = dict(log=log, ticks=ticks, status=status, final=final)
+            if return_rng_state:
+                out["rng_state"] = rs
+            return out
         if rng_state is None:
             self._ck(self.lib.mpcb_held_closed_loop_events_host(self.h, C.byref(params), N, _ptr(ini), _ptr(tg), _ptr(og),
-                                                                _ptr(thr), _ptr(sl), ev if events else None,
-                                                                len(events or ()), float(radius_u_turn), _ptr(log),
-                                                                _ptr(ticks), _ptr(status), _ptr(final)))
+                                                                _ptr(thr), _ptr(sl), ev, n_ev, float(radius_u_turn),
+                                                                _ptr(log), _ptr(ticks), _ptr(status), _ptr(final)))
             return dict(log=log, ticks=ticks, status=status, final=final)
         rs = np.array(rng_state, dtype=np.uint32, order="C")         # a copy: the library updates it in place
         if rs.shape != (N, 625):
             raise ValueError(f"rng_state must be [N][625] = [{N}][625] (key[624] + pos per robot), got {rs.shape}")
         self._ck(self.lib.mpcb_held_closed_loop_actual_host(self.h, C.byref(params), N, _ptr(ini), _ptr(tg), _ptr(og),
-                                                            _ptr(thr), _ptr(sl), ev if events else None,
-                                                            len(events or ()), float(radius_u_turn), _ptr(rs), _ptr(log),
-                                                            _ptr(ticks), _ptr(status), _ptr(final)))
+                                                            _ptr(thr), _ptr(sl), ev, n_ev, float(radius_u_turn),
+                                                            _ptr(rs), _ptr(log), _ptr(ticks), _ptr(status), _ptr(final)))
         return dict(log=log, ticks=ticks, status=status, final=final, rng_state=rs)
+
+    def seed_generators_device(self, N, keys, key_len, out):
+        """mpcb_rng_seed_device: the [N][625] records (key[624] + pos) of RandomState(keys[n]) (key_len == 0, keys[N]
+        uint32) or RandomState(keys[n, :]) (keys[N][key_len] uint32), written to ``out``.  Raw device addresses (e.g.
+        torch.Tensor.data_ptr()); enqueues on self.stream, does not synchronise."""
+        vp = lambda x: C.c_void_p(int(x)) if x else None
+        self._ck(self.lib.mpcb_rng_seed_device(self.h, int(N), vp(keys), int(key_len), vp(out)))
+
+    def held_closed_loop_device_actual(self, params: "LoopParams", N, init, target, origin, first_threshold, slow_steps,
+                                       rng_state, out_log, out_ticks, out_status, out_final=None, events=None,
+                                       radius_u_turn=0.0):
+        """mpcb_held_closed_loop_actual_device: the actual run of ``held_closed_loop`` on raw device addresses (init
+        [N][5], target / origin [N][2] float64, first_threshold [N] float64 or 0, slow_steps [N] int32 or 0, rng_state
+        [N][625] uint32 updated in place, out_log [N][max_ticks][5], out_ticks / out_status [N] int32, out_final [N][6]
+        or 0); ``events`` is a host script as for ``held_closed_loop``.  Rows of out_log after a robot's last tick are
+        not written: fill it (with NaN, as the host entry does) beforehand.  Enqueues on self.stream, does not
+        synchronise."""
+        vp = lambda x: C.c_void_p(int(x)) if x else None
+        ev, n_ev = _event_script(events)
+        self._ck(self.lib.mpcb_held_closed_loop_actual_device(self.h, C.byref(params), int(N), vp(init), vp(target),
+                                                              vp(origin), vp(first_threshold), vp(slow_steps), ev, n_ev,
+                                                              float(radius_u_turn), vp(rng_state), vp(out_log),
+                                                              vp(out_ticks), vp(out_status), vp(out_final)))
 
     def full_closed_loop(self, cost, H, init_state, target, origin, first_threshold=None, eps=0.001, max_ticks=256):
         """Closed loop of the FULL-tree scripts for a batch of robots (mpcb_full_closed_loop_host): one batched

@@ -36,6 +36,7 @@ cudaError_t launch_refine_scan(cudaStream_t, const LaunchArgs &, int sms);
 cudaError_t launch_finalize(cudaStream_t, const LaunchArgs &, double *, long long *, double *, double *);
 cudaError_t launch_dump(cudaStream_t, const LaunchArgs &, bool prefix, double *jrel, int sms);
 cudaError_t launch_held_loop(cudaStream_t, const LoopArgs &, int sms);
+cudaError_t launch_rng_seed(cudaStream_t, long long N, const unsigned *keys, int key_len, unsigned *rng_state);
 cudaError_t launch_held_small(cudaStream_t, const SmallArgs &);
 cudaError_t launch_full_apply(cudaStream_t, const FullLoopArgs &);
 cudaError_t launch_held_windows(cudaStream_t, const WindowArgs &, int sms);
@@ -288,7 +289,7 @@ int mpcb_destroy(mpcb_handle *h) {
                       &h->ctl32_slow, &h->sp, &h->segmin, &h->worklist, &h->misc, &h->tau, &h->bestJ, &h->bestIdx,
                       &h->lock, &h->ub, &h->tile_list, &h->reduce_scratch, &h->in_state, &h->in_target, &h->in_origin, &h->in_thr, &h->in_flags, &h->out_cost,
                       &h->out_index, &h->out_traj, &h->out_ctl, &h->dump_rec, &h->dump_j, &h->loop_log, &h->loop_ticks,
-                      &h->loop_status, &h->loop_events, &h->loop_final, &h->loop_rng, &h->small_in, &h->small_out, &h->fl_last, &h->fl_k, &h->fl_have, &h->fl_flags,
+                      &h->loop_status, &h->loop_events, &h->loop_final, &h->loop_rng, &h->loop_keys, &h->small_in, &h->small_out, &h->fl_last, &h->fl_k, &h->fl_have, &h->fl_flags,
                       &h->fl_count, &h->nccl_scratch, &h->cand, &h->cand_J, &h->cand_sel, &h->node_list})
         b->release();
     if (h->pin_in) cudaFreeHost(h->pin_in);
@@ -812,7 +813,26 @@ int mpcb_dump_leaves_host(mpcb_handle *h, int mode, int cost_kind, int H, int al
     return MPCB_OK;
 }
 
-// device pointers throughout; events / out_final / rng_state may be null
+// a closed loop's operator-event script (host memory: it is configuration, like the loop parameters)
+static int check_events(mpcb_handle *h, const mpcb_loop_event *events, int32_t n_events) {
+    if (n_events < 0 || n_events > 4096 || (n_events > 0 && !events))
+        return fail(h, MPCB_ERR_INVALID, "closed loop: bad event script (n_events=%d)", n_events);
+    for (int e = 0; e < n_events; ++e)
+        if (events[e].kind < MPCB_EVENT_NEW_TARGET || events[e].kind > MPCB_EVENT_TURN_RIGHT)
+            return fail(h, MPCB_ERR_INVALID, "closed loop: event %d has unknown kind %d", e, events[e].kind);
+    return MPCB_OK;
+}
+
+// numpy seeds of N generators: keys[N] integer seeds (key_len 0) or keys[N][key_len] (1 <= key_len <= 4096)
+static int check_seed_keys(mpcb_handle *h, int64_t N, const uint32_t *keys, int32_t key_len) {
+    if (N < 0 || N >= (1LL << 31)) return fail(h, MPCB_ERR_INVALID, "N out of range");
+    if (key_len < 0 || key_len > 4096) return fail(h, MPCB_ERR_INVALID, "seeding: key_len %d outside [0, 4096]", key_len);
+    if (N > 0 && !keys) return fail(h, MPCB_ERR_INVALID, "seeding: null keys");
+    return MPCB_OK;
+}
+
+// device pointers throughout, except the event script (checked by the caller with check_events), which is copied into
+// handle scratch here; events / out_final / rng_state may be null
 static int held_loop_core(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, const double *init,
                           const double *target, const double *origin, const double *first_threshold,
                           const int32_t *slow_steps, const mpcb_loop_event *events, int n_events, double radius_u_turn,
@@ -827,11 +847,17 @@ static int held_loop_core(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, 
         return fail(h, MPCB_ERR_INVALID, "closed loop: bad parameters (H=%d, max_ticks=%d, n_v=%d, n_beta=%d)", p->H,
                     p->max_ticks, p->n_v, p->n_beta);
     CK(cudaSetDevice(h->device));
+    const mpcb_loop_event *d_events = nullptr;
+    if (events && n_events > 0) {
+        CK(h->loop_events.ensure(sizeof(mpcb_loop_event) * n_events));
+        CK(cudaMemcpyAsync(h->loop_events.p, events, sizeof(mpcb_loop_event) * n_events, cudaMemcpyHostToDevice, h->stream));
+        d_events = h->loop_events.as<mpcb_loop_event>();
+    }
     LoopArgs a;
     a.p = *p; a.N = N;
     a.init = init; a.target = target; a.origin = origin; a.first_threshold = first_threshold;
     a.slow_steps = slow_steps; a.out_log = out_log; a.out_ticks = out_ticks; a.out_status = out_status;
-    a.events = events; a.n_events = events ? n_events : 0; a.radius_u_turn = radius_u_turn; a.out_final = out_final;
+    a.events = d_events; a.n_events = d_events ? n_events : 0; a.radius_u_turn = radius_u_turn; a.out_final = out_final;
     a.rng_state = rng_state;
     CK(launch_held_loop(h->stream, a, h->sms));
     h->stats = mpcb_stats{};
@@ -854,16 +880,16 @@ int mpcb_held_closed_loop_host(mpcb_handle *h, const mpcb_loop_params *p, int64_
                                              out_log, out_ticks, out_status, nullptr);
 }
 
-// host pointers; rng_state null = the noise-free loop
+// host pointers.  The actual run's generators are copied in from rng_in[N][625] or seeded on the device from keys
+// (key_len as for mpcb_rng_seed_device); with neither, the loop is the noise-free one.  rng_out[N][625] (nullable)
+// receives the generators' states after the run.
 static int held_loop_host(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, const double *init, const double *target,
                           const double *origin, const double *first_threshold, const int32_t *slow_steps,
-                          const mpcb_loop_event *events, int32_t n_events, double radius_u_turn, uint32_t *rng_state,
-                          double *out_log, int32_t *out_ticks, int32_t *out_status, double *out_final) {
-    if (n_events < 0 || n_events > 4096 || (n_events > 0 && !events))
-        return fail(h, MPCB_ERR_INVALID, "closed loop: bad event script (n_events=%d)", n_events);
-    for (int e = 0; e < n_events; ++e)
-        if (events[e].kind < MPCB_EVENT_NEW_TARGET || events[e].kind > MPCB_EVENT_TURN_RIGHT)
-            return fail(h, MPCB_ERR_INVALID, "closed loop: event %d has unknown kind %d", e, events[e].kind);
+                          const mpcb_loop_event *events, int32_t n_events, double radius_u_turn, const uint32_t *rng_in,
+                          const uint32_t *keys, int32_t key_len, uint32_t *rng_out, double *out_log, int32_t *out_ticks,
+                          int32_t *out_status, double *out_final) {
+    int rc = check_events(h, events, n_events);
+    if (rc) return rc;
     if (N <= 0) return N == 0 ? MPCB_OK : fail(h, MPCB_ERR_INVALID, "N < 0");
     if (!init || !target || !origin || !out_log || !out_ticks || !out_status)
         return fail(h, MPCB_ERR_INVALID, "closed loop: null pointer");
@@ -892,25 +918,25 @@ static int held_loop_host(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, 
         CK(cudaMemcpyAsync(h->in_flags.p, slow_steps, sizeof(int) * N, cudaMemcpyHostToDevice, st));
         d_slow = h->in_flags.as<int>();
     }
-    const mpcb_loop_event *d_events = nullptr;
-    if (n_events > 0) {
-        CK(h->loop_events.ensure(sizeof(mpcb_loop_event) * n_events));
-        CK(cudaMemcpyAsync(h->loop_events.p, events, sizeof(mpcb_loop_event) * n_events, cudaMemcpyHostToDevice, st));
-        d_events = h->loop_events.as<mpcb_loop_event>();
-    }
     const size_t nrng = (size_t)N * mpcb::kMtWords;
-    if (rng_state) {
-        CK(h->loop_rng.ensure(sizeof(uint32_t) * nrng));
-        CK(cudaMemcpyAsync(h->loop_rng.p, rng_state, sizeof(uint32_t) * nrng, cudaMemcpyHostToDevice, st));
+    const bool noise = rng_in || keys;
+    if (noise) CK(h->loop_rng.ensure(sizeof(uint32_t) * nrng));
+    if (rng_in) CK(cudaMemcpyAsync(h->loop_rng.p, rng_in, sizeof(uint32_t) * nrng, cudaMemcpyHostToDevice, st));
+    if (keys) {
+        const size_t nkeys = (size_t)N * (key_len ? key_len : 1);
+        CK(h->loop_keys.ensure(sizeof(uint32_t) * nkeys));
+        CK(cudaMemcpyAsync(h->loop_keys.p, keys, sizeof(uint32_t) * nkeys, cudaMemcpyHostToDevice, st));
+        CK(launch_rng_seed(st, N, h->loop_keys.as<unsigned>(), key_len, h->loop_rng.as<unsigned>()));
     }
     if (out_final) CK(h->loop_final.ensure(sizeof(double) * 6 * N));
     CK(cudaMemsetAsync(h->loop_log.p, 0xFF, sizeof(double) * nlog, st));     // NaN pattern for the rows no tick wrote
-    int rc = held_loop_core(h, p, N, h->in_state.as<double>(), h->in_target.as<double>(), h->in_origin.as<double>(), d_thr,
-                            d_slow, d_events, n_events, radius_u_turn, rng_state ? h->loop_rng.as<uint32_t>() : nullptr,
-                            h->loop_log.as<double>(), h->loop_ticks.as<int>(), h->loop_status.as<int>(),
-                            out_final ? h->loop_final.as<double>() : nullptr);
+    rc = held_loop_core(h, p, N, h->in_state.as<double>(), h->in_target.as<double>(), h->in_origin.as<double>(), d_thr,
+                        d_slow, events, n_events, radius_u_turn, noise ? h->loop_rng.as<uint32_t>() : nullptr,
+                        h->loop_log.as<double>(), h->loop_ticks.as<int>(), h->loop_status.as<int>(),
+                        out_final ? h->loop_final.as<double>() : nullptr);
     if (rc) return rc;
-    if (rng_state) CK(cudaMemcpyAsync(rng_state, h->loop_rng.p, sizeof(uint32_t) * nrng, cudaMemcpyDeviceToHost, st));
+    if (keys) h->stats.kernel_launches += 1;     // the seeding kernel
+    if (rng_out) CK(cudaMemcpyAsync(rng_out, h->loop_rng.p, sizeof(uint32_t) * nrng, cudaMemcpyDeviceToHost, st));
     if (out_final) CK(cudaMemcpyAsync(out_final, h->loop_final.p, sizeof(double) * 6 * N, cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(out_log, h->loop_log.p, sizeof(double) * nlog, cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(out_ticks, h->loop_ticks.p, sizeof(int) * N, cudaMemcpyDeviceToHost, st));
@@ -926,7 +952,7 @@ int mpcb_held_closed_loop_events_host(mpcb_handle *h, const mpcb_loop_params *p,
                                       double *out_final) {
     if (!h || !p) return MPCB_ERR_INVALID;
     return held_loop_host(h, p, N, init, target, origin, first_threshold, slow_steps, events, n_events, radius_u_turn,
-                          nullptr, out_log, out_ticks, out_status, out_final);
+                          nullptr, nullptr, 0, nullptr, out_log, out_ticks, out_status, out_final);
 }
 
 int mpcb_held_closed_loop_actual_host(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, const double *init,
@@ -943,7 +969,44 @@ int mpcb_held_closed_loop_actual_host(mpcb_handle *h, const mpcb_loop_params *p,
                         (long long)n, pos);
     }
     return held_loop_host(h, p, N, init, target, origin, first_threshold, slow_steps, events, n_events, radius_u_turn,
+                          rng_state, nullptr, 0, rng_state, out_log, out_ticks, out_status, out_final);
+}
+
+int mpcb_held_closed_loop_actual_device(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, const double *init,
+                                        const double *target, const double *origin, const double *first_threshold,
+                                        const int32_t *slow_steps, const mpcb_loop_event *events, int32_t n_events,
+                                        double radius_u_turn, uint32_t *rng_state, double *out_log, int32_t *out_ticks,
+                                        int32_t *out_status, double *out_final) {
+    if (!h || !p) return MPCB_ERR_INVALID;
+    int rc = check_events(h, events, n_events);
+    if (rc) return rc;
+    if (!rng_state) return fail(h, MPCB_ERR_INVALID, "actual closed loop: null rng_state");
+    return held_loop_core(h, p, N, init, target, origin, first_threshold, slow_steps, events, n_events, radius_u_turn,
                           rng_state, out_log, out_ticks, out_status, out_final);
+}
+
+int mpcb_held_closed_loop_seeded_host(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, const double *init,
+                                      const double *target, const double *origin, const double *first_threshold,
+                                      const int32_t *slow_steps, const mpcb_loop_event *events, int32_t n_events,
+                                      double radius_u_turn, const uint32_t *keys, int32_t key_len,
+                                      uint32_t *rng_state_out, double *out_log, int32_t *out_ticks, int32_t *out_status,
+                                      double *out_final) {
+    if (!h || !p) return MPCB_ERR_INVALID;
+    int rc = check_seed_keys(h, N, keys, key_len);
+    if (rc) return rc;
+    return held_loop_host(h, p, N, init, target, origin, first_threshold, slow_steps, events, n_events, radius_u_turn,
+                          nullptr, keys, key_len, rng_state_out, out_log, out_ticks, out_status, out_final);
+}
+
+int mpcb_rng_seed_device(mpcb_handle *h, int64_t N, const uint32_t *keys, int32_t key_len, uint32_t *rng_state) {
+    if (!h) return MPCB_ERR_INVALID;
+    int rc = check_seed_keys(h, N, keys, key_len);
+    if (rc) return rc;
+    if (N == 0) return MPCB_OK;
+    if (!rng_state) return fail(h, MPCB_ERR_INVALID, "seeding: null rng_state");
+    CK(cudaSetDevice(h->device));
+    CK(launch_rng_seed(h->stream, N, keys, key_len, rng_state));
+    return MPCB_OK;
 }
 
 static int check_window_params(mpcb_handle *h, const mpcb_loop_params *p) {

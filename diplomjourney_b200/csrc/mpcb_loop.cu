@@ -14,6 +14,7 @@
 // The "actual" run (math_mpc(..., True)) gives every robot its own numpy RandomState (key[624] + pos, mpcb_noise.cuh):
 // the CTA keeps it in shared memory while it runs the robot, and thread 0 perturbs the applied (v, beta) after every
 // tick, draw for draw as the reference does.  A template flag keeps the noise-free loop free of all of it.
+// rng_seed_kernel builds those generators on the device from numpy's integer seeds or keys.
 //
 // A HELD tick is tiny (S <= 451 candidates x H steps), so the loop is latency-bound, not
 // throughput-bound: everything is evaluated directly in float64 with the reference's formula and
@@ -280,6 +281,22 @@ __global__ void __launch_bounds__(kLoopThreads) held_loop_kernel(const LoopArgs 
         if constexpr (kNoise)       // thread 0's last draw came before the barrier that ended the loop
             for (int i = tid; i < kMtWords; i += kLoopThreads) a.rng_state[(size_t)n * kMtWords + i] = s_mt[i];
     }
+}
+
+// The generators of the actual run, seeded as numpy's RandomState(keys[n]) (key_len == 0) or RandomState(keys[n, :])
+// (keys[N][key_len]): one thread per generator writes its [625] record straight to global memory -- the recurrences
+// are serial, so there is nothing to split inside a generator.
+__global__ void __launch_bounds__(128) rng_seed_kernel(long long N, const unsigned *keys, int key_len, unsigned *rng_state) {
+    const long long n = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (n >= N) return;
+    unsigned *st = rng_state + (size_t)n * kMtWords;
+    if (key_len == 0) mt_seed(st, keys[n]);
+    else mt_seed_by_array(st, keys + (size_t)n * key_len, key_len);
+}
+
+cudaError_t launch_rng_seed(cudaStream_t st, long long N, const unsigned *keys, int key_len, unsigned *rng_state) {
+    rng_seed_kernel<<<(unsigned)((N + 127) / 128), 128, 0, st>>>(N, keys, key_len, rng_state);
+    return cudaGetLastError();
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -4,7 +4,8 @@
 // (tests/test_noise_on_host.py).
 //
 // Generator state = what RandomState.get_state() hands out: st[0..623] = key, st[624] = pos (624 right after seeding,
-// so the first draw twists).  Nothing is seeded here: any state, mid-stream ones included, continues where it stands.
+// so the first draw twists).  The draws continue any state where it stands, mid-stream ones included; mt_seed and
+// mt_seed_by_array build the state RandomState(int) and RandomState(array) start from (tests/test_seed_on_host.py).
 #pragma once
 #include "mpcb_types.cuh"
 
@@ -19,6 +20,34 @@ MPCB_HD double ddiv(double a, double b) {
 #else
     return a / b;
 #endif
+}
+
+// RandomState(s) / np.random.seed(s): numpy's mt19937_seed, all arithmetic mod 2^32
+MPCB_HD void mt_seed(unsigned *st, unsigned s) {
+    for (int i = 0; i < kMtN; ++i) {
+        st[i] = s;
+        s = 1812433253u * (s ^ (s >> 30)) + (unsigned)i + 1u;
+    }
+    st[kMtN] = kMtN;
+}
+
+// RandomState(key) for a 1-D key of K >= 1 words: numpy's mt19937_init_by_array.  RandomState(5) and RandomState([5])
+// are different streams.  `prev` is mt[i - 1]; on the wrap of i it is mt[623], which is also the new mt[0].
+MPCB_HD void mt_seed_by_array(unsigned *st, const unsigned *key, int K) {
+    mt_seed(st, 19650218u);
+    int i = 1, j = 0;
+    unsigned prev = st[0];
+    for (int k = K > kMtN ? K : kMtN; k > 0; --k) {
+        prev = st[i] = (st[i] ^ ((prev ^ (prev >> 30)) * 1664525u)) + key[j] + (unsigned)j;
+        if (++i >= kMtN) { st[0] = prev; i = 1; }
+        if (++j >= K) j = 0;
+    }
+    for (int k = kMtN - 1; k > 0; --k) {
+        prev = st[i] = (st[i] ^ ((prev ^ (prev >> 30)) * 1566083941u)) - (unsigned)i;
+        if (++i >= kMtN) { st[0] = prev; i = 1; }
+    }
+    st[0] = 0x80000000u;        // the most significant bit set: the state is never all zero
+    st[kMtN] = kMtN;
 }
 
 // the standard MT19937 twist of all 624 words; pos := 0.  Not inlined: it runs once per 312+ draws, and inlined into the

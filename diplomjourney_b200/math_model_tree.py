@@ -477,11 +477,15 @@ def _pack_generators(gens):
     return out
 
 
-def _math_mpc_batch_device_noise(params, ini, tgt, org, first, rngs, events):
+def _math_mpc_batch_device_noise(params, ini, tgt, org, first, rngs, events, seeds=None):
     """The actual run on the device (mpcb_held_closed_loop_actual): each robot draws from its own generator, whose state
-    goes to the device as get_state() and comes back through set_state (has_gauss / cached_gaussian kept)."""
-    gens = [random] if rngs is None else rngs
+    goes to the device as get_state() and comes back through set_state (has_gauss / cached_gaussian kept).  With
+    ``seeds`` (already checked by ``_native.seed_keys``) the generators are seeded on the device and stay there."""
     script = ACTUAL_EVENTS if events is True else list(events or ())
+    if seeds is not None:
+        return _solver().held_closed_loop(params, ini, tgt, org, first_threshold=first, events=script or None,
+                                          radius_u_turn=radius_u_turn, seeds=seeds, return_rng_state=False)
+    gens = [random] if rngs is None else rngs
     r = _solver().held_closed_loop(params, ini, tgt, org, first_threshold=first, events=script or None,
                                    radius_u_turn=radius_u_turn, rng_state=_pack_generators(gens))
     for g, st in zip(gens, r.pop("rng_state")):
@@ -491,7 +495,7 @@ def _math_mpc_batch_device_noise(params, ini, tgt, org, first, rngs, events):
 
 
 def math_mpc_batch(initial_coordinates, target_coordinates, max_ticks=512, origin=None, cost_kind=None,
-                   isActual=False, rngs=None, events=False, host_loop=False, device_noise=False):
+                   isActual=False, rngs=None, events=False, host_loop=False, device_noise=False, seeds=None):
     """EXTENSION (not in the reference): the closed loop of ``math_mpc`` for a whole batch of robots.
     ``initial_coordinates`` [N][5] = x, y, phi, v, beta; ``target_coordinates`` [N][2].  The tracked line starts at
     the module's x_0, y_0 unless ``origin`` [N][2] is given.
@@ -514,6 +518,11 @@ def math_mpc_batch(initial_coordinates, target_coordinates, max_ticks=512, origi
       which one CTA per robot cannot reproduce.  ``events=True`` is the actual run's script (new_target(2, 3) after tick
       1, then the demo script), or any ``[(tick, kind, a, b), ...]``.  Returns log, ticks, status and final as the
       noise-free device loop does (no ``robots``).
+    * ``isActual=True, device_noise=True, seeds=...`` in place of ``rngs``: robot i draws the stream of
+      ``np.random.RandomState(seeds[i])``, seeded on the device from ``seeds`` [N] (integer seeds) or [N][K] (keys; a
+      row is a key even when K == 1, see ``_native.seed_keys``).  No generator object is built and ``np.random`` is
+      not touched; the generators' final states are not returned (``_native.Solver.held_closed_loop(..., seeds=)``
+      returns them).  Same result keys as with ``rngs``.
 
     Returns dict(log[N][max_ticks][5], ticks[N], status[N])."""
     from . import config as _cfg
@@ -521,16 +530,22 @@ def math_mpc_batch(initial_coordinates, target_coordinates, max_ticks=512, origi
     org = np.array([[x_0, y_0]], dtype=np.float64) if origin is None else np.asarray(origin, np.float64).reshape(-1, 2)
     tgt = np.asarray(target_coordinates, dtype=np.float64).reshape(-1, 2)
     n = ini.shape[0]
+    if seeds is not None:
+        if rngs is not None:
+            raise ValueError("seeds and rngs both give the robots' generators: pass one of them")
+        if not device_noise:
+            raise ValueError("seeds seed the generators on the device: they need isActual=True, device_noise=True")
+        seeds = _native.seed_keys(seeds, n)[0]
     if device_noise:
         if not isActual:
             raise ValueError("device_noise=True is the actual run's actuator noise: it needs isActual=True")
         if host_loop:
             raise ValueError("device_noise=True runs the whole loop on the device; host_loop=True is the per-tick path")
-        if rngs is None:
+        if rngs is None and seeds is None:
             if n != 1:
                 raise ValueError("rngs=None shares the module generator among the robots, which interleaves their draws; "
                                  "pass one numpy RandomState per robot (or run one robot)")
-        else:
+        elif rngs is not None:
             rngs = list(rngs)
             if len(rngs) != n:
                 raise ValueError(f"rngs holds {len(rngs)} generators for {n} robots")
@@ -552,7 +567,7 @@ def math_mpc_batch(initial_coordinates, target_coordinates, max_ticks=512, origi
     params = _native.LoopParams.from_config(_cfg, _native.COST_TREE if cost_kind is None else cost_kind,
                                             prediction_horizon, max_ticks)
     if device_noise:
-        return _math_mpc_batch_device_noise(params, ini, tgt, org, first, rngs, events)
+        return _math_mpc_batch_device_noise(params, ini, tgt, org, first, rngs, events, seeds)
     if isActual or host_loop:
         if not isinstance(events, bool) and events is not None:
             raise ValueError("a custom event script runs on the device loop only (isActual=False, host_loop=False); "

@@ -269,6 +269,35 @@ MPCB_API int mpcb_held_closed_loop_actual_host(mpcb_handle *h, const mpcb_loop_p
                                       const mpcb_loop_event *events, int32_t n_events, double radius_u_turn,
                                       uint32_t *rng_state,
                                       double *out_log, int32_t *out_ticks, int32_t *out_status, double *out_final);
+/* Device flavour of mpcb_held_closed_loop_actual_host: init, target, origin, first_threshold, slow_steps, rng_state
+ * (in/out) and every output are device pointers; the event script stays a host array (configuration, like p: it is
+ * checked as the host entries check it and copied into handle scratch).  Enqueued without a sync.  Rows of out_log after
+ * a robot's last tick are not written: the caller fills out_log beforehand (the host entry fills it with NaN).  pos is
+ * not checked (that would need a copy): any pos >= 624 behaves as 624, because the generator twists before its next
+ * draw (a robot that draws nothing hands its record back unchanged).  A null rng_state is MPCB_ERR_INVALID. */
+MPCB_API int mpcb_held_closed_loop_actual_device(mpcb_handle *h, const mpcb_loop_params *p, int64_t N,
+                                        const double *init, const double *target, const double *origin,
+                                        const double *first_threshold, const int32_t *slow_steps,
+                                        const mpcb_loop_event *events, int32_t n_events, double radius_u_turn,
+                                        uint32_t *rng_state,
+                                        double *out_log, int32_t *out_ticks, int32_t *out_status, double *out_final);
+/* The actual run's generators seeded on the device as numpy seeds them (the legacy RandomState(seed), not numpy's
+ * Generator): rng_state[N][625] receives, per robot, the key[624] + pos (624) RandomState(...).get_state() hands out.
+ *   key_len == 0              keys[N] holds one integer seed per robot: RandomState(keys[n]) (mt19937_seed)
+ *   1 <= key_len <= 4096      keys[N][key_len] holds one key per robot: RandomState(keys[n, :]) (mt19937_init_by_array;
+ *                             RandomState(5) and RandomState([5]) are different streams)
+ * Device pointers, enqueued on the handle's stream without a sync.  Another key_len, N < 0 (or N >= 2^31), or a null
+ * pointer with N > 0 is MPCB_ERR_INVALID; N == 0 launches nothing. */
+MPCB_API int mpcb_rng_seed_device(mpcb_handle *h, int64_t N, const uint32_t *keys, int32_t key_len, uint32_t *rng_state);
+/* mpcb_held_closed_loop_actual_host with the generators seeded on the device from keys / key_len (as for
+ * mpcb_rng_seed_device, host pointer) in place of rng_state: no generator state crosses the bus on the way in.
+ *   rng_state_out[N][625]  (nullable) the generators' states after the run; NULL = they are not copied back */
+MPCB_API int mpcb_held_closed_loop_seeded_host(mpcb_handle *h, const mpcb_loop_params *p, int64_t N,
+                                      const double *init, const double *target, const double *origin,
+                                      const double *first_threshold, const int32_t *slow_steps,
+                                      const mpcb_loop_event *events, int32_t n_events, double radius_u_turn,
+                                      const uint32_t *keys, int32_t key_len, uint32_t *rng_state_out,
+                                      double *out_log, int32_t *out_ticks, int32_t *out_status, double *out_final);
 
 /* ONE online tick for a batch of robots that each have their OWN acceleration window (SURVEY 8f row f2).  The
  * reference rebuilds the control window per robot and per tick around the robot's current (v, beta)
