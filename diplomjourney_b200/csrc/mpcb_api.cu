@@ -20,7 +20,7 @@
 namespace mpcb {
 cudaError_t launch_prep(cudaStream_t, long long, const double *, const double *, const double *, const double *,
                         const uint8_t *, int, int, int, double, double, double, SolveParams *);
-cudaError_t launch_pass(cudaStream_t, const LaunchArgs &, int pass, bool prefix, int sms);
+cudaError_t launch_pass(cudaStream_t, const LaunchArgs &, const RowPairs &, int pass, bool prefix, int sms);
 cudaError_t launch_reduce_compact(cudaStream_t, const LaunchArgs &, double *, unsigned *, unsigned *, int sms);
 cudaError_t launch_reduce_compact_wide(cudaStream_t, const LaunchArgs &, double *, unsigned *, unsigned *, void *scratch,
                                        int sms, int *launches);
@@ -213,6 +213,7 @@ static int ensure_tables(mpcb_handle *h) {
                 const float4 x = l32[iv * nb + 2 * m], y = l32[iv * nb + std::min(2 * m + 1, nb - 1)];
                 l32r[2 * ((size_t)iv * ppr + m)] = make_float4(x.x, y.x, x.y, y.y);
                 l32r[2 * ((size_t)iv * ppr + m) + 1] = make_float4(x.z, y.z, x.w, y.w);
+                h->row_ab.ab[iv * ppr + m] = l32r[2 * ((size_t)iv * ppr + m)];
             }
     CK(h->leaf32r.ensure(sizeof(float4) * std::max<size_t>(l32r.size(), 1)));
     CK(h->leaf32.ensure(sizeof(float4) * S));
@@ -514,7 +515,7 @@ static int solve_core(mpcb_handle *h, int mode, int cost_kind, int H, int64_t N,
             }
             a.q_list = lists + ((H - 3) & 1) * cap;
             a.q_count = q_counts + ((H - 3) & 1);
-            CK(launch_pass(h->stream, a, 1, pl.prefix, h->sms)); ++launches;
+            CK(launch_pass(h->stream, a, h->row_ab, 1, pl.prefix, h->sms)); ++launches;
             a.q_list = nullptr; a.q_count = nullptr; a.gate = 0;
             // a frontier that outgrew its list: the fused tile walk redoes pass 1 -- decided on the device, the kernel
             // returns at once otherwise; the host never reads the flag
@@ -527,12 +528,12 @@ static int solve_core(mpcb_handle *h, int mode, int cost_kind, int H, int64_t N,
             for (unsigned long long g0 = 0; g0 < all; g0 += batch) {
                 if (g0 || frontier) CK(cudaMemsetAsync(tile_count, 0, sizeof(unsigned), h->stream));
                 CK(launch_tilecut(h->stream, a, g0, std::min(all, g0 + batch), lists, tile_count, batch)); ++launches;
-                CK(launch_pass(h->stream, a, 1, pl.prefix, h->sms)); ++launches;
+                CK(launch_pass(h->stream, a, h->row_ab, 1, pl.prefix, h->sms)); ++launches;
             }
             a.tile_list = nullptr; a.tile_count = nullptr;
         }
     } else if (a.total_segs > 0) {
-        CK(launch_pass(h->stream, a, 1, pl.prefix, h->sms)); ++launches;
+        CK(launch_pass(h->stream, a, h->row_ab, 1, pl.prefix, h->sms)); ++launches;
     }
     if (a.segs_per_solve >= kWideReduceSegs) {   // few solves with many segments each: reduce and compact grid-wide
         CK(h->reduce_scratch.ensure(2 * sizeof(double) * N));
@@ -542,7 +543,7 @@ static int solve_core(mpcb_handle *h, int mode, int cost_kind, int H, int64_t N,
         CK(launch_reduce_compact(h->stream, a, h->tau.as<double>(), h->worklist.as<unsigned>(), work_count, h->sms)); ++launches;
     }
     if (a.total_segs > 0) {
-        CK(launch_pass(h->stream, a, 2, pl.prefix, h->sms)); ++launches;
+        CK(launch_pass(h->stream, a, h->row_ab, 2, pl.prefix, h->sms)); ++launches;
         if (a.node_list) { CK(launch_refine_scan(h->stream, a, h->sms)); ++launches; }
         if (a.cand) { CK(launch_cand_resolve(h->stream, a, h->sms)); launches += 3; }
     }

@@ -41,6 +41,7 @@ struct mpcb_handle_s {
     double L = 0, delta_t = 0, v_min = 0, v_slow = 0;
     mpcb::GridTables g{};
     mpcb::DevBuf tab64, tab32, vtab, tab64_slow, vtab_slow, beta, leaf32, leaf32p, leaf32r, ctl32, ctl32_slow;
+    mpcb::RowPairs row_ab{};            // (a, b) of leaf32r's pairs: a kernel parameter of the exhaustive pass 1
     // options
     double tol_scale = 1.0;
     int algo = MPCB_ALGO_AUTO;

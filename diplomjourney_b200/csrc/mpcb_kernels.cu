@@ -536,10 +536,16 @@ __device__ __forceinline__ void prefix_screen_loop_rows(const float4 *__restrict
 
 // Stage 1 of the two-stage screen (option screen = 2, mpcb_screen.cuh): the same walk over the row table, forming only
 // -dd -- the same operands and operations as prefix_screen_loop_rows, so the very same values -- and keeping its maximum
-// per node: 2 FFMA2 + 1 FMNMX3 per node and leaf pair and one LDS.128 (the pair's a, b) instead of 7 + 1 + 1 and
-// LDS.128 + LDS.64.  The line and heading terms enter through a per-node bound (screen_stage1_tmax).
+// per node: 2 FFMA2 + 1 FMNMX3 per node and leaf pair.  The line and heading terms enter through a per-node bound
+// (screen_stage1_tmax).  Every lane reads the same pair at the same time, so the pairs' (a, b) come from the kernel
+// parameter `ab` (RowPairs): the uniform datapath loads them (LDCU.64 into uniform registers, which the FFMA2s take as
+// operands) instead of an LDS.128 writing the same four values into every lane's registers: 5 register writes per lane,
+// node and pair instead of 7.  ptxas emits them only in code it knows the whole warp runs together (see the skip test
+// of prefixn_kernel), and in small probes only while the loads are not addressed from the row counter, hence the two
+// pointers that advance by themselves.  The four-nodes-per-thread kernel, at its 128-register cap, reads the same
+// parameter with per-lane LDC.64.
 template <int NPT>
-__device__ __forceinline__ void prefix_dist_loop_rows(const float4 *__restrict__ tab, int nv, int ppr,
+__device__ __forceinline__ void prefix_dist_loop_rows(const RowPairs &ab, const float4 *__restrict__ tab, int nv, int ppr,
                                                       const ParentRegs (&p)[NPT], float (&mx)[NPT]) {
     float2 U[NPT], W[NPT];
     float nD[NPT], m[NPT];
@@ -550,15 +556,16 @@ __device__ __forceinline__ void prefix_dist_loop_rows(const float4 *__restrict__
         m[k] = -INFINITY;
     }
     constexpr int kUnroll = NPT == 2 ? MPCB_UNROLL_DIST : MPCB_UNROLL4;
-    for (int iv = 0; iv < nv; ++iv) {
-        const float4 *__restrict__ row = tab + 2 * iv * ppr;
+    const float4 *__restrict__ row = tab;
+    const float4 *pair = ab.ab;
+    for (int iv = 0; iv < nv; ++iv, row += 2 * ppr, pair += ppr) {
         const float rv = row[1].x;
         float2 DV[NPT];
 #pragma unroll
         for (int k = 0; k < NPT; ++k) { const float d = __fmaf_rn(-kWd2f, rv, nD[k]); DV[k] = make_float2(d, d); }
 #pragma unroll kUnroll
         for (int i = 0; i < ppr; ++i) {
-            const float4 t0 = row[2 * i];
+            const float4 t0 = pair[i];
             const float2 A = make_float2(t0.x, t0.y), B = make_float2(t0.z, t0.w);
 #pragma unroll
             for (int k = 0; k < NPT; ++k) {
@@ -1006,8 +1013,11 @@ __global__ void __launch_bounds__(kThreads, 4) refine_scan_kernel(const LaunchAr
 // chunk as a row table run the flat screen loop as with 1).
 __host__ __device__ constexpr int prefixn_cta(int npt) { return npt == 2 ? MPCB_PN_CTA2 : kPrefixCta / npt; }
 
+static_assert(sizeof(LaunchArgs) + sizeof(RowPairs) <= 32764, "prefixn_kernel's parameters exceed the launch limit");
+
 template <bool HEAD, int NPT, int SCREEN = 0>
-__global__ void __launch_bounds__(prefixn_cta(NPT), NPT / 2) prefixn_kernel(const LaunchArgs a) {
+__global__ void __launch_bounds__(prefixn_cta(NPT), NPT / 2)
+prefixn_kernel(const LaunchArgs a, const __grid_constant__ RowPairs ab) {
     extern __shared__ float4 s_leaf[];
     constexpr int kCta = prefixn_cta(NPT);
     const int tid = threadIdx.x;
@@ -1032,7 +1042,10 @@ __global__ void __launch_bounds__(prefixn_cta(NPT), NPT / 2) prefixn_kernel(cons
         const long long n = (long long)(w / qps);
         const unsigned long long tile0 = (w - (unsigned long long)n * qps) * groups;
         const SolveParams &P = a.sp[n];
-        if (P.flags & kFlagSkip) continue;
+        // one solve per work item, so the test is uniform per CTA; REDUX puts it in a uniform register, and the branch
+        // on it leaves the rest of the item in code ptxas knows to be warp-converged (a plain branch on P.flags does
+        // not, and the stage-1 loop then reads its table with per-lane LDC.64)
+        if (__reduce_or_sync(0xffffffffu, (unsigned)P.flags & kFlagSkip)) continue;
         const bool origin_case = (P.flags & kFlagStartIsOrigin) != 0;
         ParentRegs pr[NPT] = {};
         bool near[NPT], special[NPT], active[NPT];
@@ -1078,7 +1091,7 @@ __global__ void __launch_bounds__(prefixn_cta(NPT), NPT / 2) prefixn_kernel(cons
                 bool stage2 = true;
                 if (SCREEN == 2 && rows) {
                     float mdd[NPT];
-                    prefix_dist_loop_rows<NPT>(s_leaf, a.g.nv, a.g.ppr, pr, mdd);
+                    prefix_dist_loop_rows<NPT>(ab, s_leaf, a.g.nv, a.g.ppr, pr, mdd);
                     stage2 = false;
 #pragma unroll
                     for (int k = 0; k < NPT; ++k) {
@@ -2038,17 +2051,18 @@ static int resident_ctas(K kernel, size_t smem, int threads) {
 
 template <typename K>
 static cudaError_t launch_persistent(K kernel, const LaunchArgs &a, int pass, size_t smem, int sms, cudaStream_t st,
-                                     int threads = kThreads) {
+                                     int threads = kThreads, const RowPairs *ab = nullptr) {
     // pass 1: one CTA per resident slot, striding over the segments; pass 2: same grid over the
     // device-side work list (its length is not known on the host)
     if (smem > 48 * 1024) cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     const int slots = sms * resident_ctas(kernel, smem, threads);
     const int grid = pass == 1 ? (int)(a.total_segs < (unsigned long long)slots ? a.total_segs : slots) : slots;
-    kernel<<<grid, threads, smem, st>>>(a);
+    if constexpr (std::is_invocable_v<K, const LaunchArgs, const RowPairs>) kernel<<<grid, threads, smem, st>>>(a, *ab);
+    else kernel<<<grid, threads, smem, st>>>(a);
     return cudaGetLastError();
 }
 
-cudaError_t launch_pass(cudaStream_t st, const LaunchArgs &a, int pass, bool prefix, int sms) {
+cudaError_t launch_pass(cudaStream_t st, const LaunchArgs &a, const RowPairs &ab, int pass, bool prefix, int sms) {
     const bool head = a.cost_kind == 0;
     if (prefix) {
         const size_t sm = prefix_smem(a);
@@ -2068,8 +2082,8 @@ cudaError_t launch_pass(cudaStream_t st, const LaunchArgs &a, int pass, bool pre
             return head ? launch_persistent(prefix_kernel<1, true, true>, a, pass, sm, sms, st)
                         : launch_persistent(prefix_kernel<1, false, true>, a, pass, sm, sms, st);
 #define MPCB_PN(NPT_, SCR_)                                                                                      \
-    (head ? launch_persistent(prefixn_kernel<true, NPT_, SCR_>, a, pass, sm, sms, st, prefixn_cta(NPT_))         \
-          : launch_persistent(prefixn_kernel<false, NPT_, SCR_>, a, pass, sm, sms, st, prefixn_cta(NPT_)))
+    (head ? launch_persistent(prefixn_kernel<true, NPT_, SCR_>, a, pass, sm, sms, st, prefixn_cta(NPT_), &ab)    \
+          : launch_persistent(prefixn_kernel<false, NPT_, SCR_>, a, pass, sm, sms, st, prefixn_cta(NPT_), &ab))
         if (pass == 1 && a.npt == 4) return a.screen == 2 ? MPCB_PN(4, 2) : a.screen ? MPCB_PN(4, 1) : MPCB_PN(4, 0);
         if (pass == 1 && a.npt == 2) return a.screen == 2 ? MPCB_PN(2, 2) : a.screen ? MPCB_PN(2, 1) : MPCB_PN(2, 0);
 #undef MPCB_PN

@@ -141,6 +141,15 @@ struct GridTables {
     ScreenBox sbox;             // range of leaf32's a, b, g: the intervals of stage 1 of the two-stage screen (mpcb_screen.cuh)
 };
 
+// The {a_2m, a_2m+1, b_2m, b_2m+1} half of the row table (GridTables::leaf32r), for the stage-1 loop of the two-stage
+// screen, which reads it through the uniform datapath.  Filled by mpcb_set_grid when the row table exists and passed
+// BY VALUE to the exhaustive pass-1 kernel (a __grid_constant__ parameter), so every launch carries its own handle's
+// table: handles with different grids may solve concurrently on one device.  A row table fits one shared-memory chunk
+// (2 nv ppr <= kLeafChunk float4), so kLeafChunk / 2 pairs hold every one of them: 8 KiB of the 32,764 bytes a kernel's
+// parameters may take.
+constexpr int kRowPairCap = kLeafChunk / 2;
+struct RowPairs { float4 ab[kRowPairCap]; };
+
 // Per solve (float64). Built by prep_kernel from the raw inputs.
 struct __align__(16) SolveParams {
     double xs, ys, phi0;        // start pose
