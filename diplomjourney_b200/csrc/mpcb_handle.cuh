@@ -49,7 +49,7 @@ struct mpcb_handle_s {
     int small_path = 1;
     int zero_copy = 1;    // small_path with <= 64 solves: inputs and results in mapped pinned host memory, no copies
     int dump_direct = 0;  // mpcb_dump_leaves_host, prefix: dump the values pass 1 ranks with
-    int npt = 2;          // exhaustive prefix pass 1: nodes per thread (2: +6 %, tools/ubench)
+    int npt = 4;          // exhaustive prefix pass 1: nodes per thread (profiles/r3f_stage1_ab.txt)
     unsigned long long frontier_cap = mpcb::kFrontierCap;   // entries per frontier list (option, diagnostics: a tiny value forces the fallback)
     int subtree_cut = 2;       // pruned pass 1, H >= 3: 0 off, 1 depth-(H-2) bound per 256-node tile, 2 auto (frontier descent from the root for trees of more than one tile batch), 3 frontier always
     int screen = 2;       // exhaustive prefix pass 1 (prune = 0): 2 = screen in two stages (distance first), 1 = screen loop without

@@ -313,8 +313,10 @@ __device__ __forceinline__ void publish_best(const LaunchArgs &a, long long n, d
     __syncthreads();
 }
 
-// pass 1: every warp folds its partial minimum into the segment's key -- no CTA barrier
+// pass 1: every warp folds its partial minimum into the segment's key -- no CTA barrier.  Under the screen almost every
+// node publishes INFINITY, so a warp without a finite value skips the reduction (it would publish nothing anyway).
 __device__ __forceinline__ void publish_segmin(const LaunchArgs &a, unsigned seg, double v) {
+    if (!__any_sync(0xffffffffu, v < INFINITY)) return;
     v = warp_min(v);
     if ((threadIdx.x & 31) == 0 && v < INFINITY)
         atomicMin(reinterpret_cast<unsigned long long *>(a.segmin) + seg, ordered_key(v));
@@ -542,8 +544,8 @@ __device__ __forceinline__ void prefix_screen_loop_rows(const float4 *__restrict
 // operands) instead of an LDS.128 writing the same four values into every lane's registers: 5 register writes per lane,
 // node and pair instead of 7.  ptxas emits them only in code it knows the whole warp runs together (see the skip test
 // of prefixn_kernel), and in small probes only while the loads are not addressed from the row counter, hence the two
-// pointers that advance by themselves.  The four-nodes-per-thread kernel, at its 128-register cap, reads the same
-// parameter with per-lane LDC.64.
+// pointers that advance by themselves.  Each load feeds all NPT nodes of the lane: per 7 pairs, 14 LDCU.64 and the loop's
+// bookkeeping serve 28 FFMA2 with two nodes per thread and 56 with four.  Only u2s, w2s and D2s of `p` are read.
 template <int NPT>
 __device__ __forceinline__ void prefix_dist_loop_rows(const RowPairs &ab, const float4 *__restrict__ tab, int nv, int ppr,
                                                       const ParentRegs (&p)[NPT], float (&mx)[NPT]) {
@@ -555,7 +557,7 @@ __device__ __forceinline__ void prefix_dist_loop_rows(const RowPairs &ab, const 
         nD[k] = -p[k].D2s;
         m[k] = -INFINITY;
     }
-    constexpr int kUnroll = NPT == 2 ? MPCB_UNROLL_DIST : MPCB_UNROLL4;
+    constexpr int kUnroll = MPCB_UNROLL_DIST;
     const float4 *__restrict__ row = tab;
     const float4 *pair = ab.ab;
     for (int iv = 0; iv < nv; ++iv, row += 2 * ppr, pair += ppr) {
@@ -1009,8 +1011,15 @@ __global__ void __launch_bounds__(kThreads, 4) refine_scan_kernel(const LaunchAr
 // tiles as prefix_kernel<1>, thread t holding nodes t, t + 1024/NPT, ... of the work item (NPT = 4: two such CTAs per
 // SM).  Same arithmetic per node, so the segment minima (and everything downstream) are bit-identical to the
 // one-node kernel.  SCREEN (option screen): 0 = MUFU.SQRT per leaf, 1 = the screen loop, 2 = the screen in two stages
-// (prefix_dist_loop_rows first, the screen loop only if a node of the thread passes stage 1; tables that do not fit one
-// chunk as a row table run the flat screen loop as with 1).
+// (below; it needs the row table, and launch_pass runs grids whose row table does not fit one chunk with 1).
+//
+// The two-stage work item runs in three phases.  A: each node is set up and keeps only what stage 1 reads -- u2s, w2s,
+// D2s and its stage-1 bound T (screen_stage1_tmax) -- and a class: inactive, stage 1, or direct (NEAR, or unmoved on
+// the line origin: the scalar loop).  B: if any lane of the warp holds a stage-1 node, prefix_dist_loop_rows runs for
+// all NPT slots (the other classes' values are ignored).  C: each node that stage 1 passes (0.045 % of the cfg2
+// nodes) and each direct node is set up again -- the same code on the same inputs, so the very same registers -- and
+// scored alone: the screen loop, then the MUFU loop if it flags a leaf; direct nodes as in the one-stage kernel.
+// Holding only stage 1's registers through the loop is what lets four nodes per thread share each table load.
 __host__ __device__ constexpr int prefixn_cta(int npt) { return npt == 2 ? MPCB_PN_CTA2 : kPrefixCta / npt; }
 
 static_assert(sizeof(LaunchArgs) + sizeof(RowPairs) <= 32764, "prefixn_kernel's parameters exceed the launch limit");
@@ -1047,89 +1056,144 @@ prefixn_kernel(const LaunchArgs a, const __grid_constant__ RowPairs ab) {
         // not, and the stage-1 loop then reads its table with per-lane LDC.64)
         if (__reduce_or_sync(0xffffffffu, (unsigned)P.flags & kFlagSkip)) continue;
         const bool origin_case = (P.flags & kFlagStartIsOrigin) != 0;
-        ParentRegs pr[NPT] = {};
-        bool near[NPT], special[NPT], active[NPT];
-        double base[NPT];
-        float best[NPT], Lspecial[NPT], cn[NPT];
-        unsigned seg[NPT];
-        bool all = true;
+        // slot k of the thread: its node p (false: past the solve's last node) and the segment it publishes to
+        auto slot = [&](int k, unsigned long long &p, unsigned &sg) {
+            const unsigned node = tid + k * kCta;
+            const unsigned long long tile = tile0 + node / kThreads;
+            p = a.u_begin + tile * kThreads + (node % kThreads);
+            sg = (unsigned)((unsigned long long)n * a.segs_per_solve + (a.tps == 1 ? tile : tile / a.tps));
+            return tile < a.tiles_per_solve && p < a.u_end;
+        };
         // SCREEN: no leaf whose value exceeds the solve's upper bound (the exact probe, tightened by every node that
         // found something) by more than the ranking window tol1 can be the minimum or enter the refinement window
         double ubw = INFINITY;
         if (SCREEN) ubw = ordered_value(*(volatile unsigned long long *)(a.ub + n)) + P.tol1;
+        const int npairs_rows = a.g.nv * a.g.ppr;
+        double v[NPT];                  // each node's value base + best (INFINITY: nothing to publish)
+        double vhit = INFINITY;         // the least value of the nodes the screen loop flagged
 #pragma unroll
-        for (int k = 0; k < NPT; ++k) {
-            const unsigned node = tid + k * kCta;
-            const unsigned long long tile = tile0 + node / kThreads;
-            const unsigned long long p = a.u_begin + tile * kThreads + (node % kThreads);
-            active[k] = tile < a.tiles_per_solve && p < a.u_end;
-            seg[k] = (unsigned)((unsigned long long)n * a.segs_per_solve + (a.tps == 1 ? tile : tile / a.tps));
-            bool unmoved = false;
-            near[k] = false; base[k] = 0.0; best[k] = INFINITY;
-            double base_direct = 0.0;
-            if (active[k]) base[k] = parent_setup(a, P, p, pr[k], near[k], unmoved, nullptr, &base_direct);
-            special[k] = active[k] && origin_case && unmoved;
-            if (!(near[k] || special[k])) base[k] = base_direct;
-            Lspecial[k] = (float)(P.special - 0.25 * (double)pr[k].e2 * (double)pr[k].e2);
-            cn[k] = SCREEN ? __double2float_ru(ubw - base_direct) : 0.f;
-            all = all && active[k] && !near[k] && !special[k];
-        }
-        bool hit[NPT];
+        for (int k = 0; k < NPT; ++k) v[k] = INFINITY;
+        if constexpr (SCREEN == 2) {
+            // A: set-up, keeping what stage 1 reads
+            ParentRegs s1[NPT] = {};
+            float tmax[NPT];
+            unsigned staged = 0, direct = 0;     // bit k: slot k is a stage-1 / a direct node
 #pragma unroll
-        for (int k = 0; k < NPT; ++k) hit[k] = false;
-        for (int c0 = 0; c0 < S; c0 += kLeafChunk) {
-            const int cn_ = min(kLeafChunk, S - c0);
-            if (!single) {
-                __syncthreads();
-                for (int i = tid; i < chunk_f4(cn_); i += blockDim.x) s_leaf[i] = __ldg(gtab + c0 + i);
-                __syncthreads();
+            for (int k = 0; k < NPT; ++k) {
+                unsigned long long p;
+                unsigned sg;
+                tmax[k] = 0.f;
+                if (!slot(k, p, sg)) continue;
+                ParentRegs q;
+                bool nr, um;
+                double bd;
+                parent_setup(a, P, p, q, nr, um, nullptr, &bd);
+                if (nr || (origin_case && um)) { direct |= 1u << k; continue; }
+                staged |= 1u << k;
+                s1[k].u2s = q.u2s; s1[k].w2s = q.w2s; s1[k].D2s = q.D2s;
+                tmax[k] = screen_stage1_tmax(a.g.sbox, HEAD, __double2float_ru(ubw - bd), q.nu, q.nw, q.eh, q.nhh);
             }
-            const int npairs = rows ? a.g.nv * a.g.ppr : (cn_ + 1) >> 1;
-            if (all && SCREEN) {
-                // two stages: the screen loop only runs if stage 1 passes a node of the thread (almost never on the cfg2
-                // bench); it then runs for all of them, and a node stage 1 rejected has no leaf with t^2 - dd > 0 there
-                bool stage2 = true;
-                if (SCREEN == 2 && rows) {
-                    float mdd[NPT];
-                    prefix_dist_loop_rows<NPT>(ab, s_leaf, a.g.nv, a.g.ppr, pr, mdd);
-                    stage2 = false;
+            // B: stage 1, under a warp-uniform test (ptxas feeds the loop from uniform registers only in converged code)
+            unsigned rare = direct;
+            if (__reduce_or_sync(0xffffffffu, staged)) {
+                float mdd[NPT];
+                prefix_dist_loop_rows<NPT>(ab, s_leaf, a.g.nv, a.g.ppr, s1, mdd);
 #pragma unroll
-                    for (int k = 0; k < NPT; ++k) {
-                        const float tmax = screen_stage1_tmax(a.g.sbox, HEAD, cn[k], pr[k].nu, pr[k].nw, pr[k].eh, pr[k].nhh);
-                        const bool pass = screen_stage1_pass(tmax, mdd[k]);
-                        stage2 = stage2 || pass;
-                        stage2_acc += pass ? 1u : 0u;
+                for (int k = 0; k < NPT; ++k)
+                    if (((staged >> k) & 1u) && screen_stage1_pass(tmax[k], mdd[k])) { rare |= 1u << k; ++stage2_acc; }
+            }
+            // C: the nodes stage 1 passed and the direct ones, set up again and scored one at a time
+            for (unsigned m = rare; m; m &= m - 1) {
+                const int k = __ffs(m) - 1;
+                unsigned long long p;
+                unsigned sg;
+                slot(k, p, sg);
+                ParentRegs pr;
+                bool near, unmoved;
+                double bd;
+                double base = parent_setup(a, P, p, pr, near, unmoved, nullptr, &bd);
+                float best = INFINITY;
+                if ((direct >> k) & 1u) {
+                    const float Ls = (float)(P.special - 0.25 * (double)pr.e2 * (double)pr.e2);
+                    best = prefix_min_loop_scalar<HEAD>(s_leaf, npairs_rows, pr, near, origin_case && unmoved, Ls, best);
+                } else {
+                    base = bd;
+                    const ParentRegs one[1] = {pr};
+                    const float cn[1] = {__double2float_ru(ubw - bd)};
+                    float mx[1];
+                    prefix_screen_loop_rows<HEAD, 1>(s_leaf, a.g.nv, a.g.ppr, one, cn, mx);
+                    if (mx[0] > 0.f) {              // some leaf of the node has t^2 - dd > 0: it may matter
+                        best = prefix_min_loop_far2<HEAD>(s_leaf, npairs_rows, pr, best);
+                        vhit = fmin(vhit, base + (double)best);
                     }
                 }
-                if (stage2) {
+#pragma unroll
+                for (int j = 0; j < NPT; ++j)
+                    if (j == k) v[j] = base + (double)best;
+            }
+        } else {
+            ParentRegs pr[NPT] = {};
+            bool near[NPT], special[NPT], active[NPT];
+            double base[NPT];
+            float best[NPT], Lspecial[NPT], cn[NPT];
+            bool all = true;
+#pragma unroll
+            for (int k = 0; k < NPT; ++k) {
+                unsigned long long p;
+                unsigned sg;
+                active[k] = slot(k, p, sg);
+                bool unmoved = false;
+                near[k] = false; base[k] = 0.0; best[k] = INFINITY;
+                double base_direct = 0.0;
+                if (active[k]) base[k] = parent_setup(a, P, p, pr[k], near[k], unmoved, nullptr, &base_direct);
+                special[k] = active[k] && origin_case && unmoved;
+                if (!(near[k] || special[k])) base[k] = base_direct;
+                Lspecial[k] = (float)(P.special - 0.25 * (double)pr[k].e2 * (double)pr[k].e2);
+                cn[k] = SCREEN ? __double2float_ru(ubw - base_direct) : 0.f;
+                all = all && active[k] && !near[k] && !special[k];
+            }
+            bool hit[NPT];
+#pragma unroll
+            for (int k = 0; k < NPT; ++k) hit[k] = false;
+            for (int c0 = 0; c0 < S; c0 += kLeafChunk) {
+                const int cn_ = min(kLeafChunk, S - c0);
+                if (!single) {
+                    __syncthreads();
+                    for (int i = tid; i < chunk_f4(cn_); i += blockDim.x) s_leaf[i] = __ldg(gtab + c0 + i);
+                    __syncthreads();
+                }
+                const int npairs = rows ? npairs_rows : (cn_ + 1) >> 1;
+                if (all && SCREEN) {
                     float mx[NPT];
                     if (rows) prefix_screen_loop_rows<HEAD, NPT>(s_leaf, a.g.nv, a.g.ppr, pr, cn, mx);
                     else prefix_screen_loop_far2xN<HEAD, NPT>(s_leaf, npairs, pr, cn, mx);
 #pragma unroll
                     for (int k = 0; k < NPT; ++k)       // some leaf of the node has t^2 - dd > 0: it may matter
                         if (mx[k] > 0.f) { best[k] = prefix_min_loop_far2<HEAD>(s_leaf, npairs, pr[k], best[k]); hit[k] = true; }
-                }
-            } else if (all) {
-                prefix_min_loop_far2xN<HEAD, NPT>(s_leaf, npairs, pr, best);
-            } else {
+                } else if (all) {
+                    prefix_min_loop_far2xN<HEAD, NPT>(s_leaf, npairs, pr, best);
+                } else {
 #pragma unroll
-                for (int k = 0; k < NPT; ++k) {
-                    if (!active[k]) continue;
-                    best[k] = (near[k] || special[k])
-                                  ? prefix_min_loop_scalar<HEAD>(s_leaf, npairs, pr[k], near[k], special[k], Lspecial[k], best[k])
-                                  : prefix_min_loop_far2<HEAD>(s_leaf, npairs, pr[k], best[k]);
+                    for (int k = 0; k < NPT; ++k) {
+                        if (!active[k]) continue;
+                        best[k] = (near[k] || special[k])
+                                      ? prefix_min_loop_scalar<HEAD>(s_leaf, npairs, pr[k], near[k], special[k], Lspecial[k], best[k])
+                                      : prefix_min_loop_far2<HEAD>(s_leaf, npairs, pr[k], best[k]);
+                    }
                 }
+            }
+#pragma unroll
+            for (int k = 0; k < NPT; ++k) {
+                if (active[k]) v[k] = base[k] + (double)best[k];
+                if (hit[k]) vhit = fmin(vhit, v[k]);
             }
         }
         if (SCREEN) {
             // a node that found something tightens the solve's upper bound for the work items still to come:
             // its best fp32 value + the error bound of that value is >= the true cost of a leaf
-            double v = INFINITY;
-#pragma unroll
-            for (int k = 0; k < NPT; ++k) if (hit[k]) v = fmin(v, base[k] + (double)best[k]);
-            if (__any_sync(0xffffffffu, v < INFINITY)) {
-                v = warp_min(v);
-                if ((tid & 31) == 0) atomicMin(a.ub + n, ordered_key(v + 0.5 * P.tol1));
+            if (__any_sync(0xffffffffu, vhit < INFINITY)) {
+                vhit = warp_min(vhit);
+                if ((tid & 31) == 0) atomicMin(a.ub + n, ordered_key(vhit + 0.5 * P.tol1));
             }
         }
         // SCREEN: a node whose best value lies above the bound cannot hold the minimum or an in-window leaf, whichever loop
@@ -1138,8 +1202,10 @@ prefixn_kernel(const LaunchArgs a, const __grid_constant__ RowPairs ab) {
         // such nodes: on the config.py tree the 16^4 exactly tied unmoved nodes of the v = 0 share, 2.3e7 candidates.
 #pragma unroll
         for (int k = 0; k < NPT; ++k) {
-            const double v = active[k] ? base[k] + (double)best[k] : INFINITY;
-            publish_segmin(a, seg[k], (!SCREEN || v <= ubw) ? v : INFINITY);
+            unsigned long long p;
+            unsigned sg;
+            slot(k, p, sg);
+            publish_segmin(a, sg, (!SCREEN || v[k] <= ubw) ? v[k] : INFINITY);
         }
     }
     if (SCREEN == 2) {
@@ -2084,8 +2150,10 @@ cudaError_t launch_pass(cudaStream_t st, const LaunchArgs &a, const RowPairs &ab
 #define MPCB_PN(NPT_, SCR_)                                                                                      \
     (head ? launch_persistent(prefixn_kernel<true, NPT_, SCR_>, a, pass, sm, sms, st, prefixn_cta(NPT_), &ab)    \
           : launch_persistent(prefixn_kernel<false, NPT_, SCR_>, a, pass, sm, sms, st, prefixn_cta(NPT_), &ab))
-        if (pass == 1 && a.npt == 4) return a.screen == 2 ? MPCB_PN(4, 2) : a.screen ? MPCB_PN(4, 1) : MPCB_PN(4, 0);
-        if (pass == 1 && a.npt == 2) return a.screen == 2 ? MPCB_PN(2, 2) : a.screen ? MPCB_PN(2, 1) : MPCB_PN(2, 0);
+        // the two-stage screen needs the row table; without it the one-stage flat loop runs
+        const int scr = a.screen == 2 && a.g.ppr == 0 ? 1 : a.screen;
+        if (pass == 1 && a.npt == 4) return scr == 2 ? MPCB_PN(4, 2) : scr ? MPCB_PN(4, 1) : MPCB_PN(4, 0);
+        if (pass == 1 && a.npt == 2) return scr == 2 ? MPCB_PN(2, 2) : scr ? MPCB_PN(2, 1) : MPCB_PN(2, 0);
 #undef MPCB_PN
         if (pass == 1)
             return head ? launch_persistent(prefix_kernel<1, true>, a, pass, sm, sms, st, kPrefixCta)

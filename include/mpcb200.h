@@ -125,8 +125,8 @@ MPCB_API int mpcb_set_grid(mpcb_handle *h, const double *v, int nv, const double
  * a few thousand scans are spread evenly over the GPU instead of staying with the few warps that found the nodes;
  * nodes beyond the capacity -- or all of them with 0 -- are scanned where they are found, which is as good when there
  * are many),
- * "nodes_per_thread" (1, 2 or 4, default 2: depth-(H-1) nodes each thread of the exhaustive prefix pass 1 holds --
- * identical results), "dump_direct" (diagnostics: mpcb_dump_leaves_host returns the cheaper fp32 form pass 1 ranks
+ * "nodes_per_thread" (1, 2 or 4, default 4: depth-(H-1) nodes each thread of the exhaustive prefix pass 1 holds --
+ * identical results; with the two-stage screen four nodes share each table load of its stage-1 loop), "dump_direct" (diagnostics: mpcb_dump_leaves_host returns the cheaper fp32 form pass 1 ranks
  * with instead of the one pass 2 filters with; default 0), "frontier_cap" (see "subtree_cut"). */
 MPCB_API int mpcb_set_option(mpcb_handle *h, const char *name, double value);
 
