@@ -107,6 +107,11 @@ def load():
     lib.mpcb_held_closed_loop_actual_device.argtypes = lib.mpcb_held_closed_loop_actual_host.argtypes
     lib.mpcb_held_closed_loop_seeded_host.argtypes = loop[:8] + [vp, C.c_int32, C.c_double, vp, C.c_int32, vp] + loop[8:] + [vp]
     lib.mpcb_rng_seed_device.argtypes = [vp, C.c_int64, vp, C.c_int32, vp]
+    lib.mpcb_held_closed_loop_pcg64_host.argtypes = lib.mpcb_held_closed_loop_actual_host.argtypes
+    lib.mpcb_held_closed_loop_pcg64_device.argtypes = lib.mpcb_held_closed_loop_actual_host.argtypes
+    lib.mpcb_held_closed_loop_pcg64_seeded_host.argtypes = loop[:8] + [vp, C.c_int32, C.c_double, vp, C.c_int32, C.c_int32,
+                                                                       vp, C.c_int32, vp] + loop[8:] + [vp]
+    lib.mpcb_pcg64_seed_device.argtypes = [vp, C.c_int64, vp, C.c_int32, C.c_int32, vp, C.c_int32, vp]
     lib.mpcb_held_tick_host.argtypes = [vp, vp, C.c_int, vp, C.c_int, C.c_double, C.c_double, C.c_double, C.c_int, C.c_int,
                                         vp, vp, vp, C.c_double, C.c_int, vp, vp, vp, vp]
     win = [vp, C.POINTER(LoopParams), C.c_int64, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
@@ -170,6 +175,90 @@ def seed_keys(seeds, n):
     if a.size and (a.min() < 0 or a.max() > 0xFFFFFFFF):
         raise ValueError(_SEED_RANGE)
     return np.ascontiguousarray(a, dtype=np.uint32), (a.shape[1] if a.ndim == 2 else 0)
+
+
+PCG64_WORDS = 6
+_U64 = (1 << 64) - 1
+
+
+def pcg64_record(bit_generator):
+    """[6] uint64 record of a numpy PCG64 bit generator (or of its ``.state`` dict) in the form the PCG64 entries take
+    it: state >> 64, state mod 2^64, inc >> 64, inc mod 2^64, has_uint32, uinteger."""
+    st = bit_generator if isinstance(bit_generator, dict) else bit_generator.state
+    if st.get("bit_generator") != "PCG64":
+        raise TypeError(f"not a PCG64 state: {st.get('bit_generator')!r}")
+    s, inc = int(st["state"]["state"]), int(st["state"]["inc"])
+    return np.array([s >> 64, s & _U64, inc >> 64, inc & _U64, int(st["has_uint32"]), int(st["uinteger"])], np.uint64)
+
+
+def pcg64_state(record):
+    """numpy's PCG64 ``state`` dict of one [6] record (the inverse of ``pcg64_record``)."""
+    r = [int(x) for x in record]
+    return {"bit_generator": "PCG64", "state": {"state": (r[0] << 64) | r[1], "inc": (r[2] << 64) | r[3]},
+            "has_uint32": r[4], "uinteger": r[5]}
+
+
+def _words(x):
+    """SeedSequence's 32-bit little-endian words of a non-negative integer (0 -> one word) or of a sequence of them."""
+    if not isinstance(x, (int, np.integer)):
+        out = []
+        for v in x:
+            out += _words(v)
+        return out
+    x = operator.index(x)
+    if x < 0:
+        raise ValueError("expected non-negative integer")
+    w = []
+    while True:
+        w.append(x & 0xFFFFFFFF)
+        x >>= 32
+        if not x:
+            return w
+
+
+def pcg64_seed_words(seeds, n):
+    """The seeds of ``n`` Generator(PCG64) streams in the form mpcb_pcg64_seed_device takes them: returns (entropy
+    uint32, entropy_stride, spawn uint32 [n][K] or None).
+
+    * ``seeds`` an ``np.random.SeedSequence``: robot i gets ``default_rng(seeds.spawn(n)[i])`` -- the shared entropy
+      (stride 0) and per robot the spawn key ``seeds.spawn_key + (seeds.n_children_spawned + i,)``.  ``seeds`` is not
+      advanced here.
+    * ``seeds`` [n] non-negative integers: robot i gets ``default_rng(seeds[i])`` -- one entropy row per robot.
+
+    Raises what numpy raises for a negative integer, refuses a pool_size other than 4 and integer rows whose word counts
+    cannot share one stride (integers of different lengths above 2^128)."""
+    if isinstance(seeds, np.random.SeedSequence):
+        if seeds.pool_size != 4:
+            raise ValueError(f"SeedSequence pool_size {seeds.pool_size}: the PCG64 seeding works with pool_size 4")
+        ent = _words(seeds.entropy)
+        base = _words(seeds.spawn_key)
+        first = seeds.n_children_spawned
+        if first + n > 2 ** 32:                 # numpy counts children in 32 bits
+            raise ValueError(f"{first} + {n} children: more than 2^32 spawned from one SeedSequence")
+        if len(ent) > MAX_KEY_LEN or len(base) + 1 > MAX_KEY_LEN:
+            raise ValueError(f"more than {MAX_KEY_LEN} seed words")
+        keys = np.empty((n, len(base) + 1), np.uint32)
+        keys[:, :-1] = base
+        keys[:, -1] = np.arange(first, first + n, dtype=np.uint64)
+        return np.array(ent, np.uint32), 0, (keys if n else None)
+    if isinstance(seeds, np.random.Generator) or isinstance(seeds, np.random.BitGenerator):
+        raise TypeError("seeds must be a SeedSequence or integer seeds, not a generator")
+    a = list(seeds)
+    if len(a) != n:
+        raise ValueError(f"seeds holds {len(a)} rows for {n} robots")
+    try:
+        rows = [_words(operator.index(s)) for s in a]
+    except TypeError:
+        raise TypeError("seeds must be integers or a SeedSequence") from None
+    E = max([4] + [len(r) for r in rows])
+    if E > 4 and any(len(r) != E for r in rows):
+        raise ValueError("integer seeds above 2^128 must all have the same number of 32-bit words")
+    if E > MAX_KEY_LEN:
+        raise ValueError(f"more than {MAX_KEY_LEN} seed words")
+    ent = np.zeros((n, E), np.uint32)     # zero words up to the pool size do not change the stream
+    for i, r in enumerate(rows):
+        ent[i, :len(r)] = r
+    return ent, E, None
 
 
 def _event_script(events):
@@ -345,7 +434,8 @@ class Solver:
         return dict(cost=cost_o, index=idx_o, traj=traj_o, first_control=ctl_o, shape=shape_o)
 
     def held_closed_loop(self, params: "LoopParams", init, target, origin, first_threshold=None, slow_steps=None,
-                         events=None, radius_u_turn=0.0, rng_state=None, seeds=None, return_rng_state=True):
+                         events=None, radius_u_turn=0.0, rng_state=None, seeds=None, return_rng_state=True,
+                         pcg_state=None, pcg_seeds=None):
         """Whole closed loops of the online controller for a batch of robots on the device
         (mpcb_held_closed_loop_host / _events_host). ``events``: an operator script [(tick, kind, a, b), ...] with kind
         EVENT_NEW_TARGET (a, b = the new target) or EVENT_TURN_LEFT / _RIGHT (a = distance), applied to every robot
@@ -355,8 +445,15 @@ class Solver:
         ``seeds`` [N] integer seeds or [N][K] keys (see ``seed_keys``): the actual run with the generators of
         RandomState(seeds[i]), seeded on the device (mpcb_held_closed_loop_seeded_host); not together with
         ``rng_state``.  ``return_rng_state=False`` leaves the seeded generators' final states on the device.
+        ``pcg_state`` [N][6] uint64 (per robot numpy Generator(PCG64) state, see ``pcg64_record``): the actual run with
+        numpy's Generator stream in place of RandomState's (mpcb_held_closed_loop_pcg64_host); the input is not modified.
+        ``pcg_seeds`` a SeedSequence or [N] integer seeds (see ``pcg64_seed_words``): the generators of
+        default_rng(pcg_seeds.spawn(N)[i]) resp. default_rng(pcg_seeds[i]), seeded on the device
+        (mpcb_held_closed_loop_pcg64_seeded_host); a SeedSequence is advanced as spawn(N) advances it.
         Returns dict(log[N,max_ticks,5], ticks[N], status[N], final[N,6] = x_t, y_t, x_0, y_0, steps_for_slowing, m),
-        with ``rng_state`` or ``seeds`` also the generators' states after the run."""
+        with ``rng_state`` or ``seeds`` also the generators' states after the run (``pcg_state`` with the PCG64 ones)."""
+        if sum(x is not None for x in (rng_state, seeds, pcg_state, pcg_seeds)) > 1:
+            raise ValueError("rng_state, seeds, pcg_state and pcg_seeds each give the generators: pass one of them")
         ini = _arr(init, np.float64, (-1, 5))
         N = ini.shape[0]
         tg = _arr(np.broadcast_to(np.asarray(target, np.float64).reshape(-1, 2), (N, 2)), np.float64)
@@ -368,9 +465,28 @@ class Solver:
         status = np.empty(N, np.int32)
         ev, n_ev = _event_script(events)
         final = np.empty((N, 6))
+        if pcg_seeds is not None or pcg_state is not None:
+            common = (self.h, C.byref(params), N, _ptr(ini), _ptr(tg), _ptr(og), _ptr(thr), _ptr(sl), ev, n_ev,
+                      float(radius_u_turn))
+            if pcg_seeds is not None:
+                ent, stride, spawn = pcg64_seed_words(pcg_seeds, N)
+                ps = np.empty((N, PCG64_WORDS), np.uint64) if return_rng_state else None
+                self._ck(self.lib.mpcb_held_closed_loop_pcg64_seeded_host(
+                    *common, _ptr(ent), ent.shape[-1], stride, _ptr(spawn), 0 if spawn is None else spawn.shape[1],
+                    _ptr(ps), _ptr(log), _ptr(ticks), _ptr(status), _ptr(final)))
+                if isinstance(pcg_seeds, np.random.SeedSequence):
+                    pcg_seeds.spawn(N)                  # the children robots 0..N-1 drew from are now spawned
+            else:
+                ps = np.array(pcg_state, dtype=np.uint64, order="C")        # a copy: the library updates it in place
+                if ps.shape != (N, PCG64_WORDS):
+                    raise ValueError(f"pcg_state must be [N][6] = [{N}][6] (see pcg64_record), got {ps.shape}")
+                self._ck(self.lib.mpcb_held_closed_loop_pcg64_host(*common, _ptr(ps), _ptr(log), _ptr(ticks),
+                                                                   _ptr(status), _ptr(final)))
+            out = dict(log=log, ticks=ticks, status=status, final=final)
+            if ps is not None:
+                out["pcg_state"] = ps
+            return out
         if seeds is not None:
-            if rng_state is not None:
-                raise ValueError("seeds and rng_state both give the generators: pass one of them")
             keys, key_len = seed_keys(seeds, N)
             rs = np.empty((N, 625), np.uint32) if return_rng_state else None
             self._ck(self.lib.mpcb_held_closed_loop_seeded_host(self.h, C.byref(params), N, _ptr(ini), _ptr(tg), _ptr(og),
@@ -416,6 +532,28 @@ class Solver:
                                                               vp(origin), vp(first_threshold), vp(slow_steps), ev, n_ev,
                                                               float(radius_u_turn), vp(rng_state), vp(out_log),
                                                               vp(out_ticks), vp(out_status), vp(out_final)))
+
+    def seed_pcg64_device(self, N, entropy, entropy_len, entropy_stride, spawn, spawn_len, out):
+        """mpcb_pcg64_seed_device: the [N][6] uint64 records of default_rng(SeedSequence(entropy words, spawn-key
+        words)) written to ``out`` -- entropy [entropy_len] shared (stride 0) or [N][entropy_len] (stride entropy_len),
+        spawn [N][spawn_len] or 0 (uint32 words, see ``pcg64_seed_words``).  Raw device addresses; enqueues on
+        self.stream, does not synchronise."""
+        vp = lambda x: C.c_void_p(int(x)) if x else None
+        self._ck(self.lib.mpcb_pcg64_seed_device(self.h, int(N), vp(entropy), int(entropy_len), int(entropy_stride),
+                                                 vp(spawn), int(spawn_len), vp(out)))
+
+    def held_closed_loop_device_pcg64(self, params: "LoopParams", N, init, target, origin, first_threshold, slow_steps,
+                                      pcg_state, out_log, out_ticks, out_status, out_final=None, events=None,
+                                      radius_u_turn=0.0):
+        """mpcb_held_closed_loop_pcg64_device: ``held_closed_loop_device_actual`` with per-robot Generator(PCG64)
+        records, pcg_state [N][6] uint64 updated in place (raw device addresses).  Enqueues on self.stream, does not
+        synchronise."""
+        vp = lambda x: C.c_void_p(int(x)) if x else None
+        ev, n_ev = _event_script(events)
+        self._ck(self.lib.mpcb_held_closed_loop_pcg64_device(self.h, C.byref(params), int(N), vp(init), vp(target),
+                                                             vp(origin), vp(first_threshold), vp(slow_steps), ev, n_ev,
+                                                             float(radius_u_turn), vp(pcg_state), vp(out_log),
+                                                             vp(out_ticks), vp(out_status), vp(out_final)))
 
     def full_closed_loop(self, cost, H, init_state, target, origin, first_threshold=None, eps=0.001, max_ticks=256):
         """Closed loop of the FULL-tree scripts for a batch of robots (mpcb_full_closed_loop_host): one batched

@@ -16,7 +16,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.environ.get("MPCB_LIB") or os.path.join(HERE, "lib", "libmpcb200.so")   # MPCB_LIB: developer override
 SOURCES = ["mpcb_kernels.cu", "mpcb_loop.cu", "mpcb_api.cu", "mpcb_nccl.cu"]
-HEADERS = ["mpcb_types.cuh", "mpcb_bounds.cuh", "mpcb_exact.cuh", "mpcb_handle.cuh", "mpcb_events.cuh", "mpcb_noise.cuh", "mpcb_screen.cuh", os.path.join("..", "..", "include", "mpcb200.h")]
+HEADERS = ["mpcb_types.cuh", "mpcb_bounds.cuh", "mpcb_exact.cuh", "mpcb_handle.cuh", "mpcb_events.cuh", "mpcb_noise.cuh", "mpcb_pcg64.cuh", "mpcb_screen.cuh", os.path.join("..", "..", "include", "mpcb200.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
     "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "--shared",

@@ -8,6 +8,7 @@
 #include "mpcb_bounds.cuh"
 #include "mpcb_handle.cuh"
 #include "mpcb_noise.cuh"
+#include "mpcb_pcg64.cuh"
 
 #include <algorithm>
 #include <cmath>
@@ -37,6 +38,8 @@ cudaError_t launch_finalize(cudaStream_t, const LaunchArgs &, double *, long lon
 cudaError_t launch_dump(cudaStream_t, const LaunchArgs &, bool prefix, double *jrel, int sms);
 cudaError_t launch_held_loop(cudaStream_t, const LoopArgs &, int sms);
 cudaError_t launch_rng_seed(cudaStream_t, long long N, const unsigned *keys, int key_len, unsigned *rng_state);
+cudaError_t launch_pcg64_seed(cudaStream_t, long long N, const unsigned *entropy, int ent_len, int ent_stride,
+                              const unsigned *spawn, int spawn_len, unsigned long long *pcg_state);
 cudaError_t launch_held_small(cudaStream_t, const SmallArgs &);
 cudaError_t launch_full_apply(cudaStream_t, const FullLoopArgs &);
 cudaError_t launch_held_windows(cudaStream_t, const WindowArgs &, int sms);
@@ -832,13 +835,41 @@ static int check_seed_keys(mpcb_handle *h, int64_t N, const uint32_t *keys, int3
     return MPCB_OK;
 }
 
+// numpy SeedSequence words of N PCG64 generators: entropy[entropy_len] shared (stride 0) or [N][entropy_len], and
+// spawn_key[N][spawn_len] (spawn_len 0: none); 1 <= entropy_len <= 4096, 0 <= spawn_len <= 4096
+static int check_pcg64_seeds(mpcb_handle *h, int64_t N, const uint32_t *entropy, int32_t entropy_len,
+                             int32_t entropy_stride, const uint32_t *spawn_key, int32_t spawn_len) {
+    if (N < 0 || N >= (1LL << 31)) return fail(h, MPCB_ERR_INVALID, "N out of range");
+    if (entropy_len < 1 || entropy_len > 4096)
+        return fail(h, MPCB_ERR_INVALID, "PCG64 seeding: entropy_len %d outside [1, 4096]", entropy_len);
+    if (entropy_stride != 0 && entropy_stride != entropy_len)
+        return fail(h, MPCB_ERR_INVALID, "PCG64 seeding: entropy_stride %d is neither 0 nor entropy_len", entropy_stride);
+    if (spawn_len < 0 || spawn_len > 4096)
+        return fail(h, MPCB_ERR_INVALID, "PCG64 seeding: spawn_len %d outside [0, 4096]", spawn_len);
+    if (N > 0 && (!entropy || (spawn_len > 0 && !spawn_key)))
+        return fail(h, MPCB_ERR_INVALID, "PCG64 seeding: null seed words");
+    return MPCB_OK;
+}
+
+// a PCG64 record as numpy could hold it: has_uint32 0/1, uinteger of 32 bits, inc odd
+static int check_pcg64_states(mpcb_handle *h, int64_t N, const uint64_t *pcg_state) {
+    for (int64_t n = 0; n < N; ++n) {
+        const uint64_t *r = pcg_state + n * mpcb::kPcgWords;
+        if (r[4] > 1 || r[5] > 0xffffffffull || !(r[3] & 1))
+            return fail(h, MPCB_ERR_INVALID, "PCG64 closed loop: robot %lld has a record numpy cannot hold (has_uint32 %llu, "
+                        "uinteger %llu, inc %s)", (long long)n, (unsigned long long)r[4], (unsigned long long)r[5],
+                        (r[3] & 1) ? "odd" : "even");
+    }
+    return MPCB_OK;
+}
+
 // device pointers throughout, except the event script (checked by the caller with check_events), which is copied into
-// handle scratch here; events / out_final / rng_state may be null
+// handle scratch here; events / out_final / rng_state / pcg_state may be null (at most one of the last two is not)
 static int held_loop_core(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, const double *init,
                           const double *target, const double *origin, const double *first_threshold,
                           const int32_t *slow_steps, const mpcb_loop_event *events, int n_events, double radius_u_turn,
                           uint32_t *rng_state, double *out_log, int32_t *out_ticks, int32_t *out_status,
-                          double *out_final) {
+                          double *out_final, uint64_t *pcg_state = nullptr) {
     if (!h || !p) return MPCB_ERR_INVALID;
     if (N < 0 || N >= (1LL << 31)) return fail(h, MPCB_ERR_INVALID, "N out of range");
     if (N == 0) return MPCB_OK;
@@ -860,6 +891,7 @@ static int held_loop_core(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, 
     a.slow_steps = slow_steps; a.out_log = out_log; a.out_ticks = out_ticks; a.out_status = out_status;
     a.events = d_events; a.n_events = d_events ? n_events : 0; a.radius_u_turn = radius_u_turn; a.out_final = out_final;
     a.rng_state = rng_state;
+    a.pcg_state = reinterpret_cast<unsigned long long *>(pcg_state);
     CK(launch_held_loop(h->stream, a, h->sms));
     h->stats = mpcb_stats{};
     h->stats.kernel_launches = 1;
@@ -881,14 +913,24 @@ int mpcb_held_closed_loop_host(mpcb_handle *h, const mpcb_loop_params *p, int64_
                                              out_log, out_ticks, out_status, nullptr);
 }
 
+// the PCG64 generators of held_loop_host: copied in from state_in[N][6] or seeded on the device from SeedSequence
+// words (entropy != null, as for mpcb_pcg64_seed_device); state_out[N][6] (nullable) receives them after the run
+struct PcgSource {
+    const uint64_t *state_in = nullptr;
+    const uint32_t *entropy = nullptr, *spawn_key = nullptr;
+    int32_t entropy_len = 0, entropy_stride = 0, spawn_len = 0;
+    uint64_t *state_out = nullptr;
+    bool any() const { return state_in || entropy; }
+};
+
 // host pointers.  The actual run's generators are copied in from rng_in[N][625] or seeded on the device from keys
-// (key_len as for mpcb_rng_seed_device); with neither, the loop is the noise-free one.  rng_out[N][625] (nullable)
-// receives the generators' states after the run.
+// (key_len as for mpcb_rng_seed_device), or are PCG64 ones (pcg); with none of them, the loop is the noise-free one.
+// rng_out[N][625] (nullable) receives the MT19937 generators' states after the run.
 static int held_loop_host(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, const double *init, const double *target,
                           const double *origin, const double *first_threshold, const int32_t *slow_steps,
                           const mpcb_loop_event *events, int32_t n_events, double radius_u_turn, const uint32_t *rng_in,
                           const uint32_t *keys, int32_t key_len, uint32_t *rng_out, double *out_log, int32_t *out_ticks,
-                          int32_t *out_status, double *out_final) {
+                          int32_t *out_status, double *out_final, const PcgSource &pcg = PcgSource()) {
     int rc = check_events(h, events, n_events);
     if (rc) return rc;
     if (N <= 0) return N == 0 ? MPCB_OK : fail(h, MPCB_ERR_INVALID, "N < 0");
@@ -929,15 +971,35 @@ static int held_loop_host(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, 
         CK(cudaMemcpyAsync(h->loop_keys.p, keys, sizeof(uint32_t) * nkeys, cudaMemcpyHostToDevice, st));
         CK(launch_rng_seed(st, N, h->loop_keys.as<unsigned>(), key_len, h->loop_rng.as<unsigned>()));
     }
+    const size_t npcg = (size_t)N * mpcb::kPcgWords;
+    if (pcg.any()) CK(h->loop_pcg.ensure(sizeof(uint64_t) * npcg));
+    if (pcg.state_in)
+        CK(cudaMemcpyAsync(h->loop_pcg.p, pcg.state_in, sizeof(uint64_t) * npcg, cudaMemcpyHostToDevice, st));
+    if (pcg.entropy) {      // the entropy words go to loop_keys, the spawn-key words to loop_pcg_spawn
+        const size_t nent = (size_t)(pcg.entropy_stride ? N : 1) * pcg.entropy_len;
+        CK(h->loop_keys.ensure(sizeof(uint32_t) * nent));
+        CK(cudaMemcpyAsync(h->loop_keys.p, pcg.entropy, sizeof(uint32_t) * nent, cudaMemcpyHostToDevice, st));
+        const unsigned *d_spawn = nullptr;
+        if (pcg.spawn_len > 0) {
+            const size_t nsp = (size_t)N * pcg.spawn_len;
+            CK(h->loop_pcg_spawn.ensure(sizeof(uint32_t) * nsp));
+            CK(cudaMemcpyAsync(h->loop_pcg_spawn.p, pcg.spawn_key, sizeof(uint32_t) * nsp, cudaMemcpyHostToDevice, st));
+            d_spawn = h->loop_pcg_spawn.as<unsigned>();
+        }
+        CK(launch_pcg64_seed(st, N, h->loop_keys.as<unsigned>(), pcg.entropy_len, pcg.entropy_stride, d_spawn,
+                             pcg.spawn_len, h->loop_pcg.as<unsigned long long>()));
+    }
     if (out_final) CK(h->loop_final.ensure(sizeof(double) * 6 * N));
     CK(cudaMemsetAsync(h->loop_log.p, 0xFF, sizeof(double) * nlog, st));     // NaN pattern for the rows no tick wrote
     rc = held_loop_core(h, p, N, h->in_state.as<double>(), h->in_target.as<double>(), h->in_origin.as<double>(), d_thr,
                         d_slow, events, n_events, radius_u_turn, noise ? h->loop_rng.as<uint32_t>() : nullptr,
                         h->loop_log.as<double>(), h->loop_ticks.as<int>(), h->loop_status.as<int>(),
-                        out_final ? h->loop_final.as<double>() : nullptr);
+                        out_final ? h->loop_final.as<double>() : nullptr, pcg.any() ? h->loop_pcg.as<uint64_t>() : nullptr);
     if (rc) return rc;
-    if (keys) h->stats.kernel_launches += 1;     // the seeding kernel
+    if (keys || pcg.entropy) h->stats.kernel_launches += 1;     // the seeding kernel
     if (rng_out) CK(cudaMemcpyAsync(rng_out, h->loop_rng.p, sizeof(uint32_t) * nrng, cudaMemcpyDeviceToHost, st));
+    if (pcg.state_out)
+        CK(cudaMemcpyAsync(pcg.state_out, h->loop_pcg.p, sizeof(uint64_t) * npcg, cudaMemcpyDeviceToHost, st));
     if (out_final) CK(cudaMemcpyAsync(out_final, h->loop_final.p, sizeof(double) * 6 * N, cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(out_log, h->loop_log.p, sizeof(double) * nlog, cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(out_ticks, h->loop_ticks.p, sizeof(int) * N, cudaMemcpyDeviceToHost, st));
@@ -1007,6 +1069,66 @@ int mpcb_rng_seed_device(mpcb_handle *h, int64_t N, const uint32_t *keys, int32_
     if (!rng_state) return fail(h, MPCB_ERR_INVALID, "seeding: null rng_state");
     CK(cudaSetDevice(h->device));
     CK(launch_rng_seed(h->stream, N, keys, key_len, rng_state));
+    return MPCB_OK;
+}
+
+int mpcb_held_closed_loop_pcg64_host(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, const double *init,
+                                     const double *target, const double *origin, const double *first_threshold,
+                                     const int32_t *slow_steps, const mpcb_loop_event *events, int32_t n_events,
+                                     double radius_u_turn, uint64_t *pcg_state, double *out_log, int32_t *out_ticks,
+                                     int32_t *out_status, double *out_final) {
+    if (!h || !p) return MPCB_ERR_INVALID;
+    if (!pcg_state) return fail(h, MPCB_ERR_INVALID, "PCG64 closed loop: null pcg_state");
+    int rc = check_pcg64_states(h, N, pcg_state);
+    if (rc) return rc;
+    PcgSource pcg;
+    pcg.state_in = pcg_state;
+    pcg.state_out = pcg_state;
+    return held_loop_host(h, p, N, init, target, origin, first_threshold, slow_steps, events, n_events, radius_u_turn,
+                          nullptr, nullptr, 0, nullptr, out_log, out_ticks, out_status, out_final, pcg);
+}
+
+int mpcb_held_closed_loop_pcg64_device(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, const double *init,
+                                       const double *target, const double *origin, const double *first_threshold,
+                                       const int32_t *slow_steps, const mpcb_loop_event *events, int32_t n_events,
+                                       double radius_u_turn, uint64_t *pcg_state, double *out_log, int32_t *out_ticks,
+                                       int32_t *out_status, double *out_final) {
+    if (!h || !p) return MPCB_ERR_INVALID;
+    int rc = check_events(h, events, n_events);
+    if (rc) return rc;
+    if (!pcg_state) return fail(h, MPCB_ERR_INVALID, "PCG64 closed loop: null pcg_state");
+    return held_loop_core(h, p, N, init, target, origin, first_threshold, slow_steps, events, n_events, radius_u_turn,
+                          nullptr, out_log, out_ticks, out_status, out_final, pcg_state);
+}
+
+int mpcb_held_closed_loop_pcg64_seeded_host(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, const double *init,
+                                            const double *target, const double *origin, const double *first_threshold,
+                                            const int32_t *slow_steps, const mpcb_loop_event *events, int32_t n_events,
+                                            double radius_u_turn, const uint32_t *entropy, int32_t entropy_len,
+                                            int32_t entropy_stride, const uint32_t *spawn_key, int32_t spawn_len,
+                                            uint64_t *pcg_state_out, double *out_log, int32_t *out_ticks,
+                                            int32_t *out_status, double *out_final) {
+    if (!h || !p) return MPCB_ERR_INVALID;
+    int rc = check_pcg64_seeds(h, N, entropy, entropy_len, entropy_stride, spawn_key, spawn_len);
+    if (rc) return rc;
+    PcgSource pcg;
+    pcg.entropy = entropy; pcg.entropy_len = entropy_len; pcg.entropy_stride = entropy_stride;
+    pcg.spawn_key = spawn_len > 0 ? spawn_key : nullptr; pcg.spawn_len = spawn_len;
+    pcg.state_out = pcg_state_out;
+    return held_loop_host(h, p, N, init, target, origin, first_threshold, slow_steps, events, n_events, radius_u_turn,
+                          nullptr, nullptr, 0, nullptr, out_log, out_ticks, out_status, out_final, pcg);
+}
+
+int mpcb_pcg64_seed_device(mpcb_handle *h, int64_t N, const uint32_t *entropy, int32_t entropy_len,
+                           int32_t entropy_stride, const uint32_t *spawn_key, int32_t spawn_len, uint64_t *pcg_state) {
+    if (!h) return MPCB_ERR_INVALID;
+    int rc = check_pcg64_seeds(h, N, entropy, entropy_len, entropy_stride, spawn_key, spawn_len);
+    if (rc) return rc;
+    if (N == 0) return MPCB_OK;
+    if (!pcg_state) return fail(h, MPCB_ERR_INVALID, "PCG64 seeding: null pcg_state");
+    CK(cudaSetDevice(h->device));
+    CK(launch_pcg64_seed(h->stream, N, entropy, entropy_len, entropy_stride, spawn_len > 0 ? spawn_key : nullptr,
+                         spawn_len, reinterpret_cast<unsigned long long *>(pcg_state)));
     return MPCB_OK;
 }
 

@@ -65,7 +65,7 @@ struct mpcb_handle_s {
     unsigned cand_cap = 1u << 20;       // entries of that list (option "candidate_list"; 0 = evaluate where found)
     bool cand_auto = true;              // not set by the user: the prefix algorithm with a node list runs without it
     mpcb::DevBuf nccl_scratch;          // split tree: this rank's (cost, index) records + one slot per rank
-    mpcb::DevBuf loop_log, loop_ticks, loop_status, loop_events, loop_final, loop_rng, loop_keys, small_in, small_out, fl_last, fl_k, fl_have, fl_flags, fl_count;
+    mpcb::DevBuf loop_log, loop_ticks, loop_status, loop_events, loop_final, loop_rng, loop_keys, loop_pcg, loop_pcg_spawn, small_in, small_out, fl_last, fl_k, fl_have, fl_flags, fl_count;
     void *pin_in = nullptr, *pin_out = nullptr;   // pinned staging of the low-latency path
     size_t pin_in_cap = 0, pin_out_cap = 0;
     mpcb_stats stats{};

@@ -13,14 +13,17 @@
 // reloads target, line and cost constants from shared memory.
 // The "actual" run (math_mpc(..., True)) gives every robot its own numpy RandomState (key[624] + pos, mpcb_noise.cuh):
 // the CTA keeps it in shared memory while it runs the robot, and thread 0 perturbs the applied (v, beta) after every
-// tick, draw for draw as the reference does.  A template flag keeps the noise-free loop free of all of it.
-// rng_seed_kernel builds those generators on the device from numpy's integer seeds or keys.
+// tick, draw for draw as the reference does.  A robot may instead draw from numpy's Generator(PCG64) (mpcb_pcg64.cuh):
+// its 6-word record lives in thread 0's registers while the CTA runs the robot -- no shared memory, no twist.  The
+// generator kind is a template parameter, so the noise-free loop stays free of all of it.
+// rng_seed_kernel / pcg64_seed_kernel build those generators on the device from numpy's seeds.
 //
 // A HELD tick is tiny (S <= 451 candidates x H steps), so the loop is latency-bound, not
 // throughput-bound: everything is evaluated directly in float64 with the reference's formula and
 // operation order -- no fp32 stage, no refinement -- and the batch dimension (robots) fills the GPU.
 #include "mpcb_events.cuh"
 #include "mpcb_noise.cuh"
+#include "mpcb_pcg64.cuh"
 
 #include <cmath>
 
@@ -148,7 +151,9 @@ __device__ __forceinline__ void load_cost(LoopCost &cost, const double *target, 
     cost.kind = kind;
 }
 
-template <bool kNoise>
+enum LoopGen { kGenNone = 0, kGenMt19937 = 1, kGenPcg64 = 2 };    // the actual run's generator kind
+
+template <int kGen>
 __global__ void __launch_bounds__(kLoopThreads) held_loop_kernel(const LoopArgs a) {
     __shared__ double s_V[kMaxWin], s_B[kMaxWin], s_tanB[kMaxWin];
     __shared__ double s_J[kLoopThreads / 32];
@@ -162,7 +167,7 @@ __global__ void __launch_bounds__(kLoopThreads) held_loop_kernel(const LoopArgs 
     // a flag: every thread compares it with its own copy after the tick's last barrier, so it never has to be cleared)
     __shared__ double s_line[4];
     __shared__ int s_events;
-    extern __shared__ unsigned s_mt[];  // kNoise: the running robot's generator, key[624] + pos (dynamic, kMtWords words)
+    extern __shared__ unsigned s_mt[];  // MT19937: the running robot's generator, key[624] + pos (dynamic, kMtWords words)
     const mpcb_loop_params &p = a.p;
     const int tid = threadIdx.x;
     if (tid == 0) s_events = 0;
@@ -178,12 +183,14 @@ __global__ void __launch_bounds__(kLoopThreads) held_loop_kernel(const LoopArgs 
         bool recursive = false, have_traj = false;
         double opt[3 * MPCB_MAX_H], res_v = 0.0, res_beta = 0.0;
         double xprev = 0.0, yprev = 0.0;
+        Pcg64 pcg;                                 // PCG64: the running robot's generator (thread 0)
         __syncthreads();                           // the previous robot's shared state has been consumed
         if (tid == 0) {
             for (int k = 0; k < 5; ++k) s_state[k] = a.init[5 * n + k];
             xprev = s_state[0]; yprev = s_state[1];
+            if constexpr (kGen == kGenPcg64) pcg = pcg64_load(a.pcg_state + (size_t)n * kPcgWords);
         }
-        if constexpr (kNoise)
+        if constexpr (kGen == kGenMt19937)
             for (int i = tid; i < kMtWords; i += kLoopThreads) s_mt[i] = a.rng_state[(size_t)n * kMtWords + i];
         __syncthreads();
 
@@ -238,9 +245,12 @@ __global__ void __launch_bounds__(kLoopThreads) held_loop_kernel(const LoopArgs 
                     // the applied (v, beta): the commanded ones, or in the actual run what the actuators make of them
                     // (math_model_tree.py:590-597) -- velocity drawn first, then beta, and before the stall stop
                     double av = res_v, ab = res_beta;
-                    if constexpr (kNoise) {
+                    if constexpr (kGen == kGenMt19937) {
                         av = actual_velocity(res_v, s_mt);
                         ab = actual_beta(res_beta, s_mt);
+                    } else if constexpr (kGen == kGenPcg64) {
+                        av = actual_velocity(res_v, pcg);
+                        ab = actual_beta(res_beta, pcg);
                     }
                     double *log = a.out_log + ((size_t)n * p.max_ticks + ticks) * 5;
                     log[0] = rx; log[1] = ry; log[2] = rphi; log[3] = av; log[4] = ab;
@@ -277,8 +287,9 @@ __global__ void __launch_bounds__(kLoopThreads) held_loop_kernel(const LoopArgs 
                 double *f = a.out_final + 6 * n;
                 f[0] = cost.xt; f[1] = cost.yt; f[2] = cost.ox; f[3] = cost.oy; f[4] = (double)slow_steps; f[5] = (double)m;
             }
+            if constexpr (kGen == kGenPcg64) pcg64_store(pcg, a.pcg_state + (size_t)n * kPcgWords);
         }
-        if constexpr (kNoise)       // thread 0's last draw came before the barrier that ended the loop
+        if constexpr (kGen == kGenMt19937)       // thread 0's last draw came before the barrier that ended the loop
             for (int i = tid; i < kMtWords; i += kLoopThreads) a.rng_state[(size_t)n * kMtWords + i] = s_mt[i];
     }
 }
@@ -296,6 +307,25 @@ __global__ void __launch_bounds__(128) rng_seed_kernel(long long N, const unsign
 
 cudaError_t launch_rng_seed(cudaStream_t st, long long N, const unsigned *keys, int key_len, unsigned *rng_state) {
     rng_seed_kernel<<<(unsigned)((N + 127) / 128), 128, 0, st>>>(N, keys, key_len, rng_state);
+    return cudaGetLastError();
+}
+
+// The Generator(PCG64) records of the actual run, seeded as default_rng(SeedSequence(entropy, spawn_key)): one thread per
+// generator hashes its words into the 4-word pool and writes its [6] record.  entropy[ent_len] is shared by all
+// generators (ent_stride 0) or one row per generator (ent_stride = ent_len); spawn[N][spawn_len] (spawn_len 0: none).
+__global__ void __launch_bounds__(128) pcg64_seed_kernel(long long N, const unsigned *entropy, int ent_len,
+                                                         int ent_stride, const unsigned *spawn, int spawn_len,
+                                                         unsigned long long *pcg_state) {
+    const long long n = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (n >= N) return;
+    pcg64_seed(entropy + (size_t)n * ent_stride, ent_len, spawn ? spawn + (size_t)n * spawn_len : nullptr, spawn_len,
+               pcg_state + (size_t)n * kPcgWords);
+}
+
+cudaError_t launch_pcg64_seed(cudaStream_t st, long long N, const unsigned *entropy, int ent_len, int ent_stride,
+                              const unsigned *spawn, int spawn_len, unsigned long long *pcg_state) {
+    pcg64_seed_kernel<<<(unsigned)((N + 127) / 128), 128, 0, st>>>(N, entropy, ent_len, ent_stride, spawn, spawn_len,
+                                                                   pcg_state);
     return cudaGetLastError();
 }
 
@@ -479,21 +509,23 @@ cudaError_t launch_full_apply(cudaStream_t st, const FullLoopArgs &a) {
     return cudaGetLastError();
 }
 
-template <bool kNoise>
+template <int kGen>
 static cudaError_t launch_held_loop_t(cudaStream_t st, const LoopArgs &a, int sms) {
-    const size_t smem = kNoise ? sizeof(unsigned) * kMtWords : 0;
+    const size_t smem = kGen == kGenMt19937 ? sizeof(unsigned) * kMtWords : 0;
     int per_sm = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, held_loop_kernel<kNoise>, kLoopThreads, smem) != cudaSuccess ||
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, held_loop_kernel<kGen>, kLoopThreads, smem) != cudaSuccess ||
         per_sm < 1)
         per_sm = 1;
     long long grid = (long long)sms * per_sm;
     if (grid > a.N) grid = a.N;
-    held_loop_kernel<kNoise><<<(unsigned)grid, kLoopThreads, smem, st>>>(a);
+    held_loop_kernel<kGen><<<(unsigned)grid, kLoopThreads, smem, st>>>(a);
     return cudaGetLastError();
 }
 
 cudaError_t launch_held_loop(cudaStream_t st, const LoopArgs &a, int sms) {
-    return a.rng_state ? launch_held_loop_t<true>(st, a, sms) : launch_held_loop_t<false>(st, a, sms);
+    if (a.rng_state) return launch_held_loop_t<kGenMt19937>(st, a, sms);
+    if (a.pcg_state) return launch_held_loop_t<kGenPcg64>(st, a, sms);
+    return launch_held_loop_t<kGenNone>(st, a, sms);
 }
 
 }  // namespace mpcb

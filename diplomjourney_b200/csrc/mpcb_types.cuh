@@ -267,6 +267,7 @@ struct LoopArgs {
     double radius_u_turn;
     double *out_final;                                 // [N][6] x_t, y_t, x_0, y_0, steps_for_slowing, m; nullable
     unsigned *rng_state;                               // [N][625] numpy MT19937 key + pos, updated in place; null: no noise
+    unsigned long long *pcg_state;                     // [N][6] numpy PCG64 records, updated in place (with rng_state null)
 };
 
 // one online tick of a batch of robots with per-robot acceleration windows (mpcb_loop.cu); all pointers are device

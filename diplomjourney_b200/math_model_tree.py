@@ -203,21 +203,28 @@ def vector_of_beta_angles(actual_beta):
     return [pa for pa in window if abs(pa) <= (beta_max + math.radians(eps_beta))]
 
 
+def _randint(rng, lo, hi):
+    """randint(lo, hi) of a RandomState; a numpy Generator draws the same range with integers(lo, hi)."""
+    if isinstance(rng, np.random.Generator):
+        return int(rng.integers(lo, hi))
+    return rng.randint(lo, hi)
+
+
 def get_actual_velocity(velocity_ref, rng=None):
-    """Actuator disturbance (math_model_tree.py:259-267).  ``rng``: a numpy RandomState standing in for the
+    """Actuator disturbance (math_model_tree.py:259-267).  ``rng``: a numpy RandomState or Generator standing in for the
     module-level generator (one per robot in ``math_mpc_batch``)."""
     rng = random if rng is None else rng
     if rng.random() < 0.7:
         if velocity_ref < 0.4:
-            return velocity_ref + (rng.randint(0, 5) / 1000)
-        return velocity_ref + (rng.randint(-100, 10) / 1000)
+            return velocity_ref + (_randint(rng, 0, 5) / 1000)
+        return velocity_ref + (_randint(rng, -100, 10) / 1000)
     return velocity_ref
 
 
 def get_actual_beta_angle(beta_ref, rng=None):
     rng = random if rng is None else rng
     if rng.random() < 0.7:
-        return beta_ref + math.radians(rng.randint(-5, 5))
+        return beta_ref + math.radians(_randint(rng, -5, 5))
     return beta_ref
 
 
@@ -477,14 +484,43 @@ def _pack_generators(gens):
     return out
 
 
-def _math_mpc_batch_device_noise(params, ini, tgt, org, first, rngs, events, seeds=None):
+def _generator_kind(rngs):
+    """"mt19937" when every entry is a RandomState, "pcg64" when every entry is a Generator over PCG64; anything else
+    is a TypeError that names the offending type."""
+    kinds = set()
+    for g in rngs:
+        if isinstance(g, np.random.RandomState):
+            kinds.add("mt19937")
+        elif isinstance(g, np.random.Generator):
+            if type(g.bit_generator) is not np.random.PCG64:
+                raise TypeError("rngs entries that are numpy Generators must draw from PCG64 (np.random.default_rng), "
+                                f"not {type(g.bit_generator).__name__}")
+            kinds.add("pcg64")
+        else:
+            raise TypeError(f"rngs entries must be numpy RandomState or Generator(PCG64), not {type(g)!r}")
+    if len(kinds) > 1:
+        raise TypeError("rngs mixes numpy RandomState and Generator(PCG64) entries: the device loop runs one kind")
+    return kinds.pop() if kinds else "mt19937"
+
+
+def _math_mpc_batch_device_noise(params, ini, tgt, org, first, rngs, events, seeds=None, kind="mt19937"):
     """The actual run on the device (mpcb_held_closed_loop_actual): each robot draws from its own generator, whose state
     goes to the device as get_state() and comes back through set_state (has_gauss / cached_gaussian kept).  With
-    ``seeds`` (already checked by ``_native.seed_keys``) the generators are seeded on the device and stay there."""
+    ``seeds`` (already checked by ``_native.seed_keys``) the generators are seeded on the device and stay there.
+    ``kind="pcg64"``: numpy Generator(PCG64) streams (mpcb_held_closed_loop_pcg64): the bit generators' state, inc,
+    has_uint32 and uinteger go to the device and come back; ``seeds`` then is a SeedSequence or integer seeds."""
     script = ACTUAL_EVENTS if events is True else list(events or ())
+    kw = dict(first_threshold=first, events=script or None, radius_u_turn=radius_u_turn)
+    if kind == "pcg64":
+        if seeds is not None:
+            return _solver().held_closed_loop(params, ini, tgt, org, pcg_seeds=seeds, return_rng_state=False, **kw)
+        r = _solver().held_closed_loop(params, ini, tgt, org,
+                                       pcg_state=np.stack([_native.pcg64_record(g.bit_generator) for g in rngs]), **kw)
+        for g, st in zip(rngs, r.pop("pcg_state")):
+            g.bit_generator.state = _native.pcg64_state(st)
+        return r
     if seeds is not None:
-        return _solver().held_closed_loop(params, ini, tgt, org, first_threshold=first, events=script or None,
-                                          radius_u_turn=radius_u_turn, seeds=seeds, return_rng_state=False)
+        return _solver().held_closed_loop(params, ini, tgt, org, seeds=seeds, return_rng_state=False, **kw)
     gens = [random] if rngs is None else rngs
     r = _solver().held_closed_loop(params, ini, tgt, org, first_threshold=first, events=script or None,
                                    radius_u_turn=radius_u_turn, rng_state=_pack_generators(gens))
@@ -495,7 +531,8 @@ def _math_mpc_batch_device_noise(params, ini, tgt, org, first, rngs, events, see
 
 
 def math_mpc_batch(initial_coordinates, target_coordinates, max_ticks=512, origin=None, cost_kind=None,
-                   isActual=False, rngs=None, events=False, host_loop=False, device_noise=False, seeds=None):
+                   isActual=False, rngs=None, events=False, host_loop=False, device_noise=False, seeds=None,
+                   generator=None):
     """EXTENSION (not in the reference): the closed loop of ``math_mpc`` for a whole batch of robots.
     ``initial_coordinates`` [N][5] = x, y, phi, v, beta; ``target_coordinates`` [N][2].  The tracked line starts at
     the module's x_0, y_0 unless ``origin`` [N][2] is given.
@@ -523,6 +560,12 @@ def math_mpc_batch(initial_coordinates, target_coordinates, max_ticks=512, origi
       row is a key even when K == 1, see ``_native.seed_keys``).  No generator object is built and ``np.random`` is
       not touched; the generators' final states are not returned (``_native.Solver.held_closed_loop(..., seeds=)``
       returns them).  Same result keys as with ``rngs``.
+    * numpy's Generator (PCG64, ``np.random.default_rng``) in place of RandomState: ``rngs`` may be all RandomState or
+      all Generator(PCG64) -- on the per-tick path and with ``device_noise=True``, where the Generators are advanced
+      exactly as the per-tick path advances them.  With ``device_noise=True``, ``seeds=np.random.SeedSequence(...)``
+      gives robot i the stream of ``default_rng(seeds.spawn(N)[i])`` and advances ``seeds`` as ``spawn(N)`` does;
+      integer ``seeds`` with ``generator="pcg64"`` give robot i ``default_rng(seeds[i])`` (without the selector
+      integer seeds keep their RandomState meaning).
 
     Returns dict(log[N][max_ticks][5], ticks[N], status[N])."""
     from . import config as _cfg
@@ -530,12 +573,23 @@ def math_mpc_batch(initial_coordinates, target_coordinates, max_ticks=512, origi
     org = np.array([[x_0, y_0]], dtype=np.float64) if origin is None else np.asarray(origin, np.float64).reshape(-1, 2)
     tgt = np.asarray(target_coordinates, dtype=np.float64).reshape(-1, 2)
     n = ini.shape[0]
+    kind = "mt19937"
+    if generator not in (None, "mt19937", "pcg64"):
+        raise ValueError(f"generator must be 'mt19937' or 'pcg64', not {generator!r}")
+    if generator is not None and seeds is None:
+        raise ValueError("generator= says which stream integer seeds= start; rngs= carry their own kind")
     if seeds is not None:
         if rngs is not None:
             raise ValueError("seeds and rngs both give the robots' generators: pass one of them")
         if not device_noise:
             raise ValueError("seeds seed the generators on the device: they need isActual=True, device_noise=True")
-        seeds = _native.seed_keys(seeds, n)[0]
+        if isinstance(seeds, np.random.SeedSequence) or generator == "pcg64":
+            if generator == "mt19937":
+                raise ValueError("a SeedSequence seeds numpy's Generator(PCG64), not the legacy RandomState")
+            _native.pcg64_seed_words(seeds, n)          # numpy's refusals, before any solver is touched
+            kind = "pcg64"
+        else:
+            seeds = _native.seed_keys(seeds, n)[0]
     if device_noise:
         if not isActual:
             raise ValueError("device_noise=True is the actual run's actuator noise: it needs isActual=True")
@@ -549,9 +603,7 @@ def math_mpc_batch(initial_coordinates, target_coordinates, max_ticks=512, origi
             rngs = list(rngs)
             if len(rngs) != n:
                 raise ValueError(f"rngs holds {len(rngs)} generators for {n} robots")
-            for g in rngs:
-                if not isinstance(g, np.random.RandomState):
-                    raise TypeError(f"rngs entries must be numpy RandomState (the legacy MT19937 stream), not {type(g)!r}")
+            kind = _generator_kind(rngs)
     org = np.broadcast_to(org, (n, 2))
     tgt = np.broadcast_to(tgt, (n, 2))
     # optimal_criterion before the first tick = control_criterion of the line origin (math_model_tree.py:676)
@@ -567,7 +619,7 @@ def math_mpc_batch(initial_coordinates, target_coordinates, max_ticks=512, origi
     params = _native.LoopParams.from_config(_cfg, _native.COST_TREE if cost_kind is None else cost_kind,
                                             prediction_horizon, max_ticks)
     if device_noise:
-        return _math_mpc_batch_device_noise(params, ini, tgt, org, first, rngs, events, seeds)
+        return _math_mpc_batch_device_noise(params, ini, tgt, org, first, rngs, events, seeds, kind)
     if isActual or host_loop:
         if not isinstance(events, bool) and events is not None:
             raise ValueError("a custom event script runs on the device loop only (isActual=False, host_loop=False); "

@@ -299,6 +299,56 @@ MPCB_API int mpcb_held_closed_loop_seeded_host(mpcb_handle *h, const mpcb_loop_p
                                       const uint32_t *keys, int32_t key_len, uint32_t *rng_state_out,
                                       double *out_log, int32_t *out_ticks, int32_t *out_status, double *out_final);
 
+/* The actual run with numpy's Generator(PCG64) stream (np.random.default_rng) in place of the legacy RandomState: the
+ * same loop, events and draw order as mpcb_held_closed_loop_actual_host (velocity: one random(), then integers(0, 5)
+ * under 0.4 m/s, else integers(-100, 10); beta: one random(), then integers(-5, 5)), drawn as numpy's Generator draws
+ * them -- random() from one 64-bit output, integers() by Lemire's method on 32-bit draws that keep the unused upper half
+ * of a 64-bit output for the next 32-bit draw.
+ *   pcg_state[N][6]  in/out: per robot Generator.bit_generator.state as six uint64 words: state >> 64, state mod 2^64,
+ *                    inc >> 64, inc mod 2^64, has_uint32, uinteger; on return the state after the robot's draws.  NULL,
+ *                    has_uint32 outside {0, 1}, uinteger >= 2^32 or an even inc is MPCB_ERR_INVALID (checked before
+ *                    anything is copied). */
+MPCB_API int mpcb_held_closed_loop_pcg64_host(mpcb_handle *h, const mpcb_loop_params *p, int64_t N,
+                                     const double *init, const double *target, const double *origin,
+                                     const double *first_threshold, const int32_t *slow_steps,
+                                     const mpcb_loop_event *events, int32_t n_events, double radius_u_turn,
+                                     uint64_t *pcg_state,
+                                     double *out_log, int32_t *out_ticks, int32_t *out_status, double *out_final);
+/* Device flavour of mpcb_held_closed_loop_pcg64_host, as mpcb_held_closed_loop_actual_device is of the MT19937 entry:
+ * device pointers (pcg_state in/out), the event script a host array, enqueued without a sync, out_log rows after a
+ * robot's last tick not written.  The records are not checked (that would need a copy).  A null pcg_state is
+ * MPCB_ERR_INVALID. */
+MPCB_API int mpcb_held_closed_loop_pcg64_device(mpcb_handle *h, const mpcb_loop_params *p, int64_t N,
+                                       const double *init, const double *target, const double *origin,
+                                       const double *first_threshold, const int32_t *slow_steps,
+                                       const mpcb_loop_event *events, int32_t n_events, double radius_u_turn,
+                                       uint64_t *pcg_state,
+                                       double *out_log, int32_t *out_ticks, int32_t *out_status, double *out_final);
+/* The Generator(PCG64) records seeded on the device as numpy seeds them: pcg_state[N][6] receives, per robot, the state
+ * of default_rng(SeedSequence(entropy, spawn_key)) (has_uint32 = uinteger = 0).  SeedSequence works on 32-bit words:
+ *   entropy      the entropy's little-endian words (an integer expands into as many words as it needs, 0 into one;
+ *                a sequence of integers into the concatenation of theirs); 1 <= entropy_len <= 4096
+ *   entropy_stride  0: entropy[entropy_len] is shared by all robots; entropy_len: entropy[N][entropy_len], one row each
+ *   spawn_key    [N][spawn_len] the words of each robot's spawn key, 0 <= spawn_len <= 4096 (0: no spawn key, and
+ *                spawn_key may be NULL).  SeedSequence(root).spawn(N)[i] has root's entropy and the spawn key
+ *                root.spawn_key + (root.n_children_spawned + i,).
+ * Device pointers, enqueued on the handle's stream without a sync.  Other lengths or strides, N < 0 (or N >= 2^31), or a
+ * null pointer that is needed with N > 0 is MPCB_ERR_INVALID; N == 0 launches nothing. */
+MPCB_API int mpcb_pcg64_seed_device(mpcb_handle *h, int64_t N, const uint32_t *entropy, int32_t entropy_len,
+                                    int32_t entropy_stride, const uint32_t *spawn_key, int32_t spawn_len,
+                                    uint64_t *pcg_state);
+/* mpcb_held_closed_loop_pcg64_host with the generators seeded on the device from SeedSequence words (as for
+ * mpcb_pcg64_seed_device, host pointers) in place of pcg_state.
+ *   pcg_state_out[N][6]  (nullable) the generators' states after the run; NULL = they are not copied back */
+MPCB_API int mpcb_held_closed_loop_pcg64_seeded_host(mpcb_handle *h, const mpcb_loop_params *p, int64_t N,
+                                            const double *init, const double *target, const double *origin,
+                                            const double *first_threshold, const int32_t *slow_steps,
+                                            const mpcb_loop_event *events, int32_t n_events, double radius_u_turn,
+                                            const uint32_t *entropy, int32_t entropy_len, int32_t entropy_stride,
+                                            const uint32_t *spawn_key, int32_t spawn_len, uint64_t *pcg_state_out,
+                                            double *out_log, int32_t *out_ticks, int32_t *out_status,
+                                            double *out_final);
+
 /* ONE online tick for a batch of robots that each have their OWN acceleration window (SURVEY 8f row f2).  The
  * reference rebuilds the control window per robot and per tick around the robot's current (v, beta)
  * (vector_of_velocities / vector_of_beta_angles, math_model_tree.py:239-256, called at :543-545 and -- with the noisy
