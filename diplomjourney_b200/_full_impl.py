@@ -150,19 +150,21 @@ def install(g, placeholder_trajectory):
         g.update(x=x, y=y, phi=phi, v=v, beta=beta)
         return path
 
-    def run_batch(scenarios, max_ticks=256):
+    def run_batch(scenarios, max_ticks=256, trace=False):
         """EXTENSION (not in the reference): the closed loop of run_math_model.py:233-276 for a whole batch of
         scenarios at once -- rows of [x_0, y_0, phi_0, x_t, y_t]; the tracked line starts at each robot's start
         pose and ``optimal_criterion`` is seeded from it, as run_math_model.py:251-252 does.  Every tick is ONE
         batched FULL solve on the GPU with the carried thresholds; per-robot bookkeeping (repeat counter,
-        is_on_target) stays on the device.  Returns dict(log[N][max_ticks][5], ticks[N], status[N])."""
+        is_on_target) stays on the device.  Returns dict(log[N][max_ticks][5], ticks[N], status[N]); ``trace=True``
+        adds per tick pred[N][max_ticks][H][3] (the poses of optimal_trajectory, the previous path again on a stall),
+        control[N][max_ticks][2] and cost[N][max_ticks] (NaN on a stall)."""
         sc = np.asarray(scenarios, dtype=np.float64).reshape(-1, 5)
         first = np.empty(sc.shape[0])
         for i, (sx, sy, sphi, tx, ty) in enumerate(sc):
             ang = np.arctan(tx / ty) - sphi
             first[i] = 10000 * math.sqrt((tx - sx) ** 2 + (ty - sy) ** 2) + 10 * ang ** 2 + 100 * 1000 ** 2
         return _solver().full_closed_loop(_native.COST_MM, g["prediction_horizon"], sc[:, :3], sc[:, 3:5], sc[:, :2],
-                                          first_threshold=first, eps=g["eps"], max_ticks=max_ticks)
+                                          first_threshold=first, eps=g["eps"], max_ticks=max_ticks, trace=trace)
 
     def reset_scenario(x_0, y_0, phi_0, x_t, y_t):
         """run_math_model.py:233-252: new start/target, optimum re-seeded from the start pose."""

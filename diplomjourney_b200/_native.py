@@ -66,6 +66,11 @@ class LoopEvent(C.Structure):
 
 EVENT_NEW_TARGET, EVENT_TURN_LEFT, EVENT_TURN_RIGHT = 1, 2, 3
 
+
+class LoopTrace(C.Structure):
+    """mpcb_loop_trace (include/mpcb200.h): where the next closed-loop call writes its per-tick trace."""
+    _fields_ = [("pred", C.c_void_p), ("control", C.c_void_p), ("cost", C.c_void_p)]
+
 _lib = None
 _dp, _i64p, _u8p, _fp = C.POINTER(C.c_double), C.POINTER(C.c_int64), C.POINTER(C.c_uint8), C.POINTER(C.c_float)
 
@@ -118,6 +123,7 @@ def load():
     lib.mpcb_solve_held_windows_host.argtypes = win
     lib.mpcb_solve_held_windows_device.argtypes = win
     lib.mpcb_full_closed_loop_host.argtypes = [vp, C.c_int, C.c_int, C.c_int64, vp, vp, vp, vp, C.c_double, C.c_int, vp, vp, vp]
+    lib.mpcb_set_loop_trace.argtypes = [vp, C.POINTER(LoopTrace)]
     split = [vp, vp, C.c_int, C.c_int, C.c_int64, vp, vp, vp, vp, vp, vp, vp, vp]
     lib.mpcb_solve_tree_split_host.argtypes = split
     lib.mpcb_solve_tree_split_device.argtypes = split
@@ -322,6 +328,22 @@ class Solver:
     def sync(self):
         self._ck(self.lib.mpcb_sync(self.h))
 
+    def set_loop_trace(self, pred=0, control=0, cost=0):
+        """mpcb_set_loop_trace: the NEXT closed-loop call on this solver writes its per-tick trace to these addresses --
+        pred [N][max_ticks][H][3], control [N][max_ticks][2], cost [N][max_ticks] float64, each 0 = not wanted; host
+        memory for the host entries, device memory (e.g. torch.Tensor.data_ptr()) for the device ones.  That call
+        consumes the trace whether it succeeds or fails; all three 0 clears it."""
+        self._ck(self.lib.mpcb_set_loop_trace(self.h, C.byref(LoopTrace(int(pred) or None, int(control) or None,
+                                                                         int(cost) or None))))
+
+    def _host_trace(self, N, max_ticks, H):
+        """Arrays for a host entry's trace, attached to the next call (immediately before it: nothing may raise
+        between this and the call, or the trace would outlive the arrays)."""
+        tr = dict(pred=np.full((N, max_ticks, H, 3), np.nan), control=np.full((N, max_ticks, 2), np.nan),
+                  cost=np.full((N, max_ticks), np.nan))
+        self.set_loop_trace(*(tr[k].ctypes.data for k in ("pred", "control", "cost")))
+        return tr
+
     def stats(self) -> dict:
         s = Stats()
         self._ck(self.lib.mpcb_get_stats(self.h, C.byref(s)))
@@ -435,7 +457,7 @@ class Solver:
 
     def held_closed_loop(self, params: "LoopParams", init, target, origin, first_threshold=None, slow_steps=None,
                          events=None, radius_u_turn=0.0, rng_state=None, seeds=None, return_rng_state=True,
-                         pcg_state=None, pcg_seeds=None):
+                         pcg_state=None, pcg_seeds=None, trace=False):
         """Whole closed loops of the online controller for a batch of robots on the device
         (mpcb_held_closed_loop_host / _events_host). ``events``: an operator script [(tick, kind, a, b), ...] with kind
         EVENT_NEW_TARGET (a, b = the new target) or EVENT_TURN_LEFT / _RIGHT (a = distance), applied to every robot
@@ -451,7 +473,10 @@ class Solver:
         default_rng(pcg_seeds.spawn(N)[i]) resp. default_rng(pcg_seeds[i]), seeded on the device
         (mpcb_held_closed_loop_pcg64_seeded_host); a SeedSequence is advanced as spawn(N) advances it.
         Returns dict(log[N,max_ticks,5], ticks[N], status[N], final[N,6] = x_t, y_t, x_0, y_0, steps_for_slowing, m),
-        with ``rng_state`` or ``seeds`` also the generators' states after the run (``pcg_state`` with the PCG64 ones)."""
+        with ``rng_state`` or ``seeds`` also the generators' states after the run (``pcg_state`` with the PCG64 ones).
+        ``trace=True`` adds what every tick logs besides the 5-list (see ``mpcb_set_loop_trace``): pred[N,max_ticks,H,3]
+        (the poses of optimal_trajectory), control[N,max_ticks,2] (the commanded v, beta, before actuator noise) and
+        cost[N,max_ticks] (the accepted leaf's cost, NaN on a tick that accepted none); NaN after a robot's last tick."""
         if sum(x is not None for x in (rng_state, seeds, pcg_state, pcg_seeds)) > 1:
             raise ValueError("rng_state, seeds, pcg_state and pcg_seeds each give the generators: pass one of them")
         ini = _arr(init, np.float64, (-1, 5))
@@ -465,12 +490,15 @@ class Solver:
         status = np.empty(N, np.int32)
         ev, n_ev = _event_script(events)
         final = np.empty((N, 6))
+        tr = {}
+        arm = (lambda: tr.update(self._host_trace(N, params.max_ticks, params.H))) if trace else (lambda: None)
         if pcg_seeds is not None or pcg_state is not None:
             common = (self.h, C.byref(params), N, _ptr(ini), _ptr(tg), _ptr(og), _ptr(thr), _ptr(sl), ev, n_ev,
                       float(radius_u_turn))
             if pcg_seeds is not None:
                 ent, stride, spawn = pcg64_seed_words(pcg_seeds, N)
                 ps = np.empty((N, PCG64_WORDS), np.uint64) if return_rng_state else None
+                arm()
                 self._ck(self.lib.mpcb_held_closed_loop_pcg64_seeded_host(
                     *common, _ptr(ent), ent.shape[-1], stride, _ptr(spawn), 0 if spawn is None else spawn.shape[1],
                     _ptr(ps), _ptr(log), _ptr(ticks), _ptr(status), _ptr(final)))
@@ -480,35 +508,39 @@ class Solver:
                 ps = np.array(pcg_state, dtype=np.uint64, order="C")        # a copy: the library updates it in place
                 if ps.shape != (N, PCG64_WORDS):
                     raise ValueError(f"pcg_state must be [N][6] = [{N}][6] (see pcg64_record), got {ps.shape}")
+                arm()
                 self._ck(self.lib.mpcb_held_closed_loop_pcg64_host(*common, _ptr(ps), _ptr(log), _ptr(ticks),
                                                                    _ptr(status), _ptr(final)))
-            out = dict(log=log, ticks=ticks, status=status, final=final)
+            out = dict(log=log, ticks=ticks, status=status, final=final, **tr)
             if ps is not None:
                 out["pcg_state"] = ps
             return out
         if seeds is not None:
             keys, key_len = seed_keys(seeds, N)
             rs = np.empty((N, 625), np.uint32) if return_rng_state else None
+            arm()
             self._ck(self.lib.mpcb_held_closed_loop_seeded_host(self.h, C.byref(params), N, _ptr(ini), _ptr(tg), _ptr(og),
                                                                 _ptr(thr), _ptr(sl), ev, n_ev, float(radius_u_turn),
                                                                 _ptr(keys), key_len, _ptr(rs), _ptr(log), _ptr(ticks),
                                                                 _ptr(status), _ptr(final)))
-            out = dict(log=log, ticks=ticks, status=status, final=final)
+            out = dict(log=log, ticks=ticks, status=status, final=final, **tr)
             if return_rng_state:
                 out["rng_state"] = rs
             return out
         if rng_state is None:
+            arm()
             self._ck(self.lib.mpcb_held_closed_loop_events_host(self.h, C.byref(params), N, _ptr(ini), _ptr(tg), _ptr(og),
                                                                 _ptr(thr), _ptr(sl), ev, n_ev, float(radius_u_turn),
                                                                 _ptr(log), _ptr(ticks), _ptr(status), _ptr(final)))
-            return dict(log=log, ticks=ticks, status=status, final=final)
+            return dict(log=log, ticks=ticks, status=status, final=final, **tr)
         rs = np.array(rng_state, dtype=np.uint32, order="C")         # a copy: the library updates it in place
         if rs.shape != (N, 625):
             raise ValueError(f"rng_state must be [N][625] = [{N}][625] (key[624] + pos per robot), got {rs.shape}")
+        arm()
         self._ck(self.lib.mpcb_held_closed_loop_actual_host(self.h, C.byref(params), N, _ptr(ini), _ptr(tg), _ptr(og),
                                                             _ptr(thr), _ptr(sl), ev, n_ev, float(radius_u_turn),
                                                             _ptr(rs), _ptr(log), _ptr(ticks), _ptr(status), _ptr(final)))
-        return dict(log=log, ticks=ticks, status=status, final=final, rng_state=rs)
+        return dict(log=log, ticks=ticks, status=status, final=final, rng_state=rs, **tr)
 
     def seed_generators_device(self, N, keys, key_len, out):
         """mpcb_rng_seed_device: the [N][625] records (key[624] + pos) of RandomState(keys[n]) (key_len == 0, keys[N]
@@ -519,15 +551,18 @@ class Solver:
 
     def held_closed_loop_device_actual(self, params: "LoopParams", N, init, target, origin, first_threshold, slow_steps,
                                        rng_state, out_log, out_ticks, out_status, out_final=None, events=None,
-                                       radius_u_turn=0.0):
+                                       radius_u_turn=0.0, trace=None):
         """mpcb_held_closed_loop_actual_device: the actual run of ``held_closed_loop`` on raw device addresses (init
         [N][5], target / origin [N][2] float64, first_threshold [N] float64 or 0, slow_steps [N] int32 or 0, rng_state
         [N][625] uint32 updated in place, out_log [N][max_ticks][5], out_ticks / out_status [N] int32, out_final [N][6]
         or 0); ``events`` is a host script as for ``held_closed_loop``.  Rows of out_log after a robot's last tick are
-        not written: fill it (with NaN, as the host entry does) beforehand.  Enqueues on self.stream, does not
-        synchronise."""
+        not written: fill it (with NaN, as the host entry does) beforehand.  ``trace``: (pred, control, cost) device
+        addresses as for ``set_loop_trace`` (0 = not wanted), rows after a robot's last tick not written either.
+        Enqueues on self.stream, does not synchronise."""
         vp = lambda x: C.c_void_p(int(x)) if x else None
         ev, n_ev = _event_script(events)
+        if trace is not None:
+            self.set_loop_trace(*trace)
         self._ck(self.lib.mpcb_held_closed_loop_actual_device(self.h, C.byref(params), int(N), vp(init), vp(target),
                                                               vp(origin), vp(first_threshold), vp(slow_steps), ev, n_ev,
                                                               float(radius_u_turn), vp(rng_state), vp(out_log),
@@ -544,21 +579,25 @@ class Solver:
 
     def held_closed_loop_device_pcg64(self, params: "LoopParams", N, init, target, origin, first_threshold, slow_steps,
                                       pcg_state, out_log, out_ticks, out_status, out_final=None, events=None,
-                                      radius_u_turn=0.0):
+                                      radius_u_turn=0.0, trace=None):
         """mpcb_held_closed_loop_pcg64_device: ``held_closed_loop_device_actual`` with per-robot Generator(PCG64)
-        records, pcg_state [N][6] uint64 updated in place (raw device addresses).  Enqueues on self.stream, does not
-        synchronise."""
+        records, pcg_state [N][6] uint64 updated in place (raw device addresses), ``trace`` likewise.  Enqueues on
+        self.stream, does not synchronise."""
         vp = lambda x: C.c_void_p(int(x)) if x else None
         ev, n_ev = _event_script(events)
+        if trace is not None:
+            self.set_loop_trace(*trace)
         self._ck(self.lib.mpcb_held_closed_loop_pcg64_device(self.h, C.byref(params), int(N), vp(init), vp(target),
                                                              vp(origin), vp(first_threshold), vp(slow_steps), ev, n_ev,
                                                              float(radius_u_turn), vp(pcg_state), vp(out_log),
                                                              vp(out_ticks), vp(out_status), vp(out_final)))
 
-    def full_closed_loop(self, cost, H, init_state, target, origin, first_threshold=None, eps=0.001, max_ticks=256):
+    def full_closed_loop(self, cost, H, init_state, target, origin, first_threshold=None, eps=0.001, max_ticks=256,
+                         trace=False):
         """Closed loop of the FULL-tree scripts for a batch of robots (mpcb_full_closed_loop_host): one batched
         FULL solve per tick with the carried threshold; stops per robot on target / after two repeated
-        positions / at max_ticks. Returns dict(log[N,max_ticks,5], ticks[N], status[N])."""
+        positions / at max_ticks. Returns dict(log[N,max_ticks,5], ticks[N], status[N]); ``trace=True`` adds pred,
+        control and cost as ``held_closed_loop`` does (a stall tick repeats the last accepted trajectory)."""
         ini = _arr(init_state, np.float64, (-1, 3))
         N = ini.shape[0]
         tg = _arr(np.broadcast_to(np.asarray(target, np.float64).reshape(-1, 2), (N, 2)), np.float64)
@@ -567,9 +606,10 @@ class Solver:
         log = np.empty((N, max_ticks, 5))
         ticks = np.empty(N, np.int32)
         status = np.empty(N, np.int32)
+        tr = self._host_trace(N, int(max_ticks), H) if trace else {}
         self._ck(self.lib.mpcb_full_closed_loop_host(self.h, cost, H, N, _ptr(ini), _ptr(tg), _ptr(og), _ptr(thr),
                                                      float(eps), int(max_ticks), _ptr(log), _ptr(ticks), _ptr(status)))
-        return dict(log=log, ticks=ticks, status=status)
+        return dict(log=log, ticks=ticks, status=status, **tr)
 
     def dump_leaves(self, mode, cost, H, state, target, origin, flags=0, algo=ALGO_LEAFWALK, leaf_begin=0, count=None):
         st = _arr(state, np.float64).ravel()[:3].copy()

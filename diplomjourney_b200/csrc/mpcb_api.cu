@@ -294,7 +294,7 @@ int mpcb_destroy(mpcb_handle *h) {
                       &h->lock, &h->ub, &h->tile_list, &h->reduce_scratch, &h->in_state, &h->in_target, &h->in_origin, &h->in_thr, &h->in_flags, &h->out_cost,
                       &h->out_index, &h->out_traj, &h->out_ctl, &h->dump_rec, &h->dump_j, &h->loop_log, &h->loop_ticks,
                       &h->loop_status, &h->loop_events, &h->loop_final, &h->loop_rng, &h->loop_keys, &h->small_in, &h->small_out, &h->fl_last, &h->fl_k, &h->fl_have, &h->fl_flags,
-                      &h->fl_count, &h->nccl_scratch, &h->cand, &h->cand_J, &h->cand_sel, &h->node_list})
+                      &h->fl_count, &h->trace_pred, &h->trace_ctl, &h->trace_cost, &h->fl_traj, &h->nccl_scratch, &h->cand, &h->cand_J, &h->cand_sel, &h->node_list})
         b->release();
     if (h->pin_in) cudaFreeHost(h->pin_in);
     if (h->pin_out) cudaFreeHost(h->pin_out);
@@ -863,13 +863,27 @@ static int check_pcg64_states(mpcb_handle *h, int64_t N, const uint64_t *pcg_sta
     return MPCB_OK;
 }
 
+// the trace of this closed-loop call, detached from the handle: one call consumes it, whatever its outcome
+static mpcb_loop_trace take_trace(mpcb_handle *h) {
+    const mpcb_loop_trace t = h->trace;
+    h->trace = mpcb_loop_trace{};
+    return t;
+}
+
+int mpcb_set_loop_trace(mpcb_handle *h, const mpcb_loop_trace *trace) {
+    if (!h) return MPCB_ERR_INVALID;
+    h->trace = trace ? *trace : mpcb_loop_trace{};
+    return MPCB_OK;
+}
+
 // device pointers throughout, except the event script (checked by the caller with check_events), which is copied into
-// handle scratch here; events / out_final / rng_state / pcg_state may be null (at most one of the last two is not)
+// handle scratch here; events / out_final / rng_state / pcg_state and the trace's members may be null (at most one of
+// rng_state and pcg_state is not)
 static int held_loop_core(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, const double *init,
                           const double *target, const double *origin, const double *first_threshold,
                           const int32_t *slow_steps, const mpcb_loop_event *events, int n_events, double radius_u_turn,
                           uint32_t *rng_state, double *out_log, int32_t *out_ticks, int32_t *out_status,
-                          double *out_final, uint64_t *pcg_state = nullptr) {
+                          double *out_final, uint64_t *pcg_state, const mpcb_loop_trace &tr) {
     if (!h || !p) return MPCB_ERR_INVALID;
     if (N < 0 || N >= (1LL << 31)) return fail(h, MPCB_ERR_INVALID, "N out of range");
     if (N == 0) return MPCB_OK;
@@ -892,6 +906,7 @@ static int held_loop_core(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, 
     a.events = d_events; a.n_events = d_events ? n_events : 0; a.radius_u_turn = radius_u_turn; a.out_final = out_final;
     a.rng_state = rng_state;
     a.pcg_state = reinterpret_cast<unsigned long long *>(pcg_state);
+    a.trace_pred = tr.pred; a.trace_ctl = tr.control; a.trace_cost = tr.cost;
     CK(launch_held_loop(h->stream, a, h->sms));
     h->stats = mpcb_stats{};
     h->stats.kernel_launches = 1;
@@ -902,8 +917,10 @@ static int held_loop_core(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, 
 int mpcb_held_closed_loop_device(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, const double *init,
                                  const double *target, const double *origin, const double *first_threshold,
                                  const int32_t *slow_steps, double *out_log, int32_t *out_ticks, int32_t *out_status) {
+    if (!h) return MPCB_ERR_INVALID;
+    const mpcb_loop_trace tr = take_trace(h);
     return held_loop_core(h, p, N, init, target, origin, first_threshold, slow_steps, nullptr, 0, 0.0, nullptr, out_log,
-                          out_ticks, out_status, nullptr);
+                          out_ticks, out_status, nullptr, nullptr, tr);
 }
 
 int mpcb_held_closed_loop_host(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, const double *init,
@@ -911,6 +928,39 @@ int mpcb_held_closed_loop_host(mpcb_handle *h, const mpcb_loop_params *p, int64_
                                const int32_t *slow_steps, double *out_log, int32_t *out_ticks, int32_t *out_status) {
     return mpcb_held_closed_loop_events_host(h, p, N, init, target, origin, first_threshold, slow_steps, nullptr, 0, 0.0,
                                              out_log, out_ticks, out_status, nullptr);
+}
+
+// the host trace tr of nrow = N * max_ticks rows in handle scratch, NaN-filled (dtr: its device twin, members null
+// where tr's are); fl_traj: also the FULL loop's last accepted trajectories [full_robots][H][3] when pred is traced
+static int stage_trace(mpcb_handle *h, const mpcb_loop_trace &tr, size_t nrow, int H, mpcb_loop_trace &dtr,
+                       int64_t full_robots = 0) {
+    dtr = mpcb_loop_trace{};
+    if (!tr.pred && !tr.control && !tr.cost) return MPCB_OK;
+    if (H < 1 || H > MPCB_MAX_H) return fail(h, MPCB_ERR_INVALID, "closed loop trace: H=%d out of range", H);
+    cudaStream_t st = h->stream;
+    auto one = [&](double *host, mpcb::DevBuf &buf, size_t n, double *&dev) -> cudaError_t {
+        if (!host) return cudaSuccess;
+        cudaError_t e = buf.ensure(sizeof(double) * n);
+        if (e == cudaSuccess) e = cudaMemsetAsync(buf.p, 0xFF, sizeof(double) * n, st);
+        dev = buf.as<double>();
+        return e;
+    };
+    CK(one(tr.pred, h->trace_pred, nrow * 3 * H, dtr.pred));
+    CK(one(tr.control, h->trace_ctl, nrow * 2, dtr.control));
+    CK(one(tr.cost, h->trace_cost, nrow, dtr.cost));
+    if (tr.pred && full_robots) CK(h->fl_traj.ensure(sizeof(double) * full_robots * 3 * H));
+    return MPCB_OK;
+}
+
+static cudaError_t copy_back_trace(mpcb_handle *h, const mpcb_loop_trace &tr, const mpcb_loop_trace &dtr, size_t nrow,
+                                   int H) {
+    cudaError_t e = cudaSuccess;
+    if (tr.pred) e = cudaMemcpyAsync(tr.pred, dtr.pred, sizeof(double) * nrow * 3 * H, cudaMemcpyDeviceToHost, h->stream);
+    if (e == cudaSuccess && tr.control)
+        e = cudaMemcpyAsync(tr.control, dtr.control, sizeof(double) * nrow * 2, cudaMemcpyDeviceToHost, h->stream);
+    if (e == cudaSuccess && tr.cost)
+        e = cudaMemcpyAsync(tr.cost, dtr.cost, sizeof(double) * nrow, cudaMemcpyDeviceToHost, h->stream);
+    return e;
 }
 
 // the PCG64 generators of held_loop_host: copied in from state_in[N][6] or seeded on the device from SeedSequence
@@ -925,12 +975,14 @@ struct PcgSource {
 
 // host pointers.  The actual run's generators are copied in from rng_in[N][625] or seeded on the device from keys
 // (key_len as for mpcb_rng_seed_device), or are PCG64 ones (pcg); with none of them, the loop is the noise-free one.
-// rng_out[N][625] (nullable) receives the MT19937 generators' states after the run.
+// rng_out[N][625] (nullable) receives the MT19937 generators' states after the run; the trace (host pointers) is staged
+// on the device, NaN-filled as the log is, and copied back.
 static int held_loop_host(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, const double *init, const double *target,
                           const double *origin, const double *first_threshold, const int32_t *slow_steps,
                           const mpcb_loop_event *events, int32_t n_events, double radius_u_turn, const uint32_t *rng_in,
                           const uint32_t *keys, int32_t key_len, uint32_t *rng_out, double *out_log, int32_t *out_ticks,
-                          int32_t *out_status, double *out_final, const PcgSource &pcg = PcgSource()) {
+                          int32_t *out_status, double *out_final, const mpcb_loop_trace &tr,
+                          const PcgSource &pcg = PcgSource()) {
     int rc = check_events(h, events, n_events);
     if (rc) return rc;
     if (N <= 0) return N == 0 ? MPCB_OK : fail(h, MPCB_ERR_INVALID, "N < 0");
@@ -991,10 +1043,15 @@ static int held_loop_host(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, 
     }
     if (out_final) CK(h->loop_final.ensure(sizeof(double) * 6 * N));
     CK(cudaMemsetAsync(h->loop_log.p, 0xFF, sizeof(double) * nlog, st));     // NaN pattern for the rows no tick wrote
+    const size_t nrow = (size_t)N * p->max_ticks;
+    mpcb_loop_trace dtr{};
+    rc = stage_trace(h, tr, nrow, p->H, dtr);
+    if (rc) return rc;
     rc = held_loop_core(h, p, N, h->in_state.as<double>(), h->in_target.as<double>(), h->in_origin.as<double>(), d_thr,
                         d_slow, events, n_events, radius_u_turn, noise ? h->loop_rng.as<uint32_t>() : nullptr,
                         h->loop_log.as<double>(), h->loop_ticks.as<int>(), h->loop_status.as<int>(),
-                        out_final ? h->loop_final.as<double>() : nullptr, pcg.any() ? h->loop_pcg.as<uint64_t>() : nullptr);
+                        out_final ? h->loop_final.as<double>() : nullptr, pcg.any() ? h->loop_pcg.as<uint64_t>() : nullptr,
+                        dtr);
     if (rc) return rc;
     if (keys || pcg.entropy) h->stats.kernel_launches += 1;     // the seeding kernel
     if (rng_out) CK(cudaMemcpyAsync(rng_out, h->loop_rng.p, sizeof(uint32_t) * nrng, cudaMemcpyDeviceToHost, st));
@@ -1004,6 +1061,7 @@ static int held_loop_host(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, 
     CK(cudaMemcpyAsync(out_log, h->loop_log.p, sizeof(double) * nlog, cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(out_ticks, h->loop_ticks.p, sizeof(int) * N, cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(out_status, h->loop_status.p, sizeof(int) * N, cudaMemcpyDeviceToHost, st));
+    CK(copy_back_trace(h, tr, dtr, nrow, p->H));
     CK(cudaStreamSynchronize(st));
     return MPCB_OK;
 }
@@ -1013,9 +1071,11 @@ int mpcb_held_closed_loop_events_host(mpcb_handle *h, const mpcb_loop_params *p,
                                       const int32_t *slow_steps, const mpcb_loop_event *events, int32_t n_events,
                                       double radius_u_turn, double *out_log, int32_t *out_ticks, int32_t *out_status,
                                       double *out_final) {
-    if (!h || !p) return MPCB_ERR_INVALID;
+    if (!h) return MPCB_ERR_INVALID;
+    const mpcb_loop_trace tr = take_trace(h);
+    if (!p) return MPCB_ERR_INVALID;
     return held_loop_host(h, p, N, init, target, origin, first_threshold, slow_steps, events, n_events, radius_u_turn,
-                          nullptr, nullptr, 0, nullptr, out_log, out_ticks, out_status, out_final);
+                          nullptr, nullptr, 0, nullptr, out_log, out_ticks, out_status, out_final, tr);
 }
 
 int mpcb_held_closed_loop_actual_host(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, const double *init,
@@ -1023,7 +1083,9 @@ int mpcb_held_closed_loop_actual_host(mpcb_handle *h, const mpcb_loop_params *p,
                                       const int32_t *slow_steps, const mpcb_loop_event *events, int32_t n_events,
                                       double radius_u_turn, uint32_t *rng_state, double *out_log, int32_t *out_ticks,
                                       int32_t *out_status, double *out_final) {
-    if (!h || !p) return MPCB_ERR_INVALID;
+    if (!h) return MPCB_ERR_INVALID;
+    const mpcb_loop_trace tr = take_trace(h);
+    if (!p) return MPCB_ERR_INVALID;
     if (!rng_state) return fail(h, MPCB_ERR_INVALID, "actual closed loop: null rng_state");
     for (int64_t n = 0; n < N; ++n) {
         const uint32_t pos = rng_state[n * mpcb::kMtWords + mpcb::kMtN];
@@ -1032,7 +1094,7 @@ int mpcb_held_closed_loop_actual_host(mpcb_handle *h, const mpcb_loop_params *p,
                         (long long)n, pos);
     }
     return held_loop_host(h, p, N, init, target, origin, first_threshold, slow_steps, events, n_events, radius_u_turn,
-                          rng_state, nullptr, 0, rng_state, out_log, out_ticks, out_status, out_final);
+                          rng_state, nullptr, 0, rng_state, out_log, out_ticks, out_status, out_final, tr);
 }
 
 int mpcb_held_closed_loop_actual_device(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, const double *init,
@@ -1040,12 +1102,14 @@ int mpcb_held_closed_loop_actual_device(mpcb_handle *h, const mpcb_loop_params *
                                         const int32_t *slow_steps, const mpcb_loop_event *events, int32_t n_events,
                                         double radius_u_turn, uint32_t *rng_state, double *out_log, int32_t *out_ticks,
                                         int32_t *out_status, double *out_final) {
-    if (!h || !p) return MPCB_ERR_INVALID;
+    if (!h) return MPCB_ERR_INVALID;
+    const mpcb_loop_trace tr = take_trace(h);
+    if (!p) return MPCB_ERR_INVALID;
     int rc = check_events(h, events, n_events);
     if (rc) return rc;
     if (!rng_state) return fail(h, MPCB_ERR_INVALID, "actual closed loop: null rng_state");
     return held_loop_core(h, p, N, init, target, origin, first_threshold, slow_steps, events, n_events, radius_u_turn,
-                          rng_state, out_log, out_ticks, out_status, out_final);
+                          rng_state, out_log, out_ticks, out_status, out_final, nullptr, tr);
 }
 
 int mpcb_held_closed_loop_seeded_host(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, const double *init,
@@ -1054,11 +1118,13 @@ int mpcb_held_closed_loop_seeded_host(mpcb_handle *h, const mpcb_loop_params *p,
                                       double radius_u_turn, const uint32_t *keys, int32_t key_len,
                                       uint32_t *rng_state_out, double *out_log, int32_t *out_ticks, int32_t *out_status,
                                       double *out_final) {
-    if (!h || !p) return MPCB_ERR_INVALID;
+    if (!h) return MPCB_ERR_INVALID;
+    const mpcb_loop_trace tr = take_trace(h);
+    if (!p) return MPCB_ERR_INVALID;
     int rc = check_seed_keys(h, N, keys, key_len);
     if (rc) return rc;
     return held_loop_host(h, p, N, init, target, origin, first_threshold, slow_steps, events, n_events, radius_u_turn,
-                          nullptr, keys, key_len, rng_state_out, out_log, out_ticks, out_status, out_final);
+                          nullptr, keys, key_len, rng_state_out, out_log, out_ticks, out_status, out_final, tr);
 }
 
 int mpcb_rng_seed_device(mpcb_handle *h, int64_t N, const uint32_t *keys, int32_t key_len, uint32_t *rng_state) {
@@ -1077,7 +1143,9 @@ int mpcb_held_closed_loop_pcg64_host(mpcb_handle *h, const mpcb_loop_params *p, 
                                      const int32_t *slow_steps, const mpcb_loop_event *events, int32_t n_events,
                                      double radius_u_turn, uint64_t *pcg_state, double *out_log, int32_t *out_ticks,
                                      int32_t *out_status, double *out_final) {
-    if (!h || !p) return MPCB_ERR_INVALID;
+    if (!h) return MPCB_ERR_INVALID;
+    const mpcb_loop_trace tr = take_trace(h);
+    if (!p) return MPCB_ERR_INVALID;
     if (!pcg_state) return fail(h, MPCB_ERR_INVALID, "PCG64 closed loop: null pcg_state");
     int rc = check_pcg64_states(h, N, pcg_state);
     if (rc) return rc;
@@ -1085,7 +1153,7 @@ int mpcb_held_closed_loop_pcg64_host(mpcb_handle *h, const mpcb_loop_params *p, 
     pcg.state_in = pcg_state;
     pcg.state_out = pcg_state;
     return held_loop_host(h, p, N, init, target, origin, first_threshold, slow_steps, events, n_events, radius_u_turn,
-                          nullptr, nullptr, 0, nullptr, out_log, out_ticks, out_status, out_final, pcg);
+                          nullptr, nullptr, 0, nullptr, out_log, out_ticks, out_status, out_final, tr, pcg);
 }
 
 int mpcb_held_closed_loop_pcg64_device(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, const double *init,
@@ -1093,12 +1161,14 @@ int mpcb_held_closed_loop_pcg64_device(mpcb_handle *h, const mpcb_loop_params *p
                                        const int32_t *slow_steps, const mpcb_loop_event *events, int32_t n_events,
                                        double radius_u_turn, uint64_t *pcg_state, double *out_log, int32_t *out_ticks,
                                        int32_t *out_status, double *out_final) {
-    if (!h || !p) return MPCB_ERR_INVALID;
+    if (!h) return MPCB_ERR_INVALID;
+    const mpcb_loop_trace tr = take_trace(h);
+    if (!p) return MPCB_ERR_INVALID;
     int rc = check_events(h, events, n_events);
     if (rc) return rc;
     if (!pcg_state) return fail(h, MPCB_ERR_INVALID, "PCG64 closed loop: null pcg_state");
     return held_loop_core(h, p, N, init, target, origin, first_threshold, slow_steps, events, n_events, radius_u_turn,
-                          nullptr, out_log, out_ticks, out_status, out_final, pcg_state);
+                          nullptr, out_log, out_ticks, out_status, out_final, pcg_state, tr);
 }
 
 int mpcb_held_closed_loop_pcg64_seeded_host(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, const double *init,
@@ -1108,7 +1178,9 @@ int mpcb_held_closed_loop_pcg64_seeded_host(mpcb_handle *h, const mpcb_loop_para
                                             int32_t entropy_stride, const uint32_t *spawn_key, int32_t spawn_len,
                                             uint64_t *pcg_state_out, double *out_log, int32_t *out_ticks,
                                             int32_t *out_status, double *out_final) {
-    if (!h || !p) return MPCB_ERR_INVALID;
+    if (!h) return MPCB_ERR_INVALID;
+    const mpcb_loop_trace tr = take_trace(h);
+    if (!p) return MPCB_ERR_INVALID;
     int rc = check_pcg64_seeds(h, N, entropy, entropy_len, entropy_stride, spawn_key, spawn_len);
     if (rc) return rc;
     PcgSource pcg;
@@ -1116,7 +1188,7 @@ int mpcb_held_closed_loop_pcg64_seeded_host(mpcb_handle *h, const mpcb_loop_para
     pcg.spawn_key = spawn_len > 0 ? spawn_key : nullptr; pcg.spawn_len = spawn_len;
     pcg.state_out = pcg_state_out;
     return held_loop_host(h, p, N, init, target, origin, first_threshold, slow_steps, events, n_events, radius_u_turn,
-                          nullptr, nullptr, 0, nullptr, out_log, out_ticks, out_status, out_final, pcg);
+                          nullptr, nullptr, 0, nullptr, out_log, out_ticks, out_status, out_final, tr, pcg);
 }
 
 int mpcb_pcg64_seed_device(mpcb_handle *h, int64_t N, const uint32_t *entropy, int32_t entropy_len,
@@ -1217,6 +1289,7 @@ int mpcb_full_closed_loop_host(mpcb_handle *h, int cost_kind, int H, int64_t N, 
                                const double *target, const double *origin, const double *first_threshold,
                                double eps, int max_ticks, double *out_log, int32_t *out_ticks, int32_t *out_status) {
     if (!h) return MPCB_ERR_INVALID;
+    const mpcb_loop_trace tr = take_trace(h);
     if (N <= 0) return N == 0 ? MPCB_OK : fail(h, MPCB_ERR_INVALID, "N < 0");
     if (!init_state || !target || !origin || !out_log || !out_ticks || !out_status || max_ticks < 1)
         return fail(h, MPCB_ERR_INVALID, "full closed loop: bad arguments");
@@ -1232,6 +1305,10 @@ int mpcb_full_closed_loop_host(mpcb_handle *h, int cost_kind, int H, int64_t N, 
     CK(h->loop_status.ensure(sizeof(int) * N)); CK(h->fl_last.ensure(sizeof(double) * 5 * N));
     CK(h->fl_k.ensure(sizeof(int) * N)); CK(h->fl_have.ensure(sizeof(int) * N));
     CK(h->fl_flags.ensure(N)); CK(h->fl_count.ensure(sizeof(int)));
+    const size_t nrow = (size_t)N * max_ticks;
+    mpcb_loop_trace dtr{};
+    int rc = stage_trace(h, tr, nrow, H, dtr, N);
+    if (rc) return rc;
     // robots that start on their target never enter the loop (while not is_on_target, math_model.py:239)
     std::vector<int> status(N, -1);
     std::vector<unsigned char> flags(N, 0);
@@ -1263,10 +1340,12 @@ int mpcb_full_closed_loop_host(mpcb_handle *h, int cost_kind, int H, int64_t N, 
     fa.kcount = h->fl_k.as<int>(); fa.have_ret = h->fl_have.as<int>(); fa.status = h->loop_status.as<int>();
     fa.ticks = h->loop_ticks.as<int>(); fa.flags = h->fl_flags.as<unsigned char>();
     fa.log = h->loop_log.as<double>(); fa.active_count = h->fl_count.as<int>();
+    fa.trace_pred = dtr.pred; fa.trace_ctl = dtr.control; fa.trace_cost = dtr.cost;
+    fa.last_traj = dtr.pred ? h->fl_traj.as<double>() : nullptr;
     int total_launches = 0;
     for (int tick = 0; tick < max_ticks && running > 0; ++tick) {
         CK(cudaMemsetAsync(h->fl_count.p, 0, sizeof(int), st));
-        int rc = mpcb_solve_batch_device(h, MPCB_MODE_FULL, cost_kind, H, N, h->in_state.as<double>(),
+        rc = mpcb_solve_batch_device(h, MPCB_MODE_FULL, cost_kind, H, N, h->in_state.as<double>(),
                                          h->in_target.as<double>(), h->in_origin.as<double>(), h->in_thr.as<double>(),
                                          h->fl_flags.as<uint8_t>(), 0, -1, h->out_cost.as<double>(),
                                          h->out_index.as<int64_t>(), h->out_traj.as<double>(), h->out_ctl.as<double>());
@@ -1280,6 +1359,7 @@ int mpcb_full_closed_loop_host(mpcb_handle *h, int cost_kind, int H, int64_t N, 
     CK(cudaMemcpyAsync(out_log, h->loop_log.p, sizeof(double) * nlog, cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(out_ticks, h->loop_ticks.p, sizeof(int) * N, cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(out_status, h->loop_status.p, sizeof(int) * N, cudaMemcpyDeviceToHost, st));
+    CK(copy_back_trace(h, tr, dtr, nrow, H));
     CK(cudaStreamSynchronize(st));
     h->stats.kernel_launches = total_launches;
     return MPCB_OK;

@@ -66,6 +66,8 @@ struct mpcb_handle_s {
     bool cand_auto = true;              // not set by the user: the prefix algorithm with a node list runs without it
     mpcb::DevBuf nccl_scratch;          // split tree: this rank's (cost, index) records + one slot per rank
     mpcb::DevBuf loop_log, loop_ticks, loop_status, loop_events, loop_final, loop_rng, loop_keys, loop_pcg, loop_pcg_spawn, small_in, small_out, fl_last, fl_k, fl_have, fl_flags, fl_count;
+    mpcb_loop_trace trace{};            // of the next closed-loop call (mpcb_set_loop_trace), consumed by it
+    mpcb::DevBuf trace_pred, trace_ctl, trace_cost, fl_traj;   // host entries: the trace staged on the device
     void *pin_in = nullptr, *pin_out = nullptr;   // pinned staging of the low-latency path
     size_t pin_in_cap = 0, pin_out_cap = 0;
     mpcb_stats stats{};

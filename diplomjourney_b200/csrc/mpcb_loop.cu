@@ -153,7 +153,9 @@ __device__ __forceinline__ void load_cost(LoopCost &cost, const double *target, 
 
 enum LoopGen { kGenNone = 0, kGenMt19937 = 1, kGenPcg64 = 2 };    // the actual run's generator kind
 
-template <int kGen>
+// kTrace: the per-tick trace is written (LoopArgs::trace_*, each still nullable).  A template parameter, so that the loop
+// without a trace is the very code it was before the trace existed (a uniform runtime test cost it 1-2 % of its time).
+template <int kGen, bool kTrace>
 __global__ void __launch_bounds__(kLoopThreads) held_loop_kernel(const LoopArgs a) {
     __shared__ double s_V[kMaxWin], s_B[kMaxWin], s_tanB[kMaxWin];
     __shared__ double s_J[kLoopThreads / 32];
@@ -218,7 +220,8 @@ __global__ void __launch_bounds__(kLoopThreads) held_loop_kernel(const LoopArgs 
 
             // ---- apply (thread 0)
             if (tid == 0) {
-                if (bj >= 0 && bJ < thr) {                  // strict '<' (math_model_tree.py:351)
+                const bool accepted = bj >= 0 && bJ < thr;  // strict '<' (math_model_tree.py:351)
+                if (accepted) {
                     const int iv = bj / nB, ib = bj - iv * nB;
                     res_v = slow ? s_vslow : s_V[iv];
                     res_beta = s_B[ib];
@@ -252,8 +255,17 @@ __global__ void __launch_bounds__(kLoopThreads) held_loop_kernel(const LoopArgs 
                         av = actual_velocity(res_v, pcg);
                         ab = actual_beta(res_beta, pcg);
                     }
-                    double *log = a.out_log + ((size_t)n * p.max_ticks + ticks) * 5;
+                    const size_t row = (size_t)n * p.max_ticks + ticks;
+                    double *log = a.out_log + row * 5;
                     log[0] = rx; log[1] = ry; log[2] = rphi; log[3] = av; log[4] = ab;
+                    // the trace: what the reference's tick logs besides the 5-list (predicted_trajectory_*, result_v /
+                    // result_beta); opt and res_* still hold the previous tick's when this one accepted no leaf
+                    if constexpr (kTrace) {
+                        if (a.trace_pred)
+                            for (int k = 0; k < 3 * p.H; ++k) a.trace_pred[row * 3 * p.H + k] = opt[k];
+                        if (a.trace_ctl) { a.trace_ctl[2 * row] = res_v; a.trace_ctl[2 * row + 1] = res_beta; }
+                        if (a.trace_cost) a.trace_cost[row] = accepted ? bJ : NAN;
+                    }
                     s_state[0] = rx; s_state[1] = ry; s_state[2] = rphi; s_state[3] = av; s_state[4] = ab;
                     ticks += 1;
                     if (recursive) { stop = 1; status = 1; }        // "Recursive error." (math_model_tree.py:559-561)
@@ -474,8 +486,8 @@ __global__ void full_apply_kernel(const FullLoopArgs a) {
     if (n >= a.N || a.status[n] >= 0) return;
     double ret[5];
     const long long idx = a.best_index[n];
+    const double *tr = a.best_traj + (size_t)n * 3 * a.H;
     if (idx >= 0) {                                        // a leaf beat the carried optimum (strict '<')
-        const double *tr = a.best_traj + (size_t)n * 3 * a.H;
         ret[0] = tr[0]; ret[1] = tr[1]; ret[2] = tr[2];
         ret[3] = a.first_control[2 * n]; ret[4] = a.first_control[2 * n + 1];
         a.threshold[n] = a.best_cost[n];
@@ -487,8 +499,18 @@ __global__ void full_apply_kernel(const FullLoopArgs a) {
     } else {                                               // stall: the previous path is returned again
         for (int k = 0; k < 5; ++k) ret[k] = a.last_ret[5 * n + k];
     }
-    double *log = a.log + ((size_t)n * a.max_ticks + a.tick) * 5;
+    const size_t row = (size_t)n * a.max_ticks + a.tick;
+    double *log = a.log + row * 5;
     for (int k = 0; k < 5; ++k) { log[k] = ret[k]; a.last_ret[5 * n + k] = ret[k]; }
+    if (a.trace_pred) {                                    // a stall repeats the last accepted trajectory
+        double *last = a.last_traj + (size_t)n * 3 * a.H;
+        for (int k = 0; k < 3 * a.H; ++k) {
+            if (idx >= 0) last[k] = tr[k];
+            a.trace_pred[row * 3 * a.H + k] = last[k];
+        }
+    }
+    if (a.trace_ctl) { a.trace_ctl[2 * row] = ret[3]; a.trace_ctl[2 * row + 1] = ret[4]; }
+    if (a.trace_cost) a.trace_cost[row] = idx >= 0 ? a.best_cost[n] : NAN;
     const double xprev = a.state[3 * n], yprev = a.state[3 * n + 1];
     a.state[3 * n] = ret[0]; a.state[3 * n + 1] = ret[1]; a.state[3 * n + 2] = ret[2];
     a.ticks[n] = a.tick + 1;
@@ -509,23 +531,29 @@ cudaError_t launch_full_apply(cudaStream_t st, const FullLoopArgs &a) {
     return cudaGetLastError();
 }
 
-template <int kGen>
+template <int kGen, bool kTrace>
 static cudaError_t launch_held_loop_t(cudaStream_t st, const LoopArgs &a, int sms) {
     const size_t smem = kGen == kGenMt19937 ? sizeof(unsigned) * kMtWords : 0;
     int per_sm = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, held_loop_kernel<kGen>, kLoopThreads, smem) != cudaSuccess ||
-        per_sm < 1)
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, held_loop_kernel<kGen, kTrace>, kLoopThreads, smem) !=
+            cudaSuccess || per_sm < 1)
         per_sm = 1;
     long long grid = (long long)sms * per_sm;
     if (grid > a.N) grid = a.N;
-    held_loop_kernel<kGen><<<(unsigned)grid, kLoopThreads, smem, st>>>(a);
+    held_loop_kernel<kGen, kTrace><<<(unsigned)grid, kLoopThreads, smem, st>>>(a);
     return cudaGetLastError();
 }
 
+template <bool kTrace>
+static cudaError_t launch_held_loop_gen(cudaStream_t st, const LoopArgs &a, int sms) {
+    if (a.rng_state) return launch_held_loop_t<kGenMt19937, kTrace>(st, a, sms);
+    if (a.pcg_state) return launch_held_loop_t<kGenPcg64, kTrace>(st, a, sms);
+    return launch_held_loop_t<kGenNone, kTrace>(st, a, sms);
+}
+
 cudaError_t launch_held_loop(cudaStream_t st, const LoopArgs &a, int sms) {
-    if (a.rng_state) return launch_held_loop_t<kGenMt19937>(st, a, sms);
-    if (a.pcg_state) return launch_held_loop_t<kGenPcg64>(st, a, sms);
-    return launch_held_loop_t<kGenNone>(st, a, sms);
+    if (a.trace_pred || a.trace_ctl || a.trace_cost) return launch_held_loop_gen<true>(st, a, sms);
+    return launch_held_loop_gen<false>(st, a, sms);
 }
 
 }  // namespace mpcb

@@ -268,6 +268,9 @@ struct LoopArgs {
     double *out_final;                                 // [N][6] x_t, y_t, x_0, y_0, steps_for_slowing, m; nullable
     unsigned *rng_state;                               // [N][625] numpy MT19937 key + pos, updated in place; null: no noise
     unsigned long long *pcg_state;                     // [N][6] numpy PCG64 records, updated in place (with rng_state null)
+    // per-tick trace, written on out_log's row (nullable): optimal_trajectory's poses [N][max_ticks][H][3], the commanded
+    // (v, beta) before actuator noise [N][max_ticks][2], the accepted leaf's cost [N][max_ticks] (NaN: none accepted)
+    double *trace_pred, *trace_ctl, *trace_cost;
 };
 
 // one online tick of a batch of robots with per-robot acceleration windows (mpcb_loop.cu); all pointers are device
@@ -292,6 +295,8 @@ struct FullLoopArgs {
     unsigned char *flags;                              // [N] MPCB_FLAG_SKIP once a robot has stopped
     double *log;                                       // [N][max_ticks][5]
     int *active_count;
+    double *trace_pred, *trace_ctl, *trace_cost;       // per-tick trace as in LoopArgs (nullable)
+    double *last_traj;                                 // [N][H][3] the last accepted trajectory (needed with trace_pred)
 };
 
 // one-launch float64 HELD solve from the raw grids (mpcb_loop.cu); all pointers are device

@@ -323,6 +323,9 @@ def add_plot_polygon(coordinates_of_vertexes):
 
 need_scatter = False
 scripted_events = True      # the demo run's operator events at ticks 1/60/90/110; set False for a plain run
+# EXTENSION: math_mpc runs the whole loop in one launch of the device-resident loop (a module switch like the two above:
+# a keyword would change math_mpc's signature, which is the reference's)
+device_loop = False
 
 
 # the programmed run's script (math_model_tree.py:564-569) in the form mpcb_held_closed_loop_events takes
@@ -347,8 +350,12 @@ def _scripted_events(tick, px, py, pphi, pv, isActual):
 
 
 def math_mpc(initial_coordinates, target_coordinates, isActual):
-    """Closed loop (math_model_tree.py:515-635): initial [x, y, phi, v, beta], target [x_t, y_t]."""
+    """Closed loop (math_model_tree.py:515-635): initial [x, y, phi, v, beta], target [x_t, y_t].
+    EXTENSION: with the module switch ``device_loop = True`` the whole loop runs as ONE launch of the device-resident
+    closed loop and leaves every module list and global as the per-tick run would (see ``_math_mpc_device``)."""
     global x, y, phi, x_t, y_t, v, beta, recursive, need_scatter, p, t
+    if device_loop:
+        return _math_mpc_device(initial_coordinates, target_coordinates, isActual)
     p, t = 1, 0
     x_t, y_t = target_coordinates[0], target_coordinates[1]
     recursive = False
@@ -385,6 +392,128 @@ def math_mpc(initial_coordinates, target_coordinates, isActual):
             result_y_velocity.append(pv * np.sin(pphi))
             result_y_acceleration.append(((pv - previous_v) / delta_t) * np.sin(pphi))
     t = 0
+
+
+# ticks math_mpc's device loop may run; the reference's loop has no bound
+DEVICE_LOOP_MAX_TICKS = 4096
+
+
+def _math_mpc_device(initial_coordinates, target_coordinates, isActual):
+    """``math_mpc`` as one ``held_closed_loop`` launch with the trace: the loop starts from the module state
+    (optimal_criterion as the first threshold, steps_for_slowing, the line x_0, y_0, the demo or actual event script
+    when ``scripted_events`` is set; the actual run draws from ``np.random``), and ``_replay_trace`` rebuilds the
+    module's lists and globals from the log and the trace."""
+    global x, y, phi, x_t, y_t, v, beta, recursive, p, t
+    from . import config as _cfg
+    ini = np.array([[float(initial_coordinates[k]) for k in range(5)]])
+    if m != 0:
+        raise ValueError(f"math_mpc with device_loop starts with the finishing heuristic's m == 0, not {m}: the device "
+                         "loop has no way to take a carried m (reset m, or set device_loop = False)")
+    carried = optimal_trajectory != [[[0]]]
+    if carried and not (vector_of_velocities(ini[0, 3]) and vector_of_beta_angles(ini[0, 4])):
+        raise ValueError("math_mpc with device_loop: the first acceleration window is empty, so the reference would hand "
+                         "back the carried optimal_trajectory, which the device loop does not hold "
+                         "(set device_loop = False)")
+    params = _native.LoopParams.from_config(_cfg, _native.COST_TREE, prediction_horizon, DEVICE_LOOP_MAX_TICKS)
+    script = (ACTUAL_EVENTS if isActual else DEMO_EVENTS) if scripted_events else None
+    kw = dict(first_threshold=[float(optimal_criterion)], slow_steps=[int(steps_for_slowing)], events=script,
+              radius_u_turn=radius_u_turn, trace=True)
+    tgt = [[float(target_coordinates[0]), float(target_coordinates[1])]]
+    org = [[float(x_0), float(y_0)]]
+    if isActual:
+        r = _solver().held_closed_loop(params, ini, tgt, org, rng_state=_pack_generators([random]), **kw)
+    else:
+        r = _solver().held_closed_loop(params, ini, tgt, org, **kw)
+    status = int(r["status"][0])
+    if status == _native.LOOP_MAX_TICKS:
+        raise RuntimeError(f"math_mpc with device_loop: no stop within {DEVICE_LOOP_MAX_TICKS} ticks")
+    p, t = 1, 0
+    x_t, y_t = target_coordinates[0], target_coordinates[1]
+    recursive = False
+    if not isActual:
+        x, y, phi, v, beta = (initial_coordinates[k] for k in range(5))
+    if status == _native.LOOP_NO_LEAF:
+        if carried:
+            raise ValueError("math_mpc with device_loop: no leaf beat optimal_criterion on the first tick, so the "
+                             "reference would hand back the carried optimal_trajectory (set device_loop = False)")
+        raise IndexError("no leaf beat optimal_criterion on the first tick: optimal_trajectory is still the placeholder")
+    if isActual:                            # the draws the robot made on the device
+        old = random.get_state()
+        st = r["rng_state"][0]
+        random.set_state((old[0], st[:624].copy(), int(st[624]), old[3], old[4]))
+    k = int(r["ticks"][0])
+    _replay_trace(globals(), ini[0], r["log"][0], r["pred"][0], r["control"][0], k, status, r["final"][0], script,
+                  isActual)
+    if not isActual and k:
+        x, y, phi, v, beta = r["log"][0, k - 1]
+
+
+def _replay_trace(g, init, log, pred, control, ticks, status, final, script, isActual):
+    """The state ``math_mpc`` leaves in ``g`` (the module globals, or one robot's dict from ``reset_state``) when it runs
+    one robot alone, rebuilt from that robot's device loop: init[5], log[ticks][5], the trace pred[ticks][H][3] and
+    control[ticks][2], status, final[6] = x_t, y_t, x_0, y_0, steps_for_slowing, m, and the event script it ran with.
+    Appends to g's log lists as the per-tick run appends to them (math_model_tree.py:542-635, _finish_tick)."""
+    pre = "actual_" if isActual else ""
+    names = _log_names(isActual)
+    tt = 0
+    xprev, yprev, pv_prev = init[0], init[1], init[3]
+    rec, pp = False, 1
+    for k in range(ticks):
+        tt += delta_t
+        g[pre + "time_arr_for_plotting"].append(tt)
+        for c in range(3):
+            for j, name in enumerate(names[c]):
+                g[name].append(pred[k][j][c])
+        px, py, pphi, pv, pbeta = log[k]
+        cv, cb = control[k]
+        g[pre + "result_trajectory_x"].append(px)
+        g[pre + "result_trajectory_y"].append(py)
+        g[pre + "result_trajectory_phi"].append(pphi)
+        if isActual:                         # the applied (noisy) values, logged by math_mpc after the tick
+            g["actual_result_trajectory_v"].append(pv)
+            g["actual_result_trajectory_beta"].append(pbeta)
+            g["actual_result_trajectory_angle_speed"].append((pv / L) * np.tan(pbeta))
+        else:
+            g["result_trajectory_v"].append(cv)
+            g["result_trajectory_beta"].append(cb)
+            g["result_trajectory_angle_speed"].append((cv / L) * np.tan(cb))
+        if rec:                              # the "Recursive error." tick
+            break
+        if px == xprev and py == yprev:
+            rec = True
+        xprev, yprev = px, py
+        pp += 1
+        if not isActual:
+            g["result_x_velocity"].append(pv * np.cos(pphi))
+            g["result_x_acceleration"].append(((pv - pv_prev) / delta_t) * np.cos(pphi))
+            g["result_y_velocity"].append(pv * np.sin(pphi))
+            g["result_y_acceleration"].append(((pv - pv_prev) / delta_t) * np.sin(pphi))
+        pv_prev = pv
+    # every event goes through new_target, which restarts the line at the robot's pose of that tick
+    fired = [e[0] for e in (script or ()) if e[0] < ticks or (e[0] == ticks and status != _native.LOOP_STALLED)]
+    if fired:
+        g["phi_0"] = log[max(fired) - 1][2]
+    g.update(x_t=final[0], y_t=final[1], x_0=final[2], y_0=final[3], steps_for_slowing=int(final[4]), m=int(final[5]),
+             p=pp, recursive=rec, t=0)
+    if ticks:
+        cv, cb = control[ticks - 1]
+        g["optimal_trajectory"] = [[[q[0], q[1], q[2], cv, cb] for q in pred[ticks - 1]]]
+        g["result_v"], g["result_beta"] = cv, cb
+        g["optimal_criterion"] = sys.maxsize
+
+
+def _replayed_robots(r, ini, first, script, isActual):
+    """``robots`` of a device-loop result with the trace: per robot the state ``math_mpc`` leaves when it runs that robot
+    alone (``_replay_trace`` on a fresh ``reset_state`` dict)."""
+    robots = []
+    for i in range(ini.shape[0]):
+        ctx = {}
+        reset_state(ctx)
+        ctx.update(phi_0=phi_0, optimal_criterion=first[i])
+        _replay_trace(ctx, ini[i], r["log"][i], r["pred"][i], r["control"][i], int(r["ticks"][i]), int(r["status"][i]),
+                      r["final"][i], script, isActual)
+        robots.append(ctx)
+    return robots
 
 
 _EVENT_KEYS = ("x_t", "y_t", "x_0", "y_0", "phi_0", "steps_for_slowing")
@@ -503,36 +632,39 @@ def _generator_kind(rngs):
     return kinds.pop() if kinds else "mt19937"
 
 
-def _math_mpc_batch_device_noise(params, ini, tgt, org, first, rngs, events, seeds=None, kind="mt19937"):
+def _math_mpc_batch_device_noise(params, ini, tgt, org, first, rngs, events, seeds=None, kind="mt19937", logs=False):
     """The actual run on the device (mpcb_held_closed_loop_actual): each robot draws from its own generator, whose state
     goes to the device as get_state() and comes back through set_state (has_gauss / cached_gaussian kept).  With
     ``seeds`` (already checked by ``_native.seed_keys``) the generators are seeded on the device and stay there.
     ``kind="pcg64"``: numpy Generator(PCG64) streams (mpcb_held_closed_loop_pcg64): the bit generators' state, inc,
-    has_uint32 and uinteger go to the device and come back; ``seeds`` then is a SeedSequence or integer seeds."""
+    has_uint32 and uinteger go to the device and come back; ``seeds`` then is a SeedSequence or integer seeds.
+    ``logs=True``: the loop also writes its trace, and the result carries ``robots`` (``_replayed_robots``)."""
     script = ACTUAL_EVENTS if events is True else list(events or ())
-    kw = dict(first_threshold=first, events=script or None, radius_u_turn=radius_u_turn)
+    kw = dict(first_threshold=first, events=script or None, radius_u_turn=radius_u_turn, trace=logs)
     if kind == "pcg64":
         if seeds is not None:
-            return _solver().held_closed_loop(params, ini, tgt, org, pcg_seeds=seeds, return_rng_state=False, **kw)
-        r = _solver().held_closed_loop(params, ini, tgt, org,
-                                       pcg_state=np.stack([_native.pcg64_record(g.bit_generator) for g in rngs]), **kw)
-        for g, st in zip(rngs, r.pop("pcg_state")):
-            g.bit_generator.state = _native.pcg64_state(st)
-        return r
-    if seeds is not None:
-        return _solver().held_closed_loop(params, ini, tgt, org, seeds=seeds, return_rng_state=False, **kw)
-    gens = [random] if rngs is None else rngs
-    r = _solver().held_closed_loop(params, ini, tgt, org, first_threshold=first, events=script or None,
-                                   radius_u_turn=radius_u_turn, rng_state=_pack_generators(gens))
-    for g, st in zip(gens, r.pop("rng_state")):
-        old = g.get_state()
-        g.set_state((old[0], st[:624].copy(), int(st[624]), old[3], old[4]))
+            r = _solver().held_closed_loop(params, ini, tgt, org, pcg_seeds=seeds, return_rng_state=False, **kw)
+        else:
+            r = _solver().held_closed_loop(params, ini, tgt, org,
+                                           pcg_state=np.stack([_native.pcg64_record(g.bit_generator) for g in rngs]), **kw)
+            for g, st in zip(rngs, r.pop("pcg_state")):
+                g.bit_generator.state = _native.pcg64_state(st)
+    elif seeds is not None:
+        r = _solver().held_closed_loop(params, ini, tgt, org, seeds=seeds, return_rng_state=False, **kw)
+    else:
+        gens = [random] if rngs is None else rngs
+        r = _solver().held_closed_loop(params, ini, tgt, org, rng_state=_pack_generators(gens), **kw)
+        for g, st in zip(gens, r.pop("rng_state")):
+            old = g.get_state()
+            g.set_state((old[0], st[:624].copy(), int(st[624]), old[3], old[4]))
+    if logs:
+        r["robots"] = _replayed_robots(r, ini, first, script, True)
     return r
 
 
 def math_mpc_batch(initial_coordinates, target_coordinates, max_ticks=512, origin=None, cost_kind=None,
                    isActual=False, rngs=None, events=False, host_loop=False, device_noise=False, seeds=None,
-                   generator=None):
+                   generator=None, logs=False):
     """EXTENSION (not in the reference): the closed loop of ``math_mpc`` for a whole batch of robots.
     ``initial_coordinates`` [N][5] = x, y, phi, v, beta; ``target_coordinates`` [N][2].  The tracked line starts at
     the module's x_0, y_0 unless ``origin`` [N][2] is given.
@@ -554,7 +686,7 @@ def math_mpc_batch(initial_coordinates, target_coordinates, max_ticks=512, origi
       module generator ``np.random``, for N == 1 only: one generator shared by several robots interleaves their draws,
       which one CTA per robot cannot reproduce.  ``events=True`` is the actual run's script (new_target(2, 3) after tick
       1, then the demo script), or any ``[(tick, kind, a, b), ...]``.  Returns log, ticks, status and final as the
-      noise-free device loop does (no ``robots``).
+      noise-free device loop does (``robots`` with ``logs=True``).
     * ``isActual=True, device_noise=True, seeds=...`` in place of ``rngs``: robot i draws the stream of
       ``np.random.RandomState(seeds[i])``, seeded on the device from ``seeds`` [N] (integer seeds) or [N][K] (keys; a
       row is a key even when K == 1, see ``_native.seed_keys``).  No generator object is built and ``np.random`` is
@@ -566,6 +698,13 @@ def math_mpc_batch(initial_coordinates, target_coordinates, max_ticks=512, origi
       gives robot i the stream of ``default_rng(seeds.spawn(N)[i])`` and advances ``seeds`` as ``spawn(N)`` does;
       integer ``seeds`` with ``generator="pcg64"`` give robot i ``default_rng(seeds[i])`` (without the selector
       integer seeds keep their RandomState meaning).
+    * ``logs=True`` on the device paths (``isActual=False``, or ``device_noise=True``): the loop also writes what every
+      tick logs besides the 5-list, and the dict carries ``pred[N][max_ticks][H][3]`` (optimal_trajectory's poses),
+      ``control[N][max_ticks][2]`` (the commanded v, beta, before actuator noise), ``cost[N][max_ticks]`` and ``robots``:
+      per robot the module state ``math_mpc`` leaves when it runs that robot alone -- every log list of
+      ``reset_state``, p, m, recursive, steps_for_slowing, x_t, y_t, x_0, y_0, phi_0, t, optimal_trajectory, result_v,
+      result_beta.  (Unlike the per-tick path's ``robots``, result_{x,y}_{velocity,acceleration} are filled, as
+      ``math_mpc`` fills them.)
 
     Returns dict(log[N][max_ticks][5], ticks[N], status[N])."""
     from . import config as _cfg
@@ -619,15 +758,18 @@ def math_mpc_batch(initial_coordinates, target_coordinates, max_ticks=512, origi
     params = _native.LoopParams.from_config(_cfg, _native.COST_TREE if cost_kind is None else cost_kind,
                                             prediction_horizon, max_ticks)
     if device_noise:
-        return _math_mpc_batch_device_noise(params, ini, tgt, org, first, rngs, events, seeds, kind)
+        return _math_mpc_batch_device_noise(params, ini, tgt, org, first, rngs, events, seeds, kind, logs)
     if isActual or host_loop:
         if not isinstance(events, bool) and events is not None:
             raise ValueError("a custom event script runs on the device loop only (isActual=False, host_loop=False); "
                              "the per-tick path applies the demo script (events=True) with the module's own functions")
         return _math_mpc_batch_ticks(ini, tgt, org, first, max_ticks, cost_kind, isActual, rngs, bool(events))
     script = DEMO_EVENTS if events is True else list(events or ())
-    return _solver().held_closed_loop(params, ini, tgt, org, first_threshold=first, events=script or None,
-                                      radius_u_turn=radius_u_turn)
+    r = _solver().held_closed_loop(params, ini, tgt, org, first_threshold=first, events=script or None,
+                                   radius_u_turn=radius_u_turn, trace=logs)
+    if logs:
+        r["robots"] = _replayed_robots(r, ini, first, script, False)
+    return r
 
 
 def reset_state(g=None):

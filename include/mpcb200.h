@@ -349,6 +349,25 @@ MPCB_API int mpcb_held_closed_loop_pcg64_seeded_host(mpcb_handle *h, const mpcb_
                                             double *out_log, int32_t *out_ticks, int32_t *out_status,
                                             double *out_final);
 
+/* What the reference's tick logs besides the 5-list, per robot and tick, on the same row as out_log (rows after a
+ * robot's last tick: the host entries fill them with NaN, the device entries leave them alone):
+ *   pred[N][max_ticks][H][3]  the poses of optimal_trajectory as the tick logs them (predicted_trajectory_*_anim*): the
+ *                             trajectory accepted on that tick, or the previous one when the tick accepted none
+ *   control[N][max_ticks][2]  the commanded (v, beta) of that trajectory (result_v after the slow-down override,
+ *                             result_beta), before actuator noise; in the noise-free and FULL loops out_log's columns 3-4
+ *   cost[N][max_ticks]        float64 cost of the leaf accepted on that tick, NaN when none was accepted
+ * Memory: N * max_ticks * (3H + 3) * 8 bytes (0.8 GB for 16,384 robots, 512 ticks, H = 3). */
+typedef struct {
+    double *pred;      /* [N][max_ticks][H][3] */
+    double *control;   /* [N][max_ticks][2]    */
+    double *cost;      /* [N][max_ticks]       */
+} mpcb_loop_trace;
+/* Trace of the NEXT closed-loop call on this handle (any mpcb_held_closed_loop_* entry or mpcb_full_closed_loop_host).
+ * Pointers are of the kind that entry takes: host for _host, device for _device.  Each member is nullable.  The call
+ * consumes the trace whether it succeeds or fails (a trace left attached would later write into buffers the caller has
+ * freed); NULL clears it.  Without a trace every output is what it is without this call. */
+MPCB_API int mpcb_set_loop_trace(mpcb_handle *h, const mpcb_loop_trace *trace);
+
 /* ONE online tick for a batch of robots that each have their OWN acceleration window (SURVEY 8f row f2).  The
  * reference rebuilds the control window per robot and per tick around the robot's current (v, beta)
  * (vector_of_velocities / vector_of_beta_angles, math_model_tree.py:239-256, called at :543-545 and -- with the noisy
