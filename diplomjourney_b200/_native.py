@@ -123,6 +123,7 @@ def load():
     lib.mpcb_solve_held_windows_host.argtypes = win
     lib.mpcb_solve_held_windows_device.argtypes = win
     lib.mpcb_full_closed_loop_host.argtypes = [vp, C.c_int, C.c_int, C.c_int64, vp, vp, vp, vp, C.c_double, C.c_int, vp, vp, vp]
+    lib.mpcb_full_closed_loop_device.argtypes = lib.mpcb_full_closed_loop_host.argtypes
     lib.mpcb_set_loop_trace.argtypes = [vp, C.POINTER(LoopTrace)]
     split = [vp, vp, C.c_int, C.c_int, C.c_int64, vp, vp, vp, vp, vp, vp, vp, vp]
     lib.mpcb_solve_tree_split_host.argtypes = split
@@ -610,6 +611,21 @@ class Solver:
         self._ck(self.lib.mpcb_full_closed_loop_host(self.h, cost, H, N, _ptr(ini), _ptr(tg), _ptr(og), _ptr(thr),
                                                      float(eps), int(max_ticks), _ptr(log), _ptr(ticks), _ptr(status)))
         return dict(log=log, ticks=ticks, status=status, **tr)
+
+    def full_closed_loop_device(self, cost, H, N, init_state, target, origin, first_threshold, eps, max_ticks, out_log,
+                                out_ticks, out_status, trace=None):
+        """mpcb_full_closed_loop_device: ``full_closed_loop`` on raw device addresses (e.g. torch.Tensor.data_ptr()):
+        init_state [N][3], target / origin [N][2], first_threshold [N] float64 or 0 (= +inf), out_log
+        [N][max_ticks][5] float64, out_ticks / out_status [N] int32.  The inputs are only read.  Rows of out_log after
+        a robot's last tick are not written: fill it (with NaN, as the host entry does) beforehand.  ``trace``:
+        (pred, control, cost) device addresses as for ``set_loop_trace`` (0 = not wanted), rows after a robot's last
+        tick not written either.  The whole run is one graph launch on self.stream; does not synchronise."""
+        vp = lambda x: C.c_void_p(int(x)) if x else None
+        if trace is not None:
+            self.set_loop_trace(*trace)
+        self._ck(self.lib.mpcb_full_closed_loop_device(self.h, int(cost), int(H), int(N), vp(init_state), vp(target),
+                                                       vp(origin), vp(first_threshold), float(eps), int(max_ticks),
+                                                       vp(out_log), vp(out_ticks), vp(out_status)))
 
     def dump_leaves(self, mode, cost, H, state, target, origin, flags=0, algo=ALGO_LEAFWALK, leaf_begin=0, count=None):
         st = _arr(state, np.float64).ravel()[:3].copy()

@@ -42,6 +42,8 @@ cudaError_t launch_pcg64_seed(cudaStream_t, long long N, const unsigned *entropy
                               const unsigned *spawn, int spawn_len, unsigned long long *pcg_state);
 cudaError_t launch_held_small(cudaStream_t, const SmallArgs &);
 cudaError_t launch_full_apply(cudaStream_t, const FullLoopArgs &);
+cudaError_t launch_full_loop_init(cudaStream_t, const FullLoopArgs &, const double *init, const double *first_threshold);
+cudaError_t launch_full_loop_gate(cudaStream_t, cudaGraphConditionalHandle, int *ctl, int max_ticks, int advance);
 cudaError_t launch_held_windows(cudaStream_t, const WindowArgs &, int sms);
 cudaError_t launch_split_ub_min(cudaStream_t, const LaunchArgs &, const unsigned long long *all, int nranks);
 cudaError_t launch_split_pack(cudaStream_t, const LaunchArgs &, SplitRec *mine);
@@ -259,6 +261,8 @@ static int ensure_tables(mpcb_handle *h) {
 
 extern "C" {
 
+static void retire_loop_graphs(mpcb_handle *h, bool all);
+
 int mpcb_version(void) { return 100; }
 
 int mpcb_device_count(void) {
@@ -294,8 +298,10 @@ int mpcb_destroy(mpcb_handle *h) {
                       &h->lock, &h->ub, &h->tile_list, &h->reduce_scratch, &h->in_state, &h->in_target, &h->in_origin, &h->in_thr, &h->in_flags, &h->out_cost,
                       &h->out_index, &h->out_traj, &h->out_ctl, &h->dump_rec, &h->dump_j, &h->loop_log, &h->loop_ticks,
                       &h->loop_status, &h->loop_events, &h->loop_final, &h->loop_rng, &h->loop_keys, &h->small_in, &h->small_out, &h->fl_last, &h->fl_k, &h->fl_have, &h->fl_flags,
-                      &h->fl_count, &h->trace_pred, &h->trace_ctl, &h->trace_cost, &h->fl_traj, &h->nccl_scratch, &h->cand, &h->cand_J, &h->cand_sel, &h->node_list})
+                      &h->fl_count, &h->fl_state, &h->fl_thr, &h->trace_pred, &h->trace_ctl, &h->trace_cost, &h->fl_traj, &h->nccl_scratch, &h->cand, &h->cand_J, &h->cand_sel, &h->node_list})
         b->release();
+    retire_loop_graphs(h, true);
+    if (h->fl_exec) cudaGraphExecDestroy(h->fl_exec);
     if (h->pin_in) cudaFreeHost(h->pin_in);
     if (h->pin_out) cudaFreeHost(h->pin_out);
     cudaStreamDestroy(h->stream);
@@ -315,6 +321,7 @@ int mpcb_sync(mpcb_handle *h) {
 
 int mpcb_set_option(mpcb_handle *h, const char *name, double value) {
     if (!h || !name) return MPCB_ERR_INVALID;
+    ++h->epoch;
     if (!strcmp(name, "tol_scale")) h->tol_scale = value;
     else if (!strcmp(name, "algo")) h->algo = (int)value;
     else if (!strcmp(name, "refine")) h->refine = value != 0.0;
@@ -368,6 +375,7 @@ int mpcb_set_grid(mpcb_handle *h, const double *v, int nv, const double *beta, i
     h->g.S = nv * nb; h->g.nb = nb; h->g.dt = delta_t;
     h->have_grid = true;
     h->tables_ready = false;
+    ++h->epoch;
     return MPCB_OK;
 }
 
@@ -931,9 +939,8 @@ int mpcb_held_closed_loop_host(mpcb_handle *h, const mpcb_loop_params *p, int64_
 }
 
 // the host trace tr of nrow = N * max_ticks rows in handle scratch, NaN-filled (dtr: its device twin, members null
-// where tr's are); fl_traj: also the FULL loop's last accepted trajectories [full_robots][H][3] when pred is traced
-static int stage_trace(mpcb_handle *h, const mpcb_loop_trace &tr, size_t nrow, int H, mpcb_loop_trace &dtr,
-                       int64_t full_robots = 0) {
+// where tr's are)
+static int stage_trace(mpcb_handle *h, const mpcb_loop_trace &tr, size_t nrow, int H, mpcb_loop_trace &dtr) {
     dtr = mpcb_loop_trace{};
     if (!tr.pred && !tr.control && !tr.cost) return MPCB_OK;
     if (H < 1 || H > MPCB_MAX_H) return fail(h, MPCB_ERR_INVALID, "closed loop trace: H=%d out of range", H);
@@ -948,7 +955,6 @@ static int stage_trace(mpcb_handle *h, const mpcb_loop_trace &tr, size_t nrow, i
     CK(one(tr.pred, h->trace_pred, nrow * 3 * H, dtr.pred));
     CK(one(tr.control, h->trace_ctl, nrow * 2, dtr.control));
     CK(one(tr.cost, h->trace_cost, nrow, dtr.cost));
-    if (tr.pred && full_robots) CK(h->fl_traj.ensure(sizeof(double) * full_robots * 3 * H));
     return MPCB_OK;
 }
 
@@ -1285,6 +1291,174 @@ int mpcb_solve_held_windows_host(mpcb_handle *h, const mpcb_loop_params *p, int6
     return MPCB_OK;
 }
 
+// Destroys the replaced FULL loop graphs, when the handle's stream is idle (all: the caller has just synchronised it).
+// cudaGraphExecDestroy waits for the work in flight, which the device entry must not.
+static void retire_loop_graphs(mpcb_handle *h, bool all) {
+    if (h->fl_graphs.empty()) return;
+    if (!all) {
+        const cudaError_t q = cudaStreamQuery(h->stream);
+        if (q == cudaErrorNotReady && cudaPeekAtLastError() == cudaErrorNotReady)
+            (void)cudaGetLastError();            // the query's own "not ready", not an error of a launch
+        if (q != cudaSuccess) return;
+    }
+    for (cudaGraphExec_t x : h->fl_graphs) cudaGraphExecDestroy(x);
+    h->fl_graphs.clear();
+}
+
+// Launches the handle's FULL loop graph, after destroying replaced ones while the stream is still idle.
+static int launch_loop_graph(mpcb_handle *h) {
+    retire_loop_graphs(h, false);
+    const cudaError_t e = cudaGraphLaunch(h->fl_exec, h->stream);
+    if (e != cudaSuccess) return fail(h, MPCB_ERR_CUDA, "full closed loop: graph launch failed: %s", cudaGetErrorString(e));
+    return MPCB_OK;
+}
+
+// Capture of the FULL loop into g (empty on entry):
+//   [running = tick = 0] -> [init] -> [gate] -> WHILE (running > 0 && tick < max_ticks) {
+//       solve_core (as it is, every launch and memset of one batched solve) -> [apply] -> [gate] }
+// (the gate zeroes the running count after reading it)
+// Every capture begun here is ended here, also on failure.  *per_tick: the kernels one tick launches.
+static int capture_full_loop(mpcb_handle *h, cudaGraph_t g, const FullLoopArgs &fa, int cost_kind, const double *init,
+                             const double *origin, const double *first_threshold, int *per_tick) {
+    cudaStream_t st = h->stream;
+    int *ctl = fa.active_count;          // [0] running robots, [1] tick
+    cudaGraphConditionalHandle cond;
+    CK(cudaGraphConditionalHandleCreate(&cond, g, 0, 0));
+    CK(cudaStreamBeginCaptureToGraph(st, g, nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed));
+    cudaError_t e = cudaMemsetAsync(ctl, 0, 2 * sizeof(int), st);
+    if (e == cudaSuccess) e = launch_full_loop_init(st, fa, init, first_threshold);
+    if (e == cudaSuccess) e = launch_full_loop_gate(st, cond, ctl, fa.max_ticks, 0);
+    cudaGraph_t body = nullptr;
+    if (e == cudaSuccess) {              // the WHILE node after the gate
+        cudaStreamCaptureStatus cs;
+        const cudaGraphNode_t *deps = nullptr;
+        size_t ndeps = 0;
+        e = cudaStreamGetCaptureInfo(st, &cs, nullptr, nullptr, &deps, &ndeps);
+        cudaGraphNodeParams cp = {};
+        cp.type = cudaGraphNodeTypeConditional;
+        cp.conditional.handle = cond;
+        cp.conditional.type = cudaGraphCondTypeWhile;
+        cp.conditional.size = 1;
+        cudaGraphNode_t node;
+        if (e == cudaSuccess) e = cudaGraphAddNode(&node, g, deps, ndeps, &cp);
+        if (e == cudaSuccess) e = cudaStreamUpdateCaptureDependencies(st, &node, 1, cudaStreamSetCaptureDependencies);
+        if (e == cudaSuccess) body = cp.conditional.phGraph_out[0];
+    }
+    cudaGraph_t captured = nullptr;
+    const cudaError_t e_end = cudaStreamEndCapture(st, &captured);
+    if (e != cudaSuccess || e_end != cudaSuccess)
+        return fail(h, MPCB_ERR_CUDA, "full closed loop: building the loop graph failed: %s",
+                    cudaGetErrorString(e != cudaSuccess ? e : e_end));
+
+    CK(cudaStreamBeginCaptureToGraph(st, body, nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed));
+    int rc = solve_core(h, MPCB_MODE_FULL, cost_kind, fa.H, fa.N, fa.state, fa.target, origin, fa.threshold, fa.flags, 0,
+                        -1, h->out_cost.as<double>(), h->out_index.as<int64_t>(), h->out_traj.as<double>(),
+                        h->out_ctl.as<double>(), nullptr);
+    if (e == cudaSuccess && rc == MPCB_OK) {
+        *per_tick = h->stats.kernel_launches + 1;
+        e = launch_full_apply(st, fa);
+    }
+    if (e == cudaSuccess && rc == MPCB_OK) e = launch_full_loop_gate(st, cond, ctl, fa.max_ticks, 1);
+    const cudaError_t e_body = cudaStreamEndCapture(st, &captured);
+    if (rc) return rc;
+    if (e != cudaSuccess || e_body != cudaSuccess)
+        return fail(h, MPCB_ERR_CUDA, "full closed loop: capturing the tick failed: %s",
+                    cudaGetErrorString(e != cudaSuccess ? e : e_body));
+    return MPCB_OK;
+}
+
+// The FULL closed loop as ONE graph launch on the handle's stream; device pointers throughout, nothing synchronised.
+// N >= 1 and the pointers are checked by the caller; first_threshold and the trace's members are nullable.  The
+// executable graph is kept in the handle and launched again while nothing it froze at capture has changed (the key:
+// grid and options through the handle's epoch, the handle's buffers through the allocation count, the arguments);
+// otherwise the loop is captured and instantiated anew and the old graph destroyed once its last run has ended.
+// *per_tick: the kernels one tick launches (the solve's and the apply kernel).
+static int full_loop_enqueue(mpcb_handle *h, int cost_kind, int H, int64_t N, const double *init, const double *target,
+                             const double *origin, const double *first_threshold, double eps, int max_ticks,
+                             double *out_log, int32_t *out_ticks, int32_t *out_status, const mpcb_loop_trace &tr,
+                             int *per_tick) {
+    if (H < 1 || H > MPCB_MAX_H) return fail(h, MPCB_ERR_INVALID, "H=%d out of range [1,%d]", H, MPCB_MAX_H);
+    if (cost_kind != MPCB_COST_MM && cost_kind != MPCB_COST_TREE) return fail(h, MPCB_ERR_INVALID, "bad mode/cost");
+    CK(cudaSetDevice(h->device));
+    int rc = ensure_tables(h);           // not inside a capture: it uploads from host vectors that die on return
+    if (rc) return rc;
+    CK(h->fl_state.ensure(sizeof(double) * 3 * N)); CK(h->fl_thr.ensure(sizeof(double) * N));
+    CK(h->out_cost.ensure(sizeof(double) * N)); CK(h->out_index.ensure(sizeof(int64_t) * N));
+    CK(h->out_traj.ensure(sizeof(double) * 3 * H * N)); CK(h->out_ctl.ensure(sizeof(double) * 2 * N));
+    CK(h->fl_last.ensure(sizeof(double) * 5 * N));
+    CK(h->fl_k.ensure(sizeof(int) * N)); CK(h->fl_have.ensure(sizeof(int) * N));
+    CK(h->fl_flags.ensure(N)); CK(h->fl_count.ensure(2 * sizeof(int)));
+    if (tr.pred) CK(h->fl_traj.ensure(sizeof(double) * N * 3 * H));
+    FullLoopArgs fa{};
+    fa.N = N; fa.H = H; fa.max_ticks = max_ticks; fa.eps = eps;
+    fa.active_count = h->fl_count.as<int>(); fa.tick = fa.active_count + 1;
+    fa.target = target;
+    fa.best_cost = h->out_cost.as<double>(); fa.best_index = h->out_index.as<long long>();
+    fa.best_traj = h->out_traj.as<double>(); fa.first_control = h->out_ctl.as<double>();
+    fa.state = h->fl_state.as<double>(); fa.threshold = h->fl_thr.as<double>(); fa.last_ret = h->fl_last.as<double>();
+    fa.kcount = h->fl_k.as<int>(); fa.have_ret = h->fl_have.as<int>(); fa.status = out_status;
+    fa.ticks = out_ticks; fa.flags = h->fl_flags.as<unsigned char>();
+    fa.log = out_log;
+    fa.trace_pred = tr.pred; fa.trace_ctl = tr.control; fa.trace_cost = tr.cost;
+    fa.last_traj = tr.pred ? h->fl_traj.as<double>() : nullptr;
+    LoopGraphKey key;
+    memset(&key, 0, sizeof key);
+    key.epoch = h->epoch; key.N = N; key.cost_kind = cost_kind; key.H = H; key.max_ticks = max_ticks; key.eps = eps;
+    const void *io[10] = {init, target, origin, first_threshold, out_log, out_ticks, out_status, tr.pred, tr.control, tr.cost};
+    memcpy(key.io, io, sizeof io);
+    key.allocs = g_allocs.load();
+    if (h->fl_exec && !memcmp(&key, &h->fl_key, sizeof key)) {
+        h->stats = h->fl_stats;
+        *per_tick = h->fl_per_tick;
+        return launch_loop_graph(h);
+    }
+    // solve_core's scratch grows outside the capture: a capture that needed a bigger buffer is dropped, the buffer
+    // grown and the loop captured again (each round grows one more buffer; the sizes do not change between rounds)
+    for (;;) {
+        cudaGraph_t g = nullptr;
+        CK(cudaGraphCreate(&g, 0));
+        g_growth = DeferredGrowth{true, {}};
+        rc = capture_full_loop(h, g, fa, cost_kind, init, origin, first_threshold, per_tick);
+        g_growth.defer = false;
+        const std::vector<std::pair<DevBuf *, size_t>> wanted = std::move(g_growth.wanted);
+        g_growth.wanted.clear();
+        if (rc == MPCB_OK) {
+            cudaGraphExec_t exec = nullptr;
+            const cudaError_t e = cudaGraphInstantiate(&exec, g, 0);
+            cudaGraphDestroy(g);
+            if (e != cudaSuccess)
+                return fail(h, MPCB_ERR_CUDA, "full closed loop: graph instantiation failed: %s", cudaGetErrorString(e));
+            if (h->fl_exec) h->fl_graphs.push_back(h->fl_exec);   // destroyed once the stream is idle
+            key.allocs = g_allocs.load();      // the buffers grown for this capture are the ones it holds
+            h->fl_key = key; h->fl_exec = exec;
+            h->fl_stats = h->stats; h->fl_per_tick = *per_tick;
+            return launch_loop_graph(h);
+        }
+        cudaGraphDestroy(g);
+        if (wanted.empty()) return rc;
+        for (const auto &w : wanted) CK(w.first->ensure(w.second));
+    }
+}
+
+int mpcb_full_closed_loop_device(mpcb_handle *h, int cost_kind, int H, int64_t N, const double *init_state,
+                                 const double *target, const double *origin, const double *first_threshold,
+                                 double eps, int max_ticks, double *out_log, int32_t *out_ticks, int32_t *out_status) {
+    if (!h) return MPCB_ERR_INVALID;
+    const mpcb_loop_trace tr = take_trace(h);
+    if (N < 0 || N >= (1LL << 31)) return fail(h, MPCB_ERR_INVALID, "N out of range");
+    if (N == 0) return MPCB_OK;
+    if (!init_state || !target || !origin || !out_log || !out_ticks || !out_status || max_ticks < 1)
+        return fail(h, MPCB_ERR_INVALID, "full closed loop: bad arguments");
+    if (!h->have_grid) return fail(h, MPCB_ERR_NO_GRID, "mpcb_set_grid has not been called");
+    int per_tick = 0;
+    int rc = full_loop_enqueue(h, cost_kind, H, N, init_state, target, origin, first_threshold, eps, max_ticks, out_log,
+                               out_ticks, out_status, tr, &per_tick);
+    if (rc) return rc;
+    h->stats.kernel_launches = per_tick;     // the tick count is known on the device only
+    return MPCB_OK;
+}
+
+// host buffers -> device staging -> the loop graph -> host buffers, one synchronisation
 int mpcb_full_closed_loop_host(mpcb_handle *h, int cost_kind, int H, int64_t N, const double *init_state,
                                const double *target, const double *origin, const double *first_threshold,
                                double eps, int max_ticks, double *out_log, int32_t *out_ticks, int32_t *out_status) {
@@ -1294,74 +1468,42 @@ int mpcb_full_closed_loop_host(mpcb_handle *h, int cost_kind, int H, int64_t N, 
     if (!init_state || !target || !origin || !out_log || !out_ticks || !out_status || max_ticks < 1)
         return fail(h, MPCB_ERR_INVALID, "full closed loop: bad arguments");
     if (!h->have_grid) return fail(h, MPCB_ERR_NO_GRID, "mpcb_set_grid has not been called");
+    if (N >= (1LL << 31)) return fail(h, MPCB_ERR_INVALID, "N out of range");
     CK(cudaSetDevice(h->device));
     cudaStream_t st = h->stream;
     const size_t nlog = (size_t)N * max_ticks * 5;
     CK(h->in_state.ensure(sizeof(double) * 3 * N)); CK(h->in_target.ensure(sizeof(double) * 2 * N));
-    CK(h->in_origin.ensure(sizeof(double) * 2 * N)); CK(h->in_thr.ensure(sizeof(double) * N));
-    CK(h->out_cost.ensure(sizeof(double) * N)); CK(h->out_index.ensure(sizeof(int64_t) * N));
-    CK(h->out_traj.ensure(sizeof(double) * 3 * H * N)); CK(h->out_ctl.ensure(sizeof(double) * 2 * N));
+    CK(h->in_origin.ensure(sizeof(double) * 2 * N));
     CK(h->loop_log.ensure(sizeof(double) * nlog)); CK(h->loop_ticks.ensure(sizeof(int) * N));
-    CK(h->loop_status.ensure(sizeof(int) * N)); CK(h->fl_last.ensure(sizeof(double) * 5 * N));
-    CK(h->fl_k.ensure(sizeof(int) * N)); CK(h->fl_have.ensure(sizeof(int) * N));
-    CK(h->fl_flags.ensure(N)); CK(h->fl_count.ensure(sizeof(int)));
-    const size_t nrow = (size_t)N * max_ticks;
-    mpcb_loop_trace dtr{};
-    int rc = stage_trace(h, tr, nrow, H, dtr, N);
-    if (rc) return rc;
-    // robots that start on their target never enter the loop (while not is_on_target, math_model.py:239)
-    std::vector<int> status(N, -1);
-    std::vector<unsigned char> flags(N, 0);
-    std::vector<double> thr(N);
-    int running = 0;
-    for (int64_t i = 0; i < N; ++i) {
-        const double dx = target[2 * i] - init_state[3 * i], dy = target[2 * i + 1] - init_state[3 * i + 1];
-        if (dx * dx + dy * dy <= eps) { status[i] = MPCB_LOOP_ON_TARGET; flags[i] = MPCB_FLAG_SKIP; }
-        else ++running;
-        thr[i] = first_threshold ? first_threshold[i] : INFINITY;
-    }
+    CK(h->loop_status.ensure(sizeof(int) * N));
     CK(cudaMemcpyAsync(h->in_state.p, init_state, sizeof(double) * 3 * N, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(h->in_target.p, target, sizeof(double) * 2 * N, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(h->in_origin.p, origin, sizeof(double) * 2 * N, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(h->in_thr.p, thr.data(), sizeof(double) * N, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(h->loop_status.p, status.data(), sizeof(int) * N, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(h->fl_flags.p, flags.data(), N, cudaMemcpyHostToDevice, st));
-    CK(cudaMemsetAsync(h->fl_k.p, 0, sizeof(int) * N, st));
-    CK(cudaMemsetAsync(h->fl_have.p, 0, sizeof(int) * N, st));
-    CK(cudaMemsetAsync(h->loop_ticks.p, 0, sizeof(int) * N, st));
-    CK(cudaMemsetAsync(h->loop_log.p, 0xFF, sizeof(double) * nlog, st));     // NaN pattern for unused rows
-    CK(cudaStreamSynchronize(st));      // the staging vectors above are pageable
-    FullLoopArgs fa{};
-    fa.N = N; fa.H = H; fa.max_ticks = max_ticks; fa.eps = eps;
-    fa.target = h->in_target.as<double>();
-    fa.best_cost = h->out_cost.as<double>(); fa.best_index = h->out_index.as<long long>();
-    fa.best_traj = h->out_traj.as<double>(); fa.first_control = h->out_ctl.as<double>();
-    fa.state = h->in_state.as<double>(); fa.threshold = h->in_thr.as<double>(); fa.last_ret = h->fl_last.as<double>();
-    fa.kcount = h->fl_k.as<int>(); fa.have_ret = h->fl_have.as<int>(); fa.status = h->loop_status.as<int>();
-    fa.ticks = h->loop_ticks.as<int>(); fa.flags = h->fl_flags.as<unsigned char>();
-    fa.log = h->loop_log.as<double>(); fa.active_count = h->fl_count.as<int>();
-    fa.trace_pred = dtr.pred; fa.trace_ctl = dtr.control; fa.trace_cost = dtr.cost;
-    fa.last_traj = dtr.pred ? h->fl_traj.as<double>() : nullptr;
-    int total_launches = 0;
-    for (int tick = 0; tick < max_ticks && running > 0; ++tick) {
-        CK(cudaMemsetAsync(h->fl_count.p, 0, sizeof(int), st));
-        rc = mpcb_solve_batch_device(h, MPCB_MODE_FULL, cost_kind, H, N, h->in_state.as<double>(),
-                                         h->in_target.as<double>(), h->in_origin.as<double>(), h->in_thr.as<double>(),
-                                         h->fl_flags.as<uint8_t>(), 0, -1, h->out_cost.as<double>(),
-                                         h->out_index.as<int64_t>(), h->out_traj.as<double>(), h->out_ctl.as<double>());
-        if (rc) return rc;
-        total_launches += h->stats.kernel_launches + 1;
-        fa.tick = tick;
-        CK(launch_full_apply(st, fa));
-        CK(cudaMemcpyAsync(&running, h->fl_count.p, sizeof(int), cudaMemcpyDeviceToHost, st));
-        CK(cudaStreamSynchronize(st));
+    const double *d_thr = nullptr;
+    if (first_threshold) {
+        CK(h->in_thr.ensure(sizeof(double) * N));
+        CK(cudaMemcpyAsync(h->in_thr.p, first_threshold, sizeof(double) * N, cudaMemcpyHostToDevice, st));
+        d_thr = h->in_thr.as<double>();
     }
+    CK(cudaMemsetAsync(h->loop_log.p, 0xFF, sizeof(double) * nlog, st));     // NaN pattern for unused rows
+    const size_t nrow = (size_t)N * max_ticks;
+    mpcb_loop_trace dtr{};
+    int rc = stage_trace(h, tr, nrow, H, dtr);
+    if (rc) return rc;
+    int per_tick = 0;
+    rc = full_loop_enqueue(h, cost_kind, H, N, h->in_state.as<double>(), h->in_target.as<double>(),
+                           h->in_origin.as<double>(), d_thr, eps, max_ticks, h->loop_log.as<double>(),
+                           h->loop_ticks.as<int>(), h->loop_status.as<int>(), dtr, &per_tick);
+    if (rc) return rc;
+    int ticks_run = 0;
+    CK(cudaMemcpyAsync(&ticks_run, h->fl_count.as<int>() + 1, sizeof(int), cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(out_log, h->loop_log.p, sizeof(double) * nlog, cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(out_ticks, h->loop_ticks.p, sizeof(int) * N, cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(out_status, h->loop_status.p, sizeof(int) * N, cudaMemcpyDeviceToHost, st));
     CK(copy_back_trace(h, tr, dtr, nrow, H));
     CK(cudaStreamSynchronize(st));
-    h->stats.kernel_launches = total_launches;
+    retire_loop_graphs(h, true);
+    h->stats.kernel_launches = ticks_run * per_tick;   // the solve's launches and the apply kernel, per tick run
     return MPCB_OK;
 }
 

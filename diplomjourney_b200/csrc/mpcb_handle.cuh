@@ -1,6 +1,7 @@
 // mpcb_handle.cuh -- the handle behind the C ABI (private to the library): one device, one stream, its growable
 // device scratch.  Shared by mpcb_api.cu (solves) and mpcb_nccl.cu (cross-rank reconciliation).
 #pragma once
+#include <atomic>
 #include <string>
 #include <vector>
 
@@ -8,15 +9,45 @@
 
 namespace mpcb {
 
+struct DevBuf;
+
+// While the FULL closed loop captures its tick into a graph, no buffer may be freed or moved: the graph keeps the
+// addresses it was captured with, and cudaFree cannot run during a capture.  With `defer` set, a buffer that would
+// have to grow records the size wanted and ensure() fails; the loop grows the buffers after the capture and captures
+// again (full_loop_enqueue, mpcb_api.cu).
+struct DeferredGrowth {
+    bool defer = false;
+    std::vector<std::pair<DevBuf *, size_t>> wanted;
+};
+inline thread_local DeferredGrowth g_growth;
+
+// Bumped whenever a buffer is (re)allocated: a cached FULL loop graph holds the addresses it was captured with.
+inline std::atomic<unsigned long long> g_allocs{0};
+
+// What a FULL loop graph froze at capture besides the handle's buffers (mpcb_api.cu, full_loop_enqueue); compared
+// bytewise, so it is zeroed before it is filled.
+struct LoopGraphKey {
+    unsigned long long epoch, allocs;      // mpcb_handle_s::epoch, g_allocs
+    long long N;
+    int cost_kind, H, max_ticks;
+    double eps;
+    const void *io[10];                    // the caller's inputs, outputs and trace
+};
+
 struct DevBuf {
     void *p = nullptr;
     size_t cap = 0;
     cudaError_t ensure(size_t bytes) {
         if (bytes <= cap) return cudaSuccess;
+        if (g_growth.defer) {
+            g_growth.wanted.emplace_back(this, bytes);
+            return cudaErrorNotPermitted;
+        }
         if (p) cudaFree(p);
         p = nullptr; cap = 0;
         size_t want = bytes + bytes / 4 + 256;
         cudaError_t e = cudaMalloc(&p, want);
+        g_allocs.fetch_add(1);
         if (e == cudaSuccess) cap = want;
         return e;
     }
@@ -66,6 +97,16 @@ struct mpcb_handle_s {
     bool cand_auto = true;              // not set by the user: the prefix algorithm with a node list runs without it
     mpcb::DevBuf nccl_scratch;          // split tree: this rank's (cost, index) records + one slot per rank
     mpcb::DevBuf loop_log, loop_ticks, loop_status, loop_events, loop_final, loop_rng, loop_keys, loop_pcg, loop_pcg_spawn, small_in, small_out, fl_last, fl_k, fl_have, fl_flags, fl_count;
+    mpcb::DevBuf fl_state, fl_thr;      // FULL loop: the robots' running poses and carried thresholds
+    // FULL loop: the executable graph of the last call, launched again while its key holds, with the stats its capture
+    // left and the kernels of one of its ticks; replaced graphs wait in fl_graphs until the stream is idle (destroying
+    // an executable graph waits for the work in flight)
+    unsigned long long epoch = 0;         // bumped by mpcb_set_grid and mpcb_set_option
+    mpcb::LoopGraphKey fl_key{};
+    cudaGraphExec_t fl_exec = nullptr;
+    mpcb_stats fl_stats{};
+    int fl_per_tick = 0;
+    std::vector<cudaGraphExec_t> fl_graphs;
     mpcb_loop_trace trace{};            // of the next closed-loop call (mpcb_set_loop_trace), consumed by it
     mpcb::DevBuf trace_pred, trace_ctl, trace_cost, fl_traj;   // host entries: the trace staged on the device
     void *pin_in = nullptr, *pin_out = nullptr;   // pinned staging of the low-latency path

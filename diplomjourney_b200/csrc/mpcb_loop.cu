@@ -479,11 +479,54 @@ cudaError_t launch_held_small(cudaStream_t st, const SmallArgs &a) {
 }
 
 // ---------------------------------------------------------------------------------------------
-// FULL closed loop: what the host loop of math_model.py:239-254 does between two predictive_control calls,
-// one thread per robot, after the tick's batched solve.
+// FULL closed loop, one graph launch (mpcb_api.cu, full_loop_enqueue):
+//   init -> gate -> WHILE (running > 0 && tick < max_ticks) { batched solve; apply; gate }
+// The running count is ctl[0] (FullLoopArgs::active_count), the tick ctl[1] (FullLoopArgs::tick); both are zero when
+// the init kernel runs, and the gate zeroes the count after reading it, for the apply kernel of the next tick.
+
+// What the loop does before tick 0, one thread per robot: the robot's state and threshold (+inf without first_threshold),
+// zeroed counters, and the on-target test of math_model.py:239 -- a robot on target at entry never runs.
+__global__ void full_loop_init_kernel(const FullLoopArgs a, const double *init, const double *first_threshold) {
+    const long long n = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (n >= a.N) return;
+    const double x = init[3 * n], y = init[3 * n + 1];
+    a.state[3 * n] = x; a.state[3 * n + 1] = y; a.state[3 * n + 2] = init[3 * n + 2];
+    a.threshold[n] = first_threshold ? first_threshold[n] : INFINITY;
+    a.kcount[n] = 0; a.have_ret[n] = 0; a.ticks[n] = 0;
+    // rounded as is_on_target rounds it (no FMA contraction): a robot on the boundary starts as the reference's does
+    const double dx = a.target[2 * n] - x, dy = a.target[2 * n + 1] - y;
+    const bool on_target = __dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)) <= a.eps;
+    a.status[n] = on_target ? MPCB_LOOP_ON_TARGET : -1;
+    a.flags[n] = on_target ? MPCB_FLAG_SKIP : 0;
+    if (!on_target) atomicAdd(a.active_count, 1);
+}
+
+// The WHILE node's condition (one thread): advance the tick (advance = 0 ahead of the loop, 1 at the end of a tick) and
+// take the running count, leaving it zero.
+__global__ void full_loop_gate_kernel(cudaGraphConditionalHandle cond, int *ctl, int max_ticks, int advance) {
+    const int tick = ctl[1] + advance, running = ctl[0];
+    ctl[0] = 0;
+    ctl[1] = tick;
+    cudaGraphSetConditional(cond, running > 0 && tick < max_ticks ? 1u : 0u);
+}
+
+cudaError_t launch_full_loop_init(cudaStream_t st, const FullLoopArgs &a, const double *init, const double *first_threshold) {
+    const int bs = 128;
+    full_loop_init_kernel<<<(unsigned)((a.N + bs - 1) / bs), bs, 0, st>>>(a, init, first_threshold);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_full_loop_gate(cudaStream_t st, cudaGraphConditionalHandle cond, int *ctl, int max_ticks, int advance) {
+    full_loop_gate_kernel<<<1, 1, 0, st>>>(cond, ctl, max_ticks, advance);
+    return cudaGetLastError();
+}
+
+// What the host loop of math_model.py:239-254 does between two predictive_control calls, one thread per robot, after
+// the tick's batched solve.
 __global__ void full_apply_kernel(const FullLoopArgs a) {
     const long long n = blockIdx.x * (long long)blockDim.x + threadIdx.x;
     if (n >= a.N || a.status[n] >= 0) return;
+    const int tick = *a.tick;
     double ret[5];
     const long long idx = a.best_index[n];
     const double *tr = a.best_traj + (size_t)n * 3 * a.H;
@@ -499,7 +542,7 @@ __global__ void full_apply_kernel(const FullLoopArgs a) {
     } else {                                               // stall: the previous path is returned again
         for (int k = 0; k < 5; ++k) ret[k] = a.last_ret[5 * n + k];
     }
-    const size_t row = (size_t)n * a.max_ticks + a.tick;
+    const size_t row = (size_t)n * a.max_ticks + tick;
     double *log = a.log + row * 5;
     for (int k = 0; k < 5; ++k) { log[k] = ret[k]; a.last_ret[5 * n + k] = ret[k]; }
     if (a.trace_pred) {                                    // a stall repeats the last accepted trajectory
@@ -513,14 +556,14 @@ __global__ void full_apply_kernel(const FullLoopArgs a) {
     if (a.trace_cost) a.trace_cost[row] = idx >= 0 ? a.best_cost[n] : NAN;
     const double xprev = a.state[3 * n], yprev = a.state[3 * n + 1];
     a.state[3 * n] = ret[0]; a.state[3 * n + 1] = ret[1]; a.state[3 * n + 2] = ret[2];
-    a.ticks[n] = a.tick + 1;
+    a.ticks[n] = tick + 1;
     int k = a.kcount[n];
     if (ret[0] == xprev && ret[1] == yprev) a.kcount[n] = ++k;
     const double dx = a.target[2 * n] - ret[0], dy = a.target[2 * n + 1] - ret[1];
     int status = -1;
     if (k == 2) status = MPCB_LOOP_STALLED;
     else if (dx * dx + dy * dy <= a.eps) status = MPCB_LOOP_ON_TARGET;
-    else if (a.tick + 1 >= a.max_ticks) status = MPCB_LOOP_MAX_TICKS;
+    else if (tick + 1 >= a.max_ticks) status = MPCB_LOOP_MAX_TICKS;
     if (status >= 0) { a.status[n] = status; a.flags[n] = MPCB_FLAG_SKIP; }
     else atomicAdd(a.active_count, 1);
 }

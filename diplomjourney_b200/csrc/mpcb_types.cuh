@@ -286,7 +286,8 @@ struct WindowArgs {
 // per-tick bookkeeping of the FULL closed loop (mpcb_loop.cu)
 struct FullLoopArgs {
     long long N;
-    int H, tick, max_ticks;
+    int H, max_ticks;
+    const int *tick;                                   // the tick being applied (device counter, advanced by the gate)
     double eps;
     const double *target;                              // [N][2]
     const double *best_cost; const long long *best_index; const double *best_traj, *first_control;   // this tick's solve
@@ -294,7 +295,7 @@ struct FullLoopArgs {
     int *kcount, *have_ret, *status, *ticks;           // [N]
     unsigned char *flags;                              // [N] MPCB_FLAG_SKIP once a robot has stopped
     double *log;                                       // [N][max_ticks][5]
-    int *active_count;
+    int *active_count;                                 // robots still running after this tick
     double *trace_pred, *trace_ctl, *trace_cost;       // per-tick trace as in LoopArgs (nullable)
     double *last_traj;                                 // [N][H][3] the last accepted trajectory (needed with trace_pred)
 };

@@ -362,7 +362,7 @@ typedef struct {
     double *control;   /* [N][max_ticks][2]    */
     double *cost;      /* [N][max_ticks]       */
 } mpcb_loop_trace;
-/* Trace of the NEXT closed-loop call on this handle (any mpcb_held_closed_loop_* entry or mpcb_full_closed_loop_host).
+/* Trace of the NEXT closed-loop call on this handle (any mpcb_held_closed_loop_* or mpcb_full_closed_loop_* entry).
  * Pointers are of the kind that entry takes: host for _host, device for _device.  Each member is nullable.  The call
  * consumes the trace whether it succeeds or fails (a trace left attached would later write into buffers the caller has
  * freed); NULL clears it.  Without a trace every output is what it is without this call. */
@@ -395,12 +395,27 @@ MPCB_API int mpcb_solve_held_windows_device(mpcb_handle *h, const mpcb_loop_para
  * every tick solves all still-running robots in ONE batched FULL solve with the CARRIED threshold
  * (optimal_criterion is only lowered by an accepted leaf, math_model.py:195-198), applies the first pose of the
  * accepted path -- or repeats the previous one when nothing beats the threshold -- counts repeated positions
- * (stop at 2: "Recursive error") and tests is_on_target, all on the device; the host only reads one counter per tick.
- *   init_state[N][3], target[N][2], origin[N][2], first_threshold[N] (control_criterion of the start pose)
- *   out_log[N][max_ticks][5] = the 5-list each tick returns, out_ticks[N], out_status[N] (MPCB_LOOP_*) */
+ * (stop at 2: "Recursive error") and tests is_on_target, all on the device.  The whole run is ONE CUDA-graph launch:
+ * a WHILE node repeats the tick (the batched solve, the apply kernel, a one-thread gate that advances the tick) while a
+ * robot is running and tick < max_ticks, so the host neither launches nor waits per tick.
+ * The handle keeps the loop's graph and launches it again while the grid, the options, N, H, cost, max_ticks, eps
+ * and every pointer are those it was captured with; anything else captures and instantiates a new one.
+ *   init_state[N][3], target[N][2], origin[N][2], first_threshold[N] (control_criterion of the start pose; NULL = +inf)
+ *   out_log[N][max_ticks][5] = the 5-list each tick returns, out_ticks[N], out_status[N] (MPCB_LOOP_*)
+ * The host entry fills the rows of out_log after a robot's last tick with NaN and synchronises once; afterwards
+ * mpcb_get_stats' kernel_launches counts the kernels of every tick run (the solve's and the apply kernel).
+ * The trace of mpcb_set_loop_trace is honoured as by the HELD entries. */
 MPCB_API int mpcb_full_closed_loop_host(mpcb_handle *h, int cost_kind, int H, int64_t N, const double *init_state,
                                const double *target, const double *origin, const double *first_threshold,
                                double eps, int max_ticks, double *out_log, int32_t *out_ticks, int32_t *out_status);
+/* The same loop on device pointers: enqueued on the handle's stream, not synchronised, so one host thread can keep loops
+ * running on several devices at once.  The inputs are only read (the running poses and thresholds live in handle
+ * scratch).  Rows of out_log (and of a trace) after a robot's last tick are NOT written: the caller fills them
+ * beforehand (with NaN, as the host entry does).  N == 0 launches nothing.  kernel_launches (mpcb_get_stats) is the
+ * kernels of ONE tick: the tick count is known on the device only (out_ticks). */
+MPCB_API int mpcb_full_closed_loop_device(mpcb_handle *h, int cost_kind, int H, int64_t N, const double *init_state,
+                                 const double *target, const double *origin, const double *first_threshold,
+                                 double eps, int max_ticks, double *out_log, int32_t *out_ticks, int32_t *out_status);
 
 /* ONE oversized FULL tree per solve, shared by the ranks of an NCCL communicator (one process per GPU): rank r of R
  * expands the first controls of its contiguous, balanced share of [0, S) -- so rank order is leaf-index order --
