@@ -83,7 +83,8 @@ MPCB_HD double exact_terminal(const LaunchArgs &a, const SolveParams &P, double 
     double dl;
     if (x == P.ox && y == P.oy) dl = 1000.0;
     else
-        dl = fabs(dadd(dadd(dmul(P.lineA, x), -dmul(P.lineB, y)), P.lineC)) / P.line_norm;
+        dl = fabs(dadd(dadd(dadd(dmul(P.lineA, x), -dmul(P.lineB, y)), dmul(P.xt, P.oy)), -dmul(P.yt, P.ox))) /
+             P.line_norm;     // ((A x - B y) + x_t y_0) - y_t x_0, left to right as the reference
     double dl2 = dmul(dl, dl);
     if (a.cost_kind == 0) {
         double ang = P.theta - phi;

@@ -1805,8 +1805,9 @@ __global__ void prep_kernel(long long N, const double *__restrict__ state, const
     P.ox = origin[2 * n]; P.oy = origin[2 * n + 1];
     P.theta = atan(P.xt / P.yt);
     P.lineA = P.yt - P.oy; P.lineB = P.xt - P.ox;
-    P.lineC = P.xt * P.oy - P.yt * P.ox;
-    P.line_norm = sqrt(P.lineA * P.lineA + P.lineB * P.lineB);
+    P.lineC = __dadd_rn(__dmul_rn(P.xt, P.oy), -__dmul_rn(P.yt, P.ox));
+    // rounded as the reference rounds it (no FMA contraction)
+    P.line_norm = sqrt(__dadd_rn(__dmul_rn(P.lineA, P.lineA), __dmul_rn(P.lineB, P.lineB)));
     P.threshold = threshold ? threshold[n] : INFINITY;
     P.wl = cost_kind == 0 ? 10.0 : 100.0;
     P.wh = cost_kind == 0 ? 3.16227766016837952 : 0.0;
@@ -1816,7 +1817,8 @@ __global__ void prep_kernel(long long N, const double *__restrict__ state, const
     const double rx = P.xt - P.xs, ry = P.yt - P.ys;
     P.u0 = c0 * rx + s0 * ry; P.w0 = c0 * ry - s0 * rx;
     P.d0 = sqrt(rx * rx + ry * ry);
-    const double E0 = P.lineA * P.xs - P.lineB * P.ys + P.lineC;
+    // the anchor of the fp32 line offsets: its rounding is part of the error model's world-coordinate term below
+    const double E0 = __dadd_rn(__dadd_rn(__dmul_rn(P.lineA, P.xs), -__dmul_rn(P.lineB, P.ys)), P.lineC);
     P.e0 = P.wl * E0 / P.line_norm;
     P.nx0 = P.wl * (P.lineA * c0 - P.lineB * s0) / P.line_norm;
     P.ny0 = P.wl * (-P.lineA * s0 - P.lineB * c0) / P.line_norm;
@@ -1839,6 +1841,20 @@ __global__ void prep_kernel(long long N, const double *__restrict__ state, const
     double M = kWd * Rl * 16.0 + 4.0 * Q * (2.0 * E + Q) + 4.0 * Gl * (Gl + 2.0 * Hh);
     // sin.approx / cos.approx: absolute error 2^-21.4 on [-pi, pi], growing with the argument beyond it
     if (!prefix) M += kWd * Rtot * 8.0 * fmax(1.0, H * dphimax / 3.141592653589793);
+    // float64 rounding at the solve's coordinates (DESIGN.md section 3.3): the costs the window is compared with are the
+    // reference's float64 ones, whose roundings grow with |x|, |y|, |phi|, while the fp32 offsets carry none of them
+    //   heading after H steps: H roundings at |phi| <= Phi                                 -> dphi
+    //   position after H steps: H roundings at |x| <= X, |y| <= Y, and s dphi per step     -> dp (both axes)
+    //   line distance: 4 roundings of the sum at the size of its terms, and dp             -> de (scaled by wl)
+    // each enters the reference's cost once and the anchors e0, hp0 of the fp32 form once
+    const double Phi = fabs(P.phi0) + H * dphimax, X = fabs(P.xs) + Rtot, Y = fabs(P.ys) + Rtot;
+    const double dphi = H * 1.1102230246251565e-16 * Phi;                       // 2^-53
+    const double dp = H * 2.220446049250313e-16 * (X + Y) + H * smax * dphi;    // 2^-52
+    const double lsum = fabs(P.lineA) * X + fabs(P.lineB) * Y + fabs(P.xt * P.oy) + fabs(P.yt * P.ox);
+    const double de = P.wl * (4.440892098500626e-16 * lsum / P.line_norm + dp);  // 2^-51
+    const double dh = P.wh * dphi;
+    const double Mw = (kWd * dp + 2.0 * de * (2.0 * E + de) + 2.0 * dh * (2.0 * Hh + dh)) * 8388608.0;   // in 2^-23
+    M += Mw;
     P.tol = 2.0 * M * 1.1920928955078125e-07 * tol_scale;
     P.tol1 = P.tol;
     if (prefix) {
@@ -1850,7 +1866,7 @@ __global__ void prep_kernel(long long N, const double *__restrict__ state, const
         //   the two accumulating FFMAs round at the magnitude of the whole value (half an ulp each)    -> Vmax
         const double Dmax = P.d0 + Rtot, E1 = E + Q, H1 = Hh + Gl;
         const double Vmax = kWd * Dmax + E1 * E1 + H1 * H1;
-        const double M1 = 3.0 * kWd * Dmax + 2.0 * kWd * smax + 4.0 * E1 * E1 + 3.0 * H1 * H1 + Vmax;
+        const double M1 = 3.0 * kWd * Dmax + 2.0 * kWd * smax + 4.0 * E1 * E1 + 3.0 * H1 * H1 + Vmax + Mw;
         P.tol1 = fmax(P.tol, 2.0 * M1 * 1.1920928955078125e-07 * tol_scale);
     } else {
         // direct form of the leafwalk pass 1 (leaf_walk_direct): the walk's own error (M) plus

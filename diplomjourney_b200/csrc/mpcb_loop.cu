@@ -37,14 +37,14 @@ __device__ __forceinline__ void lex_min_d(double &J, int &j, double oJ, int oj) 
 }
 
 struct LoopCost {
-    double xt, yt, ox, oy, A, B, C, norm, theta;
+    double xt, yt, ox, oy, A, B, xt_oy, yt_ox, norm, theta;    // x_t y_0, y_t x_0: added one at a time
     int kind;
     __device__ double operator()(double x, double y, double phi) const {
         double dx = xt - x, dy = yt - y;
         double d = __dsqrt_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)));
         double dl;
         if (x == ox && y == oy) dl = 1000.0;
-        else dl = fabs(__dadd_rn(__dadd_rn(__dmul_rn(A, x), -__dmul_rn(B, y)), C)) / norm;
+        else dl = fabs(__dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(A, x), -__dmul_rn(B, y)), xt_oy), -yt_ox)) / norm;
         double dl2 = __dmul_rn(dl, dl);
         if (kind == 0) {
             double ang = theta - phi;
@@ -139,15 +139,21 @@ __device__ __forceinline__ void held_block_solve(const mpcb_loop_params &p, cons
         for (int i = 1; i < kLoopThreads / 32; ++i) lex_min_d(bJ, bj, s_J[i], s_j[i]);
 }
 
+// the line constants and the heading reference of a loaded target and line origin, rounded as the reference rounds
+// them (no FMA contraction of A^2 + B^2)
+__device__ __forceinline__ void line_consts(LoopCost &cost) {
+    cost.A = cost.yt - cost.oy; cost.B = cost.xt - cost.ox;
+    cost.xt_oy = __dmul_rn(cost.xt, cost.oy); cost.yt_ox = __dmul_rn(cost.yt, cost.ox);
+    cost.norm = sqrt(__dadd_rn(__dmul_rn(cost.A, cost.A), __dmul_rn(cost.B, cost.B)));
+    cost.theta = atan(cost.xt / cost.yt);
+}
+
 __device__ __forceinline__ void load_cost(LoopCost &cost, const double *target, const double *origin, long long n,
                                           int kind) {
     // (also called with n = 0 on the CTA's shared copy {x_t, y_t}, {x_0, y_0} after an operator event)
     cost.xt = target[2 * n]; cost.yt = target[2 * n + 1];
     cost.ox = origin[2 * n]; cost.oy = origin[2 * n + 1];
-    cost.A = cost.yt - cost.oy; cost.B = cost.xt - cost.ox;
-    cost.C = cost.xt * cost.oy - cost.yt * cost.ox;
-    cost.norm = sqrt(cost.A * cost.A + cost.B * cost.B);
-    cost.theta = atan(cost.xt / cost.yt);
+    line_consts(cost);
     cost.kind = kind;
 }
 
@@ -200,8 +206,8 @@ __global__ void __launch_bounds__(kLoopThreads) held_loop_kernel(const LoopArgs 
             // ---- stop test (thread 0) + acceleration windows (warps 0 and 1)
             if (tid == 0) {
                 const double dx = cost.xt - s_state[0], dy = cost.yt - s_state[1];
-                int stop = 0;
-                if (dx * dx + dy * dy <= p.eps) { stop = 1; status = 0; }
+                int stop = 0;        // rounded as is_on_target rounds it (no FMA contraction)
+                if (__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)) <= p.eps) { stop = 1; status = 0; }
                 else if (ticks >= p.max_ticks) { stop = 1; status = 2; }
                 s_ctl[2] = slow_steps > 0; s_ctl[3] = stop;
             }
@@ -240,7 +246,7 @@ __global__ void __launch_bounds__(kLoopThreads) held_loop_kernel(const LoopArgs 
                     else if (m == 1) { pick = 1; m += 1; }
                     else {
                         const double ex = cost.xt - opt[last], ey = cost.yt - opt[last + 1];
-                        if (ex * ex + ey * ey <= p.eps) m += 1;
+                        if (__dadd_rn(__dmul_rn(ex, ex), __dmul_rn(ey, ey)) <= p.eps) m += 1;
                     }
                     if (pick > p.H - 1) pick = p.H - 1;
                     const double rx = opt[3 * pick], ry = opt[3 * pick + 1], rphi = opt[3 * pick + 2];
@@ -418,10 +424,7 @@ __global__ void __launch_bounds__(kLoopThreads) held_small_kernel(const SmallArg
     LoopCost cost;
     cost.xt = a.target[2 * n]; cost.yt = a.target[2 * n + 1];
     cost.ox = a.origin[2 * n]; cost.oy = a.origin[2 * n + 1];
-    cost.A = cost.yt - cost.oy; cost.B = cost.xt - cost.ox;
-    cost.C = cost.xt * cost.oy - cost.yt * cost.ox;
-    cost.norm = sqrt(cost.A * cost.A + cost.B * cost.B);
-    cost.theta = atan(cost.xt / cost.yt);
+    line_consts(cost);
     cost.kind = a.cost_kind;
     const int fl = a.flags ? (int)a.flags[n] : 0;
     const bool slow = (fl & MPCB_FLAG_SLOW) != 0;
@@ -562,7 +565,7 @@ __global__ void full_apply_kernel(const FullLoopArgs a) {
     const double dx = a.target[2 * n] - ret[0], dy = a.target[2 * n + 1] - ret[1];
     int status = -1;
     if (k == 2) status = MPCB_LOOP_STALLED;
-    else if (dx * dx + dy * dy <= a.eps) status = MPCB_LOOP_ON_TARGET;
+    else if (__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)) <= a.eps) status = MPCB_LOOP_ON_TARGET;   // as is_on_target
     else if (tick + 1 >= a.max_ticks) status = MPCB_LOOP_MAX_TICKS;
     if (status >= 0) { a.status[n] = status; a.flags[n] = MPCB_FLAG_SKIP; }
     else atomicAdd(a.active_count, 1);

@@ -157,6 +157,8 @@ struct __align__(16) SolveParams {
     double ox, oy;              // origin of the tracked line
     double theta;               // arctan(x_t / y_t)                         (math_model.py:83)
     double lineA, lineB, lineC, line_norm;   // (y_t-y_0), (x_t-x_0), x_t y_0 - y_t x_0, sqrt(A^2+B^2)
+                                // (lineC only forms the anchor e0: a leaf's line distance adds x_t y_0 and y_t x_0 one at
+                                // a time, as the reference does -- one precomputed difference rounds otherwise far from (0, 0))
     double threshold;
     // start-frame quantities (frame: origin at the start position, x axis along the start heading)
     double u0, w0, d0;          // target, distance to target

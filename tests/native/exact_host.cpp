@@ -115,3 +115,12 @@ extern "C" void mpcb_test_exact_from_node(const double *v, int nv, const double 
         mpcb::parent_digits(hs.a, p / S, [&](unsigned d) { parent_digits_out[i * (H - 2) + k++] = d; });
     }
 }
+
+// every leaf of one solve (mode 0 FULL: S^H leaves, 1 HELD: S), leaf order, by mpcb::exact_cost
+extern "C" void mpcb_test_exact_costs(const double *v, int nv, const double *beta, int nb, double L, double delta_t,
+                                      int mode, int cost_kind, int H, const double *state, const double *target,
+                                      const double *origin, int slow, double v_min, long long count, double *out) {
+    HostSolve hs;
+    host_solve_setup(hs, v, nv, beta, nb, L, delta_t, mode, cost_kind, H, state, target, origin, slow, v_min);
+    for (long long j = 0; j < count; ++j) out[j] = mpcb::exact_cost(hs.a, hs.P, j, nullptr, nullptr);
+}

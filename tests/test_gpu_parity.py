@@ -254,22 +254,29 @@ def _eps_model(s, origin, H, cost, prefix, smax, dphimax, direct=False):
     ``direct`` tol1/2 (the cheaper direct form the prefix pass 1 ranks with)."""
     xs, ys, p0, xt, yt = s
     wl, wh = (10.0, math.sqrt(10.0)) if cost == C.COST_MM else (100.0, 0.0)
-    A, Bc, Cc = yt - origin[1], xt - origin[0], xt * origin[1] - yt * origin[0]
-    norm = math.hypot(A, Bc)
-    e0 = wl * (A * xs - Bc * ys + Cc) / norm
+    A, Bc = yt - origin[1], xt - origin[0]
+    norm = math.sqrt(A * A + Bc * Bc)
+    e0 = wl * ((A * xs - Bc * ys) + (xt * origin[1] - yt * origin[0])) / norm
     hp0 = wh * (C.heading_reference(xt, yt) - p0)
     Rtot = H * smax
     Rl = smax if prefix else Rtot
     Gl = wh * (dphimax if prefix else H * dphimax)
     E, Hh, Q = abs(e0) + wl * Rtot, abs(hp0) + wh * H * dphimax, wl * Rl
-    M = 1e4 * Rl * 16 + 4 * Q * (2 * E + Q) + 4 * Gl * (Gl + 2 * Hh)
+    # float64 rounding at the solve's coordinates (heading, position, line-distance sum; DESIGN.md section 3.3)
+    Phi, X, Y = abs(p0) + H * dphimax, abs(xs) + Rtot, abs(ys) + Rtot
+    dphi = H * 2.0 ** -53 * Phi
+    dp = H * 2.0 ** -52 * (X + Y) + H * smax * dphi
+    de = wl * (2.0 ** -51 * (abs(A) * X + abs(Bc) * Y + abs(xt * origin[1]) + abs(yt * origin[0])) / norm + dp)
+    dh = wh * dphi
+    Mw = (1e4 * dp + 2 * de * (2 * E + de) + 2 * dh * (2 * Hh + dh)) * 2.0 ** 23
+    M = 1e4 * Rl * 16 + 4 * Q * (2 * E + Q) + 4 * Gl * (Gl + 2 * Hh) + Mw
     if not prefix:
         M += 1e4 * Rtot * 8 * max(1.0, H * dphimax / math.pi)
     if direct:
         d0 = math.hypot(xt - xs, yt - ys)
         Vmax = 1e4 * (d0 + Rtot) + (E + Q) ** 2 + (Hh + Gl) ** 2      # the accumulating FFMAs round at this size
         if prefix:
-            M1 = 3 * 1e4 * (d0 + Rtot) + 2 * 1e4 * smax + 4 * (E + Q) ** 2 + 3 * (Hh + Gl) ** 2 + Vmax
+            M1 = 3 * 1e4 * (d0 + Rtot) + 2 * 1e4 * smax + 4 * (E + Q) ** 2 + 3 * (Hh + Gl) ** 2 + Vmax + Mw
             M = max(M, M1)
         else:
             M = M + 4 * 1e4 * (d0 + Rtot) + 4 * (E + Q) ** 2 + 3 * (Hh + Gl) ** 2 + Vmax

@@ -27,13 +27,15 @@ def _quad_min(e, Q):
     return np.where(ae <= 2 * Q, -0.25 * e * e, Q * (Q - ae))
 
 
-def _bounds(V, B, H, x, k, cost, want_poses=False):
-    """(isotropic bound, heading-aware bound, true minimum over the leaves below) for every depth-(H-k) node."""
+def _bounds(V, B, H, x, k, cost, want_poses=False, og=None):
+    """(isotropic bound, heading-aware bound, true minimum over the leaves below) for every depth-(H-k) node; the
+    line origin `og` is the start unless given."""
     vv, bb, dphi = C.control_tables(V, B, L, DT)
     S = len(vv)
     s = vv * DT
     smax, smin, dmax = np.abs(s).max(), s.min(), np.abs(dphi).max()
-    st, tg, og = x[:3], x[3:5], x[:2]
+    st, tg = x[:3], x[3:5]
+    og = x[:2] if og is None else og
     wl, wh = (10.0, math.sqrt(10.0)) if cost == C.COST_MM else (100.0, 0.0)
     J = C.full_leaf_costs(st, tg, og, V, B, H, cost)
     X, Y, P = np.array([st[0]]), np.array([st[1]]), np.array([st[2]])
@@ -43,8 +45,8 @@ def _bounds(V, B, H, x, k, cost, want_poses=False):
         Y = np.repeat(Y, S) + np.tile(s, len(Y)) * np.sin(P)
     relx, rely = tg[0] - X, tg[1] - Y
     D = np.hypot(relx, rely)
-    A, Bc, Cc = tg[1] - og[1], tg[0] - og[0], tg[0] * og[1] - tg[1] * og[0]
-    e = wl * (A * X - Bc * Y + Cc) / math.hypot(A, Bc)
+    A, Bc = tg[1] - og[1], tg[0] - og[0]
+    e = wl * ((A * X - Bc * Y) + tg[0] * og[1] - tg[1] * og[0]) / math.hypot(A, Bc)
     hp = wh * (C.heading_reference(tg[0], tg[1]) - P)
     reach_iso = k * smax
     Q = wl * k * smax
@@ -135,6 +137,33 @@ def test_line_offset_interval_matters_for_the_tree_cost():
     assert np.mean(surv_new) < 0.25 * np.mean(surv_iso), (np.mean(surv_iso), np.mean(surv_new))
 
 
+def tol_model(x, og, H, cost, smax, dphimax):
+    """Python mirror of the window widths prep_kernel gives a prefix-algorithm solve (csrc/mpcb_kernels.cu, DESIGN.md
+    section 3.3): (tol, tol1), each twice an error bound, incl. the float64 rounding at the solve's coordinates."""
+    xs, ys, p0, xt, yt = x
+    ox, oy = og
+    wl, wh = (10.0, math.sqrt(10.0)) if cost == C.COST_MM else (100.0, 0.0)
+    A, Bc = yt - oy, xt - ox
+    norm = math.sqrt(A * A + Bc * Bc)
+    e0 = wl * ((A * xs - Bc * ys) + (xt * oy - yt * ox)) / norm
+    hp0 = wh * (C.heading_reference(xt, yt) - p0)
+    d0 = math.hypot(xt - xs, yt - ys)
+    Rtot, Rl, Gl = H * smax, smax, wh * dphimax
+    E, Hh, Q = abs(e0) + wl * Rtot, abs(hp0) + wh * H * dphimax, wl * Rl
+    Phi, X, Y = abs(p0) + H * dphimax, abs(xs) + Rtot, abs(ys) + Rtot
+    dphi = H * 2.0 ** -53 * Phi
+    dp = H * 2.0 ** -52 * (X + Y) + H * smax * dphi
+    de = wl * (2.0 ** -51 * (abs(A) * X + abs(Bc) * Y + abs(xt * oy) + abs(yt * ox)) / norm + dp)
+    dh = wh * dphi
+    Mw = (1e4 * dp + 2 * de * (2 * E + de) + 2 * dh * (2 * Hh + dh)) * 2.0 ** 23
+    M = 1e4 * Rl * 16 + 4 * Q * (2 * E + Q) + 4 * Gl * (Gl + 2 * Hh) + Mw
+    Dmax, E1, H1 = d0 + Rtot, E + Q, Hh + Gl
+    Vmax = 1e4 * Dmax + E1 * E1 + H1 * H1
+    M1 = 3e4 * Dmax + 2e4 * smax + 4 * E1 * E1 + 3 * H1 * H1 + Vmax + Mw
+    tol = 2 * M * 2.0 ** -23
+    return tol, max(tol, 2 * M1 * 2.0 ** -23)
+
+
 # ---------------------------------------------------------------- the shipped CUDA source, compiled for the host
 @pytest.fixture(scope="module")
 def shipped_bound():
@@ -150,19 +179,20 @@ def shipped_bound():
     dp = ctypes.POINTER(ctypes.c_double)
     lib.mpcb_test_subtree_lower_bounds.argtypes = [ctypes.c_double] * 3 + [dp, ctypes.c_longlong, dp, dp, dp, ctypes.c_int, dp]
 
-    def bound(x, cost, poses, consts, k):
-        """J lower bound (absolute cost) of every node in `poses` with k steps to go, by the library's own code."""
+    def bound(x, cost, poses, consts, k, og=None):
+        """J lower bound (absolute cost) of every node in `poses` with k steps to go, by the library's own code (line
+        origin `og`, default the start)."""
         X, Y, P = poses
         smax, smin, dmax, wl, wh = consts
         xs, ys, p0, xt, yt = x
-        ox, oy = x[0], x[1]                                           # the line origin is the start in these scenarios
+        ox, oy = (xs, ys) if og is None else og
         c0, s0 = math.cos(p0), math.sin(p0)
-        # SolveParams exactly as prep_kernel builds them (csrc/mpcb_kernels.cu)
-        A, Bc, Cc = yt - oy, xt - ox, xt * oy - yt * ox
-        norm = math.hypot(A, Bc)
+        # SolveParams exactly as prep_kernel builds them (csrc/mpcb_kernels.cu); e0 in the reference's order
+        A, Bc = yt - oy, xt - ox
+        norm = math.sqrt(A * A + Bc * Bc)
         rx, ry = xt - xs, yt - ys
         u0, w0, d0 = c0 * rx + s0 * ry, c0 * ry - s0 * rx, math.hypot(rx, ry)
-        e0 = wl * (A * xs - Bc * ys + Cc) / norm
+        e0 = wl * ((A * xs - Bc * ys) + (xt * oy - yt * ox)) / norm
         nx0, ny0 = wl * (A * c0 - Bc * s0) / norm, wl * (-A * s0 - Bc * c0) / norm
         hp0 = wh * (C.heading_reference(xt, yt) - p0)
         kbase = 1e4 * d0 + e0 * e0 + hp0 * hp0
@@ -177,12 +207,7 @@ def shipped_bound():
             out32 = np.empty(len(xi), np.float32)
             lib.mpcb_test_prefilter32(smax, smin, dmax, p(solve), len(xi), p(xi), p(eta), p(psi),
                                       out32.ctypes.data_as(ctypes.POINTER(ctypes.c_float)), k)
-            H = 3
-            Rtot = H * smax
-            E1 = abs(e0) + wl * Rtot + wl * smax
-            H1 = abs(hp0) + wh * H * dmax + wh * dmax
-            Dmax = d0 + Rtot
-            tol1 = 2.0 ** -22 * (4e4 * Dmax + 2e4 * smax + 5 * E1 * E1 + 4 * H1 * H1)      # prep_kernel's tol1 (prefix)
+            _, tol1 = tol_model(x, (ox, oy), 3, cost, smax, dmax)
             bound.prefilter = (out32.astype(np.float64), out, tol1)
         return kbase + out
     lib.mpcb_test_prefilter32.argtypes = [ctypes.c_double] * 3 + [dp, ctypes.c_longlong, dp, dp, dp, ctypes.POINTER(ctypes.c_float),
@@ -231,3 +256,57 @@ def test_fp32_prefilter_stays_within_its_margin_of_the_float64_bound(shipped_bou
             assert err <= tol1, (grid, cost, steps, err, tol1)        # the analysis in mpcb_bounds.cuh; the kernel allows 8x
         assert worst > 0.0
         print(f"fp32 pre-filter, {steps} step(s): worst |lb32 - lb64| = {worst:.3f} tol1 ({grid}, {cost})")
+
+
+WORLD_SHIFTS = [0.0, 1e3, 1e5, 5e5, 5e6]
+
+
+def world_bound_scenarios(shift, seed):
+    """(x, origin) around the world point (shift, 0.9 shift): the line origin 0-300 m off the start, headings accumulated
+    to +-10..60 rad as closed loops leave them, targets 30-3,000 m away, and one robot next to its target."""
+    rng = np.random.default_rng(seed)
+    out = []
+    for k in range(8):
+        x = C.random_scenarios(1, seed * 10 + k)[0]
+        x[[0, 3]] += shift
+        x[[1, 4]] += 0.9 * shift
+        og = x[:2] + rng.uniform(-300, 300, 2) * [0.0, 0.02, 0.1, 1.0][k % 4]
+        if k % 3 == 1:
+            x[2] += rng.choice([-1.0, 1.0]) * rng.uniform(10, 60)
+        if k % 4 == 2:
+            ang, dist = rng.uniform(-math.pi, math.pi), rng.uniform(30, 3000)
+            x[3:5] = x[:2] + dist * np.array([math.cos(ang), math.sin(ang)])
+        if k == 7:
+            x[3:5] = x[:2] + [0.05, 0.02]
+        out.append((x, og))
+    return out
+
+
+@pytest.mark.parametrize("grid", sorted(GRIDS))
+@pytest.mark.parametrize("cost", [C.COST_MM, C.COST_TREE])
+def test_shipped_bound_cuts_only_what_the_window_allows_far_from_the_world_origin(shipped_bound, grid, cost):
+    """Off the line origin and far from the world origin the oracle's float64 costs carry rounding noise that grows with
+    the coordinates (tens of cost units at 5e6 m), which the bound, formed from anchors in the start frame, does not.
+    The kernel cuts a node when LB > UB + tol1 + tol, so what must hold is LB <= true_min + tol1 + tol with the windows
+    prep_kernel computes (tol_model) -- for every node of small trees, with the shipped code, in every region -- and the
+    fp32 pre-filter must stay within tol1 of the float64 bound."""
+    V, B = GRIDS[grid]
+    for shift in WORLD_SHIFTS:
+        worst, worst32 = -np.inf, 0.0
+        for x, og in world_bound_scenarios(shift, int(shift) % 997 + 3):
+            for k in (1, 2, 3):
+                _, true_min, poses, consts = _bounds(V, B, 3, x, k, cost, want_poses=True, og=og)
+                lb = shipped_bound(x, cost, poses, consts, k, og=og)
+                tol, tol1 = tol_model(x, og, 3, cost, consts[0], consts[2])
+                ok = np.isfinite(true_min)
+                excess = (lb[ok] - true_min[ok]).max()
+                assert excess <= tol1 + tol, (shift, k, excess, tol1 + tol)
+                worst = max(worst, excess / (tol1 + tol))
+                if k in (1, 2):
+                    lb32, lb64, ptol1 = shipped_bound.prefilter
+                    fin = np.isfinite(lb64)
+                    err = np.abs(lb32[fin] - lb64[fin]).max()
+                    assert err <= ptol1, (shift, k, err, ptol1)
+                    worst32 = max(worst32, err / ptol1)
+        print(f"{grid} {cost} shift {shift:g}: worst (LB - true min) = {worst:.3g} (tol1 + tol), "
+              f"|lb32 - lb64| = {worst32:.3g} tol1")
