@@ -57,6 +57,15 @@ class LoopParams(C.Structure):
 
 
 LOOP_ON_TARGET, LOOP_STALLED, LOOP_MAX_TICKS, LOOP_NO_LEAF = 0, 1, 2, 3
+LOOP_RUNNING = -1
+
+
+class HeldCtrl(C.Structure):
+    """mpcb_held_ctrl (include/mpcb200.h): one robot's online controller between two steps, in device memory."""
+    _fields_ = [("pose", C.c_double * 5), ("line", C.c_double * 4), ("threshold", C.c_double), ("prev", C.c_double * 2),
+                ("opt", C.c_double * (3 * MAX_H)), ("command", C.c_double * 2), ("slow_steps", C.c_int32), ("m", C.c_int32),
+                ("ticks", C.c_int32), ("status", C.c_int32), ("recursive", C.c_int32), ("have_traj", C.c_int32),
+                ("pending", C.c_int32), ("reserved", C.c_int32)]
 
 
 class LoopEvent(C.Structure):
@@ -125,6 +134,9 @@ def load():
     lib.mpcb_full_closed_loop_host.argtypes = [vp, C.c_int, C.c_int, C.c_int64, vp, vp, vp, vp, C.c_double, C.c_int, vp, vp, vp]
     lib.mpcb_full_closed_loop_device.argtypes = lib.mpcb_full_closed_loop_host.argtypes
     lib.mpcb_set_loop_trace.argtypes = [vp, C.POINTER(LoopTrace)]
+    lib.mpcb_held_ctrl_init_device.argtypes = [vp, C.POINTER(LoopParams), C.c_int64, vp, vp, vp, vp, vp, vp]
+    lib.mpcb_held_ctrl_step_device.argtypes = [vp, C.POINTER(LoopParams), C.c_int64, vp, vp, vp, C.c_int32, C.c_double,
+                                               vp, vp]
     split = [vp, vp, C.c_int, C.c_int, C.c_int64, vp, vp, vp, vp, vp, vp, vp, vp]
     lib.mpcb_solve_tree_split_host.argtypes = split
     lib.mpcb_solve_tree_split_device.argtypes = split
@@ -592,6 +604,30 @@ class Solver:
                                                              vp(origin), vp(first_threshold), vp(slow_steps), ev, n_ev,
                                                              float(radius_u_turn), vp(pcg_state), vp(out_log),
                                                              vp(out_ticks), vp(out_status), vp(out_final)))
+
+    def held_ctrl_init_device(self, params: "LoopParams", N, init, target, origin, first_threshold, slow_steps, ctrl):
+        """mpcb_held_ctrl_init_device: sets up the [N] ``HeldCtrl`` records at ``ctrl`` as the closed loop sets up a robot
+        -- init [N][5] x, y, phi, v, beta, target / origin [N][2] float64, first_threshold [N] float64 or 0 (= +inf),
+        slow_steps [N] int32 or 0.  Raw device addresses (e.g. torch.Tensor.data_ptr()); enqueues on self.stream, does
+        not synchronise."""
+        vp = lambda x: C.c_void_p(int(x)) if x else None
+        self._ck(self.lib.mpcb_held_ctrl_init_device(self.h, C.byref(params), int(N), vp(init), vp(target), vp(origin),
+                                                     vp(first_threshold), vp(slow_steps), vp(ctrl)))
+
+    def held_ctrl_step_device(self, params: "LoopParams", N, ctrl, measured=0, events=0, n_ev=0, radius_u_turn=0.0,
+                              proposal=0, running=0):
+        """mpcb_held_ctrl_step_device: one step of the online controller on the [N] ``HeldCtrl`` records at ``ctrl``
+        (set up by ``held_ctrl_init_device`` with the same ``params``).  A robot holding a proposal commits measured[n]
+        (the [N][5] applied x, y, phi, v, beta; 0 = the proposal unchanged) and then its events [N][n_ev]
+        (``LoopEvent`` rows, ``tick`` ignored, kind 0 = empty slot); a running robot then writes its next proposal to
+        proposal [N][5] (NaN rows for the others), and ``running`` (a device int32, zeroed by the caller) receives the
+        number of robots holding one.  Raw device addresses; enqueues on self.stream, does not synchronise.
+        Run the plant between two steps on ``torch.cuda.ExternalStream(solver.stream)``: then the stream orders the
+        plant after the step that made the proposal and before the step that commits it, and no step needs a
+        synchronisation (reading ``running`` is the only one)."""
+        vp = lambda x: C.c_void_p(int(x)) if x else None
+        self._ck(self.lib.mpcb_held_ctrl_step_device(self.h, C.byref(params), int(N), vp(ctrl), vp(measured), vp(events),
+                                                     int(n_ev), float(radius_u_turn), vp(proposal), vp(running)))
 
     def full_closed_loop(self, cost, H, init_state, target, origin, first_threshold=None, eps=0.001, max_ticks=256,
                          trace=False):

@@ -45,6 +45,10 @@ cudaError_t launch_full_apply(cudaStream_t, const FullLoopArgs &);
 cudaError_t launch_full_loop_init(cudaStream_t, const FullLoopArgs &, const double *init, const double *first_threshold);
 cudaError_t launch_full_loop_gate(cudaStream_t, cudaGraphConditionalHandle, int *ctl, int max_ticks, int advance);
 cudaError_t launch_held_windows(cudaStream_t, const WindowArgs &, int sms);
+cudaError_t launch_held_ctrl_init(cudaStream_t, long long N, const double *init, const double *target,
+                                  const double *origin, const double *first_threshold, const int *slow_steps,
+                                  mpcb_held_ctrl *ctrl);
+cudaError_t launch_held_ctrl_step(cudaStream_t, const HeldCtrlArgs &, int sms);
 cudaError_t launch_split_ub_min(cudaStream_t, const LaunchArgs &, const unsigned long long *all, int nranks);
 cudaError_t launch_split_pack(cudaStream_t, const LaunchArgs &, SplitRec *mine);
 cudaError_t launch_split_pick(cudaStream_t, const LaunchArgs &, const SplitRec *all, int nranks);
@@ -884,6 +888,14 @@ int mpcb_set_loop_trace(mpcb_handle *h, const mpcb_loop_trace *trace) {
     return MPCB_OK;
 }
 
+// the ranges of a closed loop's parameters
+static int check_loop_params(mpcb_handle *h, const mpcb_loop_params *p) {
+    if (p->H < 1 || p->H > MPCB_MAX_H || p->max_ticks < 1 || p->n_v < 1 || p->n_beta < 1 || p->n_v > 128 || p->n_beta > 128)
+        return fail(h, MPCB_ERR_INVALID, "closed loop: bad parameters (H=%d, max_ticks=%d, n_v=%d, n_beta=%d)", p->H,
+                    p->max_ticks, p->n_v, p->n_beta);
+    return MPCB_OK;
+}
+
 // device pointers throughout, except the event script (checked by the caller with check_events), which is copied into
 // handle scratch here; events / out_final / rng_state / pcg_state and the trace's members may be null (at most one of
 // rng_state and pcg_state is not)
@@ -897,9 +909,8 @@ static int held_loop_core(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, 
     if (N == 0) return MPCB_OK;
     if (!init || !target || !origin || !out_log || !out_ticks || !out_status)
         return fail(h, MPCB_ERR_INVALID, "closed loop: null pointer");
-    if (p->H < 1 || p->H > MPCB_MAX_H || p->max_ticks < 1 || p->n_v < 1 || p->n_beta < 1 || p->n_v > 128 || p->n_beta > 128)
-        return fail(h, MPCB_ERR_INVALID, "closed loop: bad parameters (H=%d, max_ticks=%d, n_v=%d, n_beta=%d)", p->H,
-                    p->max_ticks, p->n_v, p->n_beta);
+    int rc = check_loop_params(h, p);
+    if (rc) return rc;
     CK(cudaSetDevice(h->device));
     const mpcb_loop_event *d_events = nullptr;
     if (events && n_events > 0) {
@@ -1207,6 +1218,45 @@ int mpcb_pcg64_seed_device(mpcb_handle *h, int64_t N, const uint32_t *entropy, i
     CK(cudaSetDevice(h->device));
     CK(launch_pcg64_seed(h->stream, N, entropy, entropy_len, entropy_stride, spawn_len > 0 ? spawn_key : nullptr,
                          spawn_len, reinterpret_cast<unsigned long long *>(pcg_state)));
+    return MPCB_OK;
+}
+
+int mpcb_held_ctrl_init_device(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, const double *init,
+                               const double *target, const double *origin, const double *first_threshold,
+                               const int32_t *slow_steps, mpcb_held_ctrl *ctrl) {
+    if (!h || !p) return MPCB_ERR_INVALID;
+    if (N < 0 || N >= (1LL << 31)) return fail(h, MPCB_ERR_INVALID, "N out of range");
+    if (N == 0) return MPCB_OK;
+    if (!init || !target || !origin || !ctrl) return fail(h, MPCB_ERR_INVALID, "controller records: null pointer");
+    int rc = check_loop_params(h, p);
+    if (rc) return rc;
+    CK(cudaSetDevice(h->device));
+    CK(launch_held_ctrl_init(h->stream, N, init, target, origin, first_threshold, slow_steps, ctrl));
+    h->stats = mpcb_stats{};
+    h->stats.kernel_launches = 1;
+    return MPCB_OK;
+}
+
+int mpcb_held_ctrl_step_device(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, mpcb_held_ctrl *ctrl,
+                               const double *measured, const mpcb_loop_event *events, int32_t n_ev,
+                               double radius_u_turn, double *proposal, int32_t *running) {
+    if (!h || !p) return MPCB_ERR_INVALID;
+    if (N < 0 || N >= (1LL << 31)) return fail(h, MPCB_ERR_INVALID, "N out of range");
+    if (n_ev < 0 || n_ev > 64 || (n_ev > 0 && !events))
+        return fail(h, MPCB_ERR_INVALID, "controller step: bad events (n_ev=%d, events %s)", n_ev, events ? "set" : "null");
+    if (N == 0) return MPCB_OK;
+    if (!ctrl) return fail(h, MPCB_ERR_INVALID, "controller step: null records");
+    int rc = check_loop_params(h, p);
+    if (rc) return rc;
+    CK(cudaSetDevice(h->device));
+    HeldCtrlArgs a{};
+    a.p = *p; a.N = N; a.ctrl = ctrl; a.measured = measured;
+    a.events = n_ev > 0 ? events : nullptr; a.n_ev = n_ev > 0 ? n_ev : 0; a.radius_u_turn = radius_u_turn;
+    a.proposal = proposal; a.running = running;
+    CK(launch_held_ctrl_step(h->stream, a, h->sms));
+    h->stats = mpcb_stats{};
+    h->stats.kernel_launches = 1;
+    h->stats.algo = MPCB_ALGO_LEAFWALK;
     return MPCB_OK;
 }
 

@@ -157,6 +157,78 @@ __device__ __forceinline__ void load_cost(LoopCost &cost, const double *target, 
     cost.kind = kind;
 }
 
+// ---- the tick of the online controller, shared by held_loop_kernel (the whole loop in one launch) and
+// held_ctrl_step_kernel (one tick per launch, the state in an mpcb_held_ctrl record): what thread 0 carries from tick to
+// tick (math_mpc's locals and the module globals it touches), and the thread-0 parts of a tick on it.  A tick splits
+// where the actuator sits: the head proposes a pose and a command, the plant (the identity, numpy's noise, or a
+// caller's own) turns them into the applied state, and the tail commits that state.
+struct LoopTick {
+    double thr;                             // optimal_criterion
+    int slow_steps, m, ticks, status;       // steps_for_slowing, the finishing counter, ticks committed, MPCB_LOOP_*
+    bool recursive, have_traj;              // repeated position seen; optimal_trajectory is no longer the placeholder
+    double res_v, res_beta;                 // optimal_trajectory's commanded (v, beta); its poses are an array of their own
+    double xprev, yprev;                    // the position committed by the previous tick
+};
+
+// stop test at the top of a tick (the while condition of math_mpc and the tick bound), on the committed position
+__device__ __forceinline__ bool tick_stop(const mpcb_loop_params &p, const LoopCost &cost, LoopTick &t, double x, double y) {
+    const double dx = cost.xt - x, dy = cost.yt - y;
+    bool stop = false;                      // rounded as is_on_target rounds it (no FMA contraction)
+    if (__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)) <= p.eps) { stop = true; t.status = MPCB_LOOP_ON_TARGET; }
+    else if (t.ticks >= p.max_ticks) { stop = true; t.status = MPCB_LOOP_MAX_TICKS; }
+    return stop;
+}
+
+// head, after the HELD solve (thread 0): accept the solve's leaf under the threshold, the slow-down countdown, the no-leaf
+// stop and the finishing heuristic (math_model_tree.py:351-429).  Returns false on the no-leaf stop; otherwise the
+// proposed pose is (rx, ry, rphi) and the command (t.res_v, t.res_beta).  opt[3 H]: optimal_trajectory's poses (kept out
+// of LoopTick: an indexed array inside the struct would take the whole struct to the stack).
+__device__ __forceinline__ bool tick_propose(const mpcb_loop_params &p, const LoopCost &cost, LoopTick &t, double *opt,
+                                             bool accepted,
+                                             int bj, int nB, bool slow, double vslow, const double *s_V,
+                                             const double *s_B, const double *s_tanB, double x0, double y0,
+                                             double phi0, double &rx, double &ry, double &rphi) {
+    if (accepted) {
+        const int iv = bj / nB, ib = bj - iv * nB;
+        t.res_v = slow ? vslow : s_V[iv];
+        t.res_beta = s_B[ib];
+        double x = x0, y = y0, phi = phi0;
+        loop_walk(p, t.res_v, s_tanB[ib], x, y, phi, opt);
+        t.have_traj = true;
+    }
+    t.slow_steps -= 1;
+    if (!t.have_traj) { t.status = MPCB_LOOP_NO_LEAF; return false; }  // reference: IndexError on the [[[0]]] placeholder
+    // finishing heuristic (math_model_tree.py:392-414)
+    int pick = 0;
+    const int last = 3 * (p.H - 1);
+    if (t.m == 2) pick = 2;
+    else if (t.m == 1) { pick = 1; t.m += 1; }
+    else {
+        const double ex = cost.xt - opt[last], ey = cost.yt - opt[last + 1];
+        if (__dadd_rn(__dmul_rn(ex, ex), __dmul_rn(ey, ey)) <= p.eps) t.m += 1;
+    }
+    if (pick > p.H - 1) pick = p.H - 1;
+    rx = opt[3 * pick]; ry = opt[3 * pick + 1]; rphi = opt[3 * pick + 2];
+    t.thr = 9223372036854775807.0;            // sys.maxsize (math_model_tree.py:428)
+    return true;
+}
+
+// tail (thread 0): commit the applied position (x, y) -- the repeated-position stop ("Recursive error.",
+// math_model_tree.py:559-563) and, when the robot goes on, `events()`, the operator events of this tick (:564-569).
+// Returns true on the stall stop.
+template <class Events>
+__device__ __forceinline__ bool tick_commit(LoopTick &t, double x, double y, Events &&events) {
+    t.ticks += 1;
+    bool stop = false;
+    if (t.recursive) { stop = true; t.status = MPCB_LOOP_STALLED; }
+    else {
+        if (x == t.xprev && y == t.yprev) t.recursive = true;
+        events();
+    }
+    t.xprev = x; t.yprev = y;
+    return stop;
+}
+
 enum LoopGen { kGenNone = 0, kGenMt19937 = 1, kGenPcg64 = 2 };    // the actual run's generator kind
 
 // kTrace: the per-tick trace is written (LoopArgs::trace_*, each still nullable).  A template parameter, so that the loop
@@ -185,17 +257,19 @@ __global__ void __launch_bounds__(kLoopThreads) held_loop_kernel(const LoopArgs 
         LoopCost cost;
         load_cost(cost, a.target, a.origin, n, p.cost_kind);
         // thread-0 state of the loop (math_mpc locals and the module globals it touches)
-        double thr = a.first_threshold ? a.first_threshold[n] : INFINITY;
-        int slow_steps = a.slow_steps ? a.slow_steps[n] : 0;
-        int m = 0, ticks = 0, status = 2;
-        bool recursive = false, have_traj = false;
-        double opt[3 * MPCB_MAX_H], res_v = 0.0, res_beta = 0.0;
-        double xprev = 0.0, yprev = 0.0;
+        LoopTick t;
+        t.thr = a.first_threshold ? a.first_threshold[n] : INFINITY;
+        t.slow_steps = a.slow_steps ? a.slow_steps[n] : 0;
+        t.m = 0; t.ticks = 0; t.status = MPCB_LOOP_MAX_TICKS;
+        t.recursive = false; t.have_traj = false;
+        t.res_v = 0.0; t.res_beta = 0.0;
+        t.xprev = 0.0; t.yprev = 0.0;
+        double opt[3 * MPCB_MAX_H];
         Pcg64 pcg;                                 // PCG64: the running robot's generator (thread 0)
         __syncthreads();                           // the previous robot's shared state has been consumed
         if (tid == 0) {
             for (int k = 0; k < 5; ++k) s_state[k] = a.init[5 * n + k];
-            xprev = s_state[0]; yprev = s_state[1];
+            t.xprev = s_state[0]; t.yprev = s_state[1];
             if constexpr (kGen == kGenPcg64) pcg = pcg64_load(a.pcg_state + (size_t)n * kPcgWords);
         }
         if constexpr (kGen == kGenMt19937)
@@ -205,11 +279,8 @@ __global__ void __launch_bounds__(kLoopThreads) held_loop_kernel(const LoopArgs 
         for (;;) {
             // ---- stop test (thread 0) + acceleration windows (warps 0 and 1)
             if (tid == 0) {
-                const double dx = cost.xt - s_state[0], dy = cost.yt - s_state[1];
-                int stop = 0;        // rounded as is_on_target rounds it (no FMA contraction)
-                if (__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)) <= p.eps) { stop = 1; status = 0; }
-                else if (ticks >= p.max_ticks) { stop = 1; status = 2; }
-                s_ctl[2] = slow_steps > 0; s_ctl[3] = stop;
+                const bool stop = tick_stop(p, cost, t, s_state[0], s_state[1]);
+                s_ctl[2] = t.slow_steps > 0; s_ctl[3] = stop;
             }
             build_windows(p, s_state[3], s_state[4], s_V, s_B, s_ctl, &s_vslow);
             __syncthreads();
@@ -226,42 +297,23 @@ __global__ void __launch_bounds__(kLoopThreads) held_loop_kernel(const LoopArgs 
 
             // ---- apply (thread 0)
             if (tid == 0) {
-                const bool accepted = bj >= 0 && bJ < thr;  // strict '<' (math_model_tree.py:351)
-                if (accepted) {
-                    const int iv = bj / nB, ib = bj - iv * nB;
-                    res_v = slow ? s_vslow : s_V[iv];
-                    res_beta = s_B[ib];
-                    double x = x0, y = y0, phi = phi0;
-                    loop_walk(p, res_v, s_tanB[ib], x, y, phi, opt);
-                    have_traj = true;
-                }
-                slow_steps -= 1;
+                const bool accepted = bj >= 0 && bJ < t.thr;  // strict '<' (math_model_tree.py:351)
+                double rx, ry, rphi;
                 int stop = 0;
-                if (!have_traj) { stop = 1; status = 3; }   // reference: IndexError on the [[[0]]] placeholder
+                if (!tick_propose(p, cost, t, opt, accepted, bj, nB, slow, s_vslow, s_V, s_B, s_tanB, x0, y0, phi0, rx, ry,
+                                  rphi)) stop = 1;
                 else {
-                    // finishing heuristic (math_model_tree.py:392-414)
-                    int pick = 0;
-                    const int last = 3 * (p.H - 1);
-                    if (m == 2) pick = 2;
-                    else if (m == 1) { pick = 1; m += 1; }
-                    else {
-                        const double ex = cost.xt - opt[last], ey = cost.yt - opt[last + 1];
-                        if (__dadd_rn(__dmul_rn(ex, ex), __dmul_rn(ey, ey)) <= p.eps) m += 1;
-                    }
-                    if (pick > p.H - 1) pick = p.H - 1;
-                    const double rx = opt[3 * pick], ry = opt[3 * pick + 1], rphi = opt[3 * pick + 2];
-                    thr = 9223372036854775807.0;            // sys.maxsize (math_model_tree.py:428)
                     // the applied (v, beta): the commanded ones, or in the actual run what the actuators make of them
                     // (math_model_tree.py:590-597) -- velocity drawn first, then beta, and before the stall stop
-                    double av = res_v, ab = res_beta;
+                    double av = t.res_v, ab = t.res_beta;
                     if constexpr (kGen == kGenMt19937) {
-                        av = actual_velocity(res_v, s_mt);
-                        ab = actual_beta(res_beta, s_mt);
+                        av = actual_velocity(t.res_v, s_mt);
+                        ab = actual_beta(t.res_beta, s_mt);
                     } else if constexpr (kGen == kGenPcg64) {
-                        av = actual_velocity(res_v, pcg);
-                        ab = actual_beta(res_beta, pcg);
+                        av = actual_velocity(t.res_v, pcg);
+                        ab = actual_beta(t.res_beta, pcg);
                     }
-                    const size_t row = (size_t)n * p.max_ticks + ticks;
+                    const size_t row = (size_t)n * p.max_ticks + t.ticks;
                     double *log = a.out_log + row * 5;
                     log[0] = rx; log[1] = ry; log[2] = rphi; log[3] = av; log[4] = ab;
                     // the trace: what the reference's tick logs besides the 5-list (predicted_trajectory_*, result_v /
@@ -269,25 +321,21 @@ __global__ void __launch_bounds__(kLoopThreads) held_loop_kernel(const LoopArgs 
                     if constexpr (kTrace) {
                         if (a.trace_pred)
                             for (int k = 0; k < 3 * p.H; ++k) a.trace_pred[row * 3 * p.H + k] = opt[k];
-                        if (a.trace_ctl) { a.trace_ctl[2 * row] = res_v; a.trace_ctl[2 * row + 1] = res_beta; }
+                        if (a.trace_ctl) { a.trace_ctl[2 * row] = t.res_v; a.trace_ctl[2 * row + 1] = t.res_beta; }
                         if (a.trace_cost) a.trace_cost[row] = accepted ? bJ : NAN;
                     }
                     s_state[0] = rx; s_state[1] = ry; s_state[2] = rphi; s_state[3] = av; s_state[4] = ab;
-                    ticks += 1;
-                    if (recursive) { stop = 1; status = 1; }        // "Recursive error." (math_model_tree.py:559-561)
-                    else {
-                        if (rx == xprev && ry == yprev) recursive = true;
+                    stop = tick_commit(t, rx, ry, [&] {
                         // operator events of this tick (math_model_tree.py:564-569), in script order
                         bool fired = false;
                         for (int e = 0; e < a.n_events; ++e)
-                            if (a.events[e].tick == ticks) {
+                            if (a.events[e].tick == t.ticks) {
                                 if (!fired) { s_line[0] = cost.xt; s_line[1] = cost.yt; s_line[2] = cost.ox; s_line[3] = cost.oy; }
-                                apply_event(a.events[e], a.radius_u_turn, rx, ry, rphi, s_line, slow_steps);
+                                apply_event(a.events[e], a.radius_u_turn, rx, ry, rphi, s_line, t.slow_steps);
                                 fired = true;
                             }
                         if (fired) s_events += 1;
-                    }
-                    xprev = rx; yprev = ry;
+                    });
                 }
                 s_ctl[4] = stop;
             }
@@ -299,17 +347,154 @@ __global__ void __launch_bounds__(kLoopThreads) held_loop_kernel(const LoopArgs 
             }
         }
         if (tid == 0) {
-            a.out_ticks[n] = ticks;
-            a.out_status[n] = status;
+            a.out_ticks[n] = t.ticks;
+            a.out_status[n] = t.status;
             if (a.out_final) {
                 double *f = a.out_final + 6 * n;
-                f[0] = cost.xt; f[1] = cost.yt; f[2] = cost.ox; f[3] = cost.oy; f[4] = (double)slow_steps; f[5] = (double)m;
+                f[0] = cost.xt; f[1] = cost.yt; f[2] = cost.ox; f[3] = cost.oy; f[4] = (double)t.slow_steps;
+                f[5] = (double)t.m;
             }
             if constexpr (kGen == kGenPcg64) pcg64_store(pcg, a.pcg_state + (size_t)n * kPcgWords);
         }
         if constexpr (kGen == kGenMt19937)       // thread 0's last draw came before the barrier that ended the loop
             for (int i = tid; i < kMtWords; i += kLoopThreads) a.rng_state[(size_t)n * kMtWords + i] = s_mt[i];
     }
+}
+
+// ---------------------------------------------------------------------------------------------
+// The online controller stepped one tick at a time on per-robot records (mpcb_held_ctrl, include/mpcb200.h), so that the
+// caller's plant sits between two steps.  One CTA per robot, grid-stride: thread 0 loads the record into the LoopTick of
+// held_loop_kernel and commits the pending proposal with the caller's measured state (tick_commit, then the robot's own
+// events of this step); the CTA then runs the head of the next tick with the loop's windows, solve and tick_propose, and
+// thread 0 stores the record back.  The loop kernel keeps the same state in registers and shared memory for a whole run.
+__device__ __forceinline__ void ctrl_store(mpcb_held_ctrl *rec, const LoopTick &t, const double *opt, int H,
+                                           const double *pose, const double *line, bool pending) {
+    for (int k = 0; k < 5; ++k) rec->pose[k] = pose[k];
+    for (int k = 0; k < 4; ++k) rec->line[k] = line[k];
+    rec->threshold = t.thr;
+    rec->prev[0] = t.xprev; rec->prev[1] = t.yprev;
+    for (int k = 0; k < 3 * H; ++k) rec->opt[k] = opt[k];
+    rec->command[0] = t.res_v; rec->command[1] = t.res_beta;
+    rec->slow_steps = t.slow_steps; rec->m = t.m; rec->ticks = t.ticks; rec->status = t.status;
+    rec->recursive = t.recursive; rec->have_traj = t.have_traj; rec->pending = pending;
+}
+
+__global__ void __launch_bounds__(kLoopThreads) held_ctrl_step_kernel(const HeldCtrlArgs a) {
+    __shared__ double s_V[kMaxWin], s_B[kMaxWin], s_tanB[kMaxWin];
+    __shared__ double s_J[kLoopThreads / 32];
+    __shared__ int s_j[kLoopThreads / 32];
+    __shared__ double s_state[5];      // the committed x, y, phi, v, beta the head starts from
+    __shared__ double s_line[4];       // x_t, y_t, x_0, y_0 after this step's events
+    __shared__ int s_ctl[4];           // nV, nB, slow flag, the robot runs the head
+    __shared__ double s_vslow;
+    const mpcb_loop_params &p = a.p;
+    const int tid = threadIdx.x;
+    for (long long n = blockIdx.x; n < a.N; n += gridDim.x) {
+        mpcb_held_ctrl *rec = a.ctrl + n;
+        LoopTick t;
+        double opt[3 * MPCB_MAX_H];
+        LoopCost cost;
+        bool committed = false;
+        __syncthreads();                           // the previous robot's shared state has been consumed
+        if (tid == 0) {
+            for (int k = 0; k < 5; ++k) s_state[k] = rec->pose[k];
+            for (int k = 0; k < 4; ++k) s_line[k] = rec->line[k];
+            t.thr = rec->threshold;
+            t.xprev = rec->prev[0]; t.yprev = rec->prev[1];
+            for (int k = 0; k < 3 * p.H; ++k) opt[k] = rec->opt[k];
+            t.res_v = rec->command[0]; t.res_beta = rec->command[1];
+            t.slow_steps = rec->slow_steps; t.m = rec->m; t.ticks = rec->ticks; t.status = rec->status;
+            t.recursive = rec->recursive != 0; t.have_traj = rec->have_traj != 0;
+            const int status0 = t.status;
+            bool run = t.status == MPCB_LOOP_RUNNING;
+            if (run && rec->pending) {
+                // ---- tail of the previous tick: the plant's answer to the proposal
+                committed = true;
+                if (a.measured)
+                    for (int k = 0; k < 5; ++k) s_state[k] = a.measured[5 * n + k];
+                const double x = s_state[0], y = s_state[1], phi = s_state[2];
+                if (tick_commit(t, x, y, [&] {
+                        for (int e = 0; e < a.n_ev; ++e) {
+                            const mpcb_loop_event &ev = a.events[(size_t)n * a.n_ev + e];
+                            if (ev.kind >= MPCB_EVENT_NEW_TARGET && ev.kind <= MPCB_EVENT_TURN_RIGHT)
+                                apply_event(ev, a.radius_u_turn, x, y, phi, s_line, t.slow_steps);
+                        }
+                    }))
+                    run = false;
+            }
+            load_cost(cost, s_line, s_line + 2, 0, p.cost_kind);
+            if (run && tick_stop(p, cost, t, s_state[0], s_state[1])) run = false;
+            s_ctl[2] = t.slow_steps > 0; s_ctl[3] = run;
+            if (!run) {
+                if (a.proposal)
+                    for (int k = 0; k < 5; ++k) a.proposal[5 * n + k] = NAN;
+                if (committed || t.status != status0) ctrl_store(rec, t, opt, p.H, s_state, s_line, false);
+            }
+        }
+        __syncthreads();
+        if (!s_ctl[3]) continue;
+        if (tid != 0) load_cost(cost, s_line, s_line + 2, 0, p.cost_kind);
+
+        // ---- head of the next tick: windows, HELD solve, proposal
+        build_windows(p, s_state[3], s_state[4], s_V, s_B, s_ctl, &s_vslow);
+        __syncthreads();
+        const int nV = s_ctl[0], nB = s_ctl[1];
+        const bool slow = s_ctl[2] != 0;
+        for (int i = tid; i < nB; i += kLoopThreads) s_tanB[i] = tan(s_B[i]);
+        __syncthreads();
+        const double x0 = s_state[0], y0 = s_state[1], phi0 = s_state[2];
+        double bJ; int bj;
+        held_block_solve(p, cost, s_V, s_tanB, nV, nB, slow, s_vslow, x0, y0, phi0, s_J, s_j, bJ, bj);
+        if (tid == 0) {
+            const bool accepted = bj >= 0 && bJ < t.thr;  // strict '<' (math_model_tree.py:351)
+            double r[5];
+            const bool proposed = tick_propose(p, cost, t, opt, accepted, bj, nB, slow, s_vslow, s_V, s_B, s_tanB, x0, y0,
+                                               phi0, r[0], r[1], r[2]);
+            r[3] = t.res_v; r[4] = t.res_beta;
+            if (a.proposal)
+                for (int k = 0; k < 5; ++k) a.proposal[5 * n + k] = proposed ? r[k] : NAN;
+            if (proposed && a.running) atomicAdd(a.running, 1);
+            ctrl_store(rec, t, opt, p.H, proposed ? r : s_state, s_line, proposed);
+        }
+    }
+}
+
+// the records of mpcb_held_ctrl_init_device, one thread per robot
+__global__ void __launch_bounds__(128) held_ctrl_init_kernel(long long N, const double *init, const double *target,
+                                                             const double *origin, const double *first_threshold,
+                                                             const int *slow_steps, mpcb_held_ctrl *ctrl) {
+    const long long n = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (n >= N) return;
+    mpcb_held_ctrl *rec = ctrl + n;
+    for (int k = 0; k < 5; ++k) rec->pose[k] = init[5 * n + k];
+    rec->line[0] = target[2 * n]; rec->line[1] = target[2 * n + 1];
+    rec->line[2] = origin[2 * n]; rec->line[3] = origin[2 * n + 1];
+    rec->threshold = first_threshold ? first_threshold[n] : INFINITY;
+    rec->prev[0] = init[5 * n]; rec->prev[1] = init[5 * n + 1];
+    for (int k = 0; k < 3 * MPCB_MAX_H; ++k) rec->opt[k] = 0.0;
+    rec->command[0] = 0.0; rec->command[1] = 0.0;
+    rec->slow_steps = slow_steps ? slow_steps[n] : 0;
+    rec->m = 0; rec->ticks = 0; rec->status = MPCB_LOOP_RUNNING;
+    rec->recursive = 0; rec->have_traj = 0; rec->pending = 0; rec->reserved = 0;
+}
+
+cudaError_t launch_held_ctrl_init(cudaStream_t st, long long N, const double *init, const double *target,
+                                  const double *origin, const double *first_threshold, const int *slow_steps,
+                                  mpcb_held_ctrl *ctrl) {
+    held_ctrl_init_kernel<<<(unsigned)((N + 127) / 128), 128, 0, st>>>(N, init, target, origin, first_threshold,
+                                                                       slow_steps, ctrl);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_held_ctrl_step(cudaStream_t st, const HeldCtrlArgs &a, int sms) {
+    int per_sm = 0;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, held_ctrl_step_kernel, kLoopThreads, 0) != cudaSuccess ||
+        per_sm < 1)
+        per_sm = 1;
+    long long grid = (long long)sms * per_sm;
+    if (grid > a.N) grid = a.N;
+    held_ctrl_step_kernel<<<(unsigned)grid, kLoopThreads, 0, st>>>(a);
+    return cudaGetLastError();
 }
 
 // The generators of the actual run, seeded as numpy's RandomState(keys[n]) (key_len == 0) or RandomState(keys[n, :])

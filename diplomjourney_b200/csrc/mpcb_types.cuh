@@ -275,6 +275,19 @@ struct LoopArgs {
     double *trace_pred, *trace_ctl, *trace_cost;
 };
 
+// one step of the online controller on per-robot records (mpcb_loop.cu, held_ctrl_step_kernel); all pointers are device
+struct HeldCtrlArgs {
+    mpcb_loop_params p;
+    long long N;
+    mpcb_held_ctrl *ctrl;                              // [N] in/out
+    const double *measured;                            // [N][5] applied state of the pending proposals, nullable
+    const mpcb_loop_event *events;                     // [N][n_ev], nullable with n_ev == 0
+    int n_ev;
+    double radius_u_turn;
+    double *proposal;                                  // [N][5], nullable
+    int *running;                                      // robots holding a proposal after the step (added), nullable
+};
+
 // one online tick of a batch of robots with per-robot acceleration windows (mpcb_loop.cu); all pointers are device
 struct WindowArgs {
     mpcb_loop_params p;

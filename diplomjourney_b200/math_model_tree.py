@@ -662,9 +662,68 @@ def _math_mpc_batch_device_noise(params, ini, tgt, org, first, rngs, events, see
     return r
 
 
+def _math_mpc_batch_actuator(params, ini, tgt, org, first, events, actuator):
+    """The actual run with the caller's actuator model in place of get_actual_velocity / get_actual_beta_angle: the
+    online controller stepped one tick at a time on the device (``mpcb_held_ctrl_step_device``), ``actuator`` run
+    between two steps on the solver's stream, so that nothing waits for the device but the one read of the running
+    count per step.  The committed rows (the proposal's pose with the applied v, beta) are appended to the log on the
+    device."""
+    import ctypes
+
+    import torch
+    solver = _solver()
+    n, T = ini.shape[0], params.max_ticks
+    script = ACTUAL_EVENTS if events is True else list(events or ())
+    if any(int(e[1]) not in (_native.EVENT_NEW_TARGET, _native.EVENT_TURN_LEFT, _native.EVENT_TURN_RIGHT) for e in script):
+        raise ValueError("event kinds are _native.EVENT_NEW_TARGET, EVENT_TURN_LEFT or EVENT_TURN_RIGHT")
+    dev = torch.device("cuda", solver.device)
+    f64 = dict(dtype=torch.float64, device=dev)
+    with torch.cuda.device(dev), torch.cuda.stream(torch.cuda.ExternalStream(solver.stream, device=dev)):
+        ini_d, tgt_d = torch.tensor(ini, **f64), torch.tensor(np.ascontiguousarray(tgt), **f64)
+        org_d, first_d = torch.tensor(np.ascontiguousarray(org), **f64), torch.tensor(first, **f64)
+        ctrl = torch.empty((n, ctypes.sizeof(_native.HeldCtrl)), dtype=torch.uint8, device=dev)
+        log = torch.full((n, T, 5), math.nan, **f64)
+        proposal, measured = torch.empty((n, 5), **f64), torch.empty((n, 5), **f64)
+        running = torch.zeros(1, dtype=torch.int32, device=dev)
+        count = torch.zeros(n, dtype=torch.int64, device=dev)      # rows each robot has committed
+        rows = torch.arange(n, device=dev) * T
+        # the script's tick s goes to the step that commits tick s, the same events for every robot
+        step_events = {}
+        for s in sorted({int(e[0]) for e in script}):
+            todo = [e for e in script if int(e[0]) == s]
+            ev = (_native.LoopEvent * len(todo))(*(_native.LoopEvent(s, int(k), float(a), float(b)) for _, k, a, b in todo))
+            row = np.frombuffer(bytes(ev), np.uint8)
+            step_events[s] = (torch.tensor(np.tile(row, (n, 1)), device=dev), len(todo))
+        solver.held_ctrl_init_device(params, n, ini_d.data_ptr(), tgt_d.data_ptr(), org_d.data_ptr(), first_d.data_ptr(),
+                                     0, ctrl.data_ptr())
+        solver.held_ctrl_step_device(params, n, ctrl.data_ptr(), proposal=proposal.data_ptr(), running=running.data_ptr())
+        step = 0
+        while int(running.item()):
+            step += 1
+            mask = ~torch.isnan(proposal[:, 0])
+            applied = torch.as_tensor(actuator(proposal[:, 3:5].clone(), mask), **f64).reshape(n, 2)
+            measured[:, :3] = proposal[:, :3]
+            measured[:, 3:] = applied
+            flat, lf = rows + count.clamp(max=T - 1), log.view(-1, 5)
+            lf[flat] = torch.where(mask[:, None], measured, lf[flat])
+            count += mask
+            running.zero_()
+            ev, n_ev = step_events.get(step, (None, 0))
+            solver.held_ctrl_step_device(params, n, ctrl.data_ptr(), measured.data_ptr(),
+                                         0 if ev is None else ev.data_ptr(), n_ev, radius_u_turn, proposal.data_ptr(),
+                                         running.data_ptr())
+        rec = ctrl.cpu().numpy()
+        log = log.cpu().numpy()
+    d, w = rec.view(np.float64), rec.view(np.int32)
+    R = _native.HeldCtrl
+    line = d[:, R.line.offset // 8:R.line.offset // 8 + 4]
+    final = np.concatenate([line, w[:, [R.slow_steps.offset // 4, R.m.offset // 4]].astype(np.float64)], axis=1)
+    return dict(log=log, ticks=w[:, R.ticks.offset // 4].copy(), status=w[:, R.status.offset // 4].copy(), final=final)
+
+
 def math_mpc_batch(initial_coordinates, target_coordinates, max_ticks=512, origin=None, cost_kind=None,
                    isActual=False, rngs=None, events=False, host_loop=False, device_noise=False, seeds=None,
-                   generator=None, logs=False):
+                   generator=None, logs=False, actuator=None):
     """EXTENSION (not in the reference): the closed loop of ``math_mpc`` for a whole batch of robots.
     ``initial_coordinates`` [N][5] = x, y, phi, v, beta; ``target_coordinates`` [N][2].  The tracked line starts at
     the module's x_0, y_0 unless ``origin`` [N][2] is given.
@@ -706,7 +765,24 @@ def math_mpc_batch(initial_coordinates, target_coordinates, max_ticks=512, origi
       result_beta.  (Unlike the per-tick path's ``robots``, result_{x,y}_{velocity,acceleration} are filled, as
       ``math_mpc`` fills them.)
 
+    * ``isActual=True, actuator=fn``: the actual run with the caller's actuator model in place of
+      get_actual_velocity / get_actual_beta_angle, the controller stepped on the device one tick at a time
+      (``mpcb_held_ctrl_step_device``).  ``fn(commanded, running)`` gets a float64 CUDA tensor [N][2] of this tick's
+      commanded (v, beta) (NaN rows for robots without a proposal) and a bool mask of the robots with one, on the
+      solver's stream, and returns the applied [N][2]; the tick commits the proposed pose with those.  Events as with
+      ``device_noise``.  Returns log, ticks, status and final as the device loops do.  Not together with ``rngs``,
+      ``seeds``, ``device_noise``, ``host_loop`` or ``logs``.
+
     Returns dict(log[N][max_ticks][5], ticks[N], status[N])."""
+    if actuator is not None:
+        if not isActual:
+            raise ValueError("actuator= replaces the actual run's actuator noise: it needs isActual=True")
+        clash = [k for k, on in (("rngs", rngs is not None), ("seeds", seeds is not None), ("device_noise", device_noise),
+                                 ("host_loop", host_loop), ("logs", logs)) if on]
+        if clash:
+            raise ValueError(f"actuator= is the actuator model of the stepped run; it does not go with {', '.join(clash)}")
+        if not callable(actuator):
+            raise TypeError("actuator must be callable: fn(commanded[N][2], running[N]) -> applied[N][2]")
     from . import config as _cfg
     ini = np.asarray(initial_coordinates, dtype=np.float64).reshape(-1, 5)
     org = np.array([[x_0, y_0]], dtype=np.float64) if origin is None else np.asarray(origin, np.float64).reshape(-1, 2)
@@ -757,6 +833,8 @@ def math_mpc_batch(initial_coordinates, target_coordinates, max_ticks=512, origi
         g.update(x_t=saved[0], y_t=saved[1], x_0=saved[2], y_0=saved[3])
     params = _native.LoopParams.from_config(_cfg, _native.COST_TREE if cost_kind is None else cost_kind,
                                             prediction_horizon, max_ticks)
+    if actuator is not None:
+        return _math_mpc_batch_actuator(params, ini, tgt, org, first, events, actuator)
     if device_noise:
         return _math_mpc_batch_device_noise(params, ini, tgt, org, first, rngs, events, seeds, kind, logs)
     if isActual or host_loop:

@@ -349,6 +349,69 @@ MPCB_API int mpcb_held_closed_loop_pcg64_seeded_host(mpcb_handle *h, const mpcb_
                                             double *out_log, int32_t *out_ticks, int32_t *out_status,
                                             double *out_final);
 
+/* The online controller stepped ONE tick at a time, so that a caller's own plant -- a simulator, an actuator model --
+ * closes the loop.  The controller's per-robot state lives in device memory, in one mpcb_held_ctrl record per robot,
+ * between calls.  A tick of the closed loop splits where the actuator sits:
+ *   head  stop test (on target: MPCB_LOOP_ON_TARGET; ticks >= max_ticks: MPCB_LOOP_MAX_TICKS), the acceleration windows,
+ *         the HELD solve, accept under the threshold, the slow-down countdown, the no-leaf stop, the finishing heuristic,
+ *         threshold := sys.maxsize.  Its result is the proposal (x, y, phi, v, beta): the pose the controller predicts
+ *         and the (v, beta) it commands.
+ *   tail  commit the applied state (ticks += 1), the "Recursive error" stop, the repeated-position test, the operator
+ *         events of this tick.
+ * ONE step = the tail of the previous tick + the head of the next:
+ *   1. a robot holding a proposal commits measured[n] = (x, y, phi, v, beta), what the caller's plant made of the
+ *      proposal (measured == NULL commits the proposal unchanged: the noise-free loop).  Then its events of this step are
+ *      applied in order, to the committed pose, as mpcb_held_closed_loop_events_host applies a script's events after a
+ *      tick; a robot that stopped in the commit ignores them.
+ *   2. a robot still running runs the head and writes its proposal to proposal[n]; a robot that is not running gets a
+ *      NaN row.
+ * Call the step until no robot is running.  The step that commits a robot's last proposal is the one that stops it, so
+ * the last step writes only NaN rows.  Events passed to a step with nothing to commit (the first) are ignored, as a
+ * script's tick-0 event is.  With measured == NULL (or measured = the proposal handed back) the proposals are, tick by
+ * tick, the log of mpcb_held_closed_loop_events_host on the same robots, and the records' ticks, status, line,
+ * slow_steps and m its out_ticks, out_status and out_final; with measured = (proposal pose, get_actual_velocity(v),
+ * get_actual_beta_angle(beta)) they are the actual run.
+ * The record's layout is part of the ABI (336 bytes, 8-byte aligned); callers read ticks, status, line, slow_steps and
+ * m from it. */
+#define MPCB_LOOP_RUNNING (-1)  /* mpcb_held_ctrl::status of a robot that has not stopped */
+typedef struct {
+    double pose[5];           /* x, y, phi, v, beta: the committed state; while a proposal is pending, the proposal */
+    double line[4];           /* x_t, y_t, x_0, y_0: the target and the origin of the tracked line (events move them) */
+    double threshold;         /* optimal_criterion */
+    double prev[2];           /* the position committed by the previous tick (repeated-position test) */
+    double opt[3 * MPCB_MAX_H];  /* optimal_trajectory's poses [H][3] */
+    double command[2];        /* its commanded (v, beta): result_v (after the slow-down override), result_beta */
+    int32_t slow_steps;       /* steps_for_slowing */
+    int32_t m;                /* the finishing heuristic's counter */
+    int32_t ticks;            /* ticks committed */
+    int32_t status;           /* MPCB_LOOP_RUNNING, then MPCB_LOOP_* */
+    int32_t recursive;        /* a repeated position was seen: the next commit stops the robot */
+    int32_t have_traj;        /* optimal_trajectory is no longer the reference's [[[0]]] placeholder */
+    int32_t pending;          /* a proposal waits for its commit */
+    int32_t reserved;
+} mpcb_held_ctrl;
+/* The records ctrl[N] set up as mpcb_held_closed_loop_device sets up a robot: init[N][5] x, y, phi, v, beta,
+ * target[N][2], origin[N][2], first_threshold[N] (NULL = +inf), slow_steps[N] (NULL = 0).  Device pointers, enqueued on
+ * the handle's stream without a sync; the same records may be set up again at any time.  N < 0 (or N >= 2^31), a null
+ * pointer that is needed with N > 0 or p out of range (as for the closed loop) is MPCB_ERR_INVALID; N == 0 launches
+ * nothing. */
+MPCB_API int mpcb_held_ctrl_init_device(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, const double *init,
+                                        const double *target, const double *origin, const double *first_threshold,
+                                        const int32_t *slow_steps, mpcb_held_ctrl *ctrl);
+/* One step of the records ctrl[N] (see above).  p must be the one the records were set up with.
+ *   measured[N][5]      (nullable) the applied state of each robot's pending proposal; rows of other robots are not read
+ *   events[N][n_ev]     (nullable with n_ev == 0) per robot, the operator events of this step in order, as
+ *                       mpcb_loop_event with `tick` ignored; a kind outside 1..3 is no event (kind 0: an empty slot).
+ *                       0 <= n_ev <= 64.  radius_u_turn as for the closed loop.
+ *   proposal[N][5]      (nullable) each running robot's proposal, NaN for a robot that is not running
+ *   running             (nullable) a device int32 that receives, added to it, the number of robots holding a proposal
+ *                       after the step: zero it before the step
+ * Device pointers; enqueued on the handle's stream, no allocation, no copy, no sync, no handle scratch.  The records and
+ * events are device data and are not checked. */
+MPCB_API int mpcb_held_ctrl_step_device(mpcb_handle *h, const mpcb_loop_params *p, int64_t N, mpcb_held_ctrl *ctrl,
+                                        const double *measured, const mpcb_loop_event *events, int32_t n_ev,
+                                        double radius_u_turn, double *proposal, int32_t *running);
+
 /* What the reference's tick logs besides the 5-list, per robot and tick, on the same row as out_log (rows after a
  * robot's last tick: the host entries fill them with NaN, the device entries leave them alone):
  *   pred[N][max_ticks][H][3]  the poses of optimal_trajectory as the tick logs them (predicted_trajectory_*_anim*): the
